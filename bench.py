@@ -2,6 +2,7 @@
 """Benchmark of the scan hot path (BASELINE.json metric: scanned GB/s; configs[1] = 32 mixed patterns over 10 GiB).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--gib G] [--strong] [--no-extras]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One step = one pass of the hot path over one batch of synthetic syslog text (per rank: --gib GiB, default 10).
@@ -12,6 +13,8 @@ One step = one pass of the hot path over one batch of synthetic syslog text (per
   e2e_python : hypergrep_b200.grep(path, count_only=True) and hypergrep_b200.scan(path, python callback, buffer_count=16).
   roofline   : the streaming kernel (k_stream) against the measured HBM copy peak (MEASURED_PEAKS.json).
   parity     : the matched line numbers of the timed text (a bounded prefix) equal the oracle's, order included.
+  --dump-outputs DIR: what the last timed step computed, for comparing two builds on the same seeded text (see
+               dump_outputs).
   extra      : device-resident throughput of BASELINE configs[0], [2], [4] and the configs[3] file leg (N=1 only).
   cpu_baseline / --impl reference: the oracle port (reference loop shape, PCRE2-JIT matcher; the reference itself needs
                Hyperscan, which is not installable here) on the box's host cores, bounded sample.
@@ -50,6 +53,7 @@ def parse_args() -> argparse.Namespace:
     parser.add_argument("--cpu-seconds", type=float, default=15.0, help="target CPU time of the cpu_baseline sample")
     parser.add_argument("--strong", action="store_true", help="one text of --gib GiB split over the ranks, merged and checked")
     parser.add_argument("--no-extras", action="store_true", help="skip the extra configs / Python-level legs")
+    parser.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy")
     return parser.parse_args()
 
 
@@ -277,6 +281,30 @@ class LineCollector:
         return self.np.concatenate(self.parts) if self.parts else self.np.empty(0, dtype=self.np.uint64)
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(directory: str, prefix: str, last, scan_records) -> None:
+    """Write what the last timed step computed (float64 .npy files, at most DUMP_BYTES in all):
+      counts       : [bytes_scanned, lines, matches] of that step's statistics, what the timed call returns;
+      line_numbers : the matched line numbers in delivery order, from one more pass of the same call over the same device
+                     text with a callback (the timed call only counts them); a fixed seeded sample of them, kept in order,
+                     when there are more than fit."""
+    import numpy as np  # pylint: disable=import-outside-toplevel
+
+    counts = np.array([last.bytes_scanned, last.lines, last.matches], dtype=np.float64)
+    collector = LineCollector()
+    scan_records(ctypes.cast(collector.func, ctypes.c_void_p))
+    lines = collector.lines()
+    assert lines.size == last.matches, f"{lines.size} delivered records, the timed step counted {last.matches}"
+    cap = (DUMP_BYTES - counts.nbytes) // 8
+    if lines.size > cap:
+        lines = lines[np.sort(np.random.default_rng(0).choice(lines.size, cap, replace=False))]
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, f"{prefix}counts.npy"), counts)
+    np.save(os.path.join(directory, f"{prefix}line_numbers.npy"), lines.astype(np.float64))
+
+
 def main() -> None:  # pylint: disable=too-many-locals,too-many-statements,too-many-branches
     args = parse_args()
     rank = int(os.environ.get("RANK", "0"))
@@ -381,6 +409,7 @@ def main() -> None:  # pylint: disable=too-many-locals,too-many-statements,too-m
     matches = candidates = 0
     stream.wait_stream(torch.cuda.current_stream())
     begin.record(stream)
+    st = None
     for _ in range(args.steps):
         st = scan(dev.data_ptr(), size, 1, None)
         launches += st.launches
@@ -391,6 +420,9 @@ def main() -> None:  # pylint: disable=too-many-locals,too-many-statements,too-m
     end.record(stream)
     barrier()
     sampler.windows.append((window_begin, time.perf_counter()))
+    if args.dump_outputs and st is not None:
+        dump_outputs(args.dump_outputs, f"rank{rank}_" if world > 1 else "", st,
+                     lambda callback: scan(dev.data_ptr(), size, 1, callback))
     dev_ms = max_over_ranks(begin.elapsed_time(end))
     total_bytes = sum_over_ranks(float(size))
     value = total_bytes * args.steps / (dev_ms / 1e3) / 1e9

@@ -567,10 +567,6 @@ def test_device_text_reads_stay_inside_the_buffer():
     done = subprocess.run([sys.executable, script], capture_output=True, text=True, timeout=900, check=False)
     assert done.returncode == 0, done.stdout[-2000:] + done.stderr[-2000:]
     assert "guarded scans ok" in done.stdout
-    # control: the pages behind the mapping are not accessible to the device - a scan that is told the text is 64 bytes
-    # longer than the mapping ends with code 7
-    control = subprocess.run([sys.executable, script, "--negative"], capture_output=True, text=True, timeout=300, check=False)
-    assert control.returncode == 0 and "rc=7" in control.stdout, control.stdout[-1000:] + control.stderr[-1000:]
 
 
 def test_match_ends_from_host_and_device_memory(gpu_lib):
