@@ -438,6 +438,7 @@ struct Params {
     unsigned long long max_match;
     void* user_stream;
     EndsSink* ends = nullptr;   // gpugrep_match_ends(): end offsets instead of lines
+    bool invert = false;        // gpugrep_invert_scan_*(): deliver the pseudo-lines in which no pattern reports
 };
 
 // Largest prefix of [p, p+have) that ends on a pseudo-line boundary; 0 if none exists yet.
@@ -451,14 +452,28 @@ size_t cut_point(const uint8_t* p, size_t have, bool final, size_t limit) {
     return cut;
 }
 
+// slot_set_invert is weak (engine.hpp): absent only from CPU stand-ins of the engine without inverted scans (setup_job refuses
+// inverted scans there).
+void set_invert(ScanSlot* slot, bool invert) {
+    if (slot_set_invert) slot_set_invert(slot, invert);
+}
+
 int setup_job(const Params& pr, Job& job, Deliverer& out, unsigned long long weight = 0) {
     int rc = 0;
     job.db = cached_database(pr.patterns, pr.flags, pr.ids, pr.elements, rc, job.error);
+    if (job.db && pr.invert) {
+        // Which lines match does not depend on ids or SINGLEMATCH: once the set compiles as given, it is scanned as "every
+        // pattern SINGLEMATCH, one id 0" (simple mode, so multi-id sets take the fast path too), CASELESS/DOTALL/MULTILINE kept.
+        std::vector<unsigned> flags(pr.elements), ids(pr.elements, 0u);
+        for (unsigned i = 0; i < pr.elements; i++) flags[i] = (pr.flags ? pr.flags[i] : 0u) | 8u;
+        job.db = cached_database(pr.patterns, flags.data(), ids.data(), pr.elements, rc, job.error);
+    }
     if (!job.db) {
         std::fprintf(stderr, "ERROR: Unable to create database. Exiting.\n");   // same text as hyperscanner.c:297
         return GPUGREP_DB;
     }
     if (pr.buffer_size < 2) { job.error = "buffer_size must be at least 2"; return GPUGREP_SCAN; }
+    if (pr.invert && !slot_set_invert) { job.error = "this build of the engine has no inverted scan"; return GPUGREP_SCAN; }
     job.device_weight = weight;
     job.device = pick_device(weight, &job.device_charged);
     if (engine_select_device(job.device, job.error) != 0) {
@@ -564,7 +579,10 @@ int scan_file(const char* path, const Params& pr, gpugrep_stats* stats_out, cons
     }
 
     const bool count_only = !out.wants_lines() && pr.max_match == 0 && job.db->simple;
-    for (ScanSlot* sl : slots) slot_set_want_records(sl, !count_only);
+    for (ScanSlot* sl : slots) {
+        slot_set_want_records(sl, !count_only);
+        set_invert(sl, pr.invert);
+    }
     SegmentQueue q;
     for (int i = 0; i < kSlots; i++) q.free_slots.push_back(i);
     std::thread reader([&] {
@@ -726,8 +744,10 @@ int scan_memory(const uint8_t* data, size_t size, int location, const Params& pr
     ScanSlot* slots[2] = {engine_acquire_slot(err, location != GPUGREP_LOC_DEVICE), engine_acquire_slot(err, location != GPUGREP_LOC_DEVICE)};
     if (!slots[0] || !slots[1]) { engine_release_slot(slots[0]); engine_release_slot(slots[1]); set_last_error(err); return GPUGREP_SCRATCH; }
     const bool count_only = !out.wants_lines() && pr.max_match == 0 && job.db->simple;
-    slot_set_want_records(slots[0], !count_only);
-    slot_set_want_records(slots[1], !count_only);
+    for (ScanSlot* sl : slots) {
+        slot_set_want_records(sl, !count_only);
+        set_invert(sl, pr.invert);
+    }
     const uint8_t* seg_host[2] = {nullptr, nullptr};
     const uint8_t* seg_dev[2] = {nullptr, nullptr};
     size_t seg_len[2] = {0, 0};
@@ -1025,6 +1045,21 @@ static int scan_path(const char* path, const Params& pr, gpugrep_stats* stats) {
     }
     return scan_file(path, pr, stats);
 }
+
+// gpugrep_scan_buffer / gpugrep_invert_scan_buffer: one device, or - host memory, $GPUGREP_DEVICES - one byte range per device.
+static int scan_buffer(const void* data, size_t size, int location, const Params& pr, gpugrep_stats* stats) {
+    if (location == GPUGREP_LOC_HOST) {
+        const std::vector<int> devices = shard_devices();
+        if (!devices.empty() && size >= 2 * min_shard_bytes() && pr.buffer_size >= 2) {
+            const size_t shards = std::min(devices.size(), size / min_shard_bytes());
+            const std::vector<size_t> bounds = buffer_bounds((const uint8_t*)data, size, shards);
+            return scan_sharded(devices, bounds, pr, stats, [&](size_t, const ShardSpec& spec, gpugrep_stats* st) {
+                return scan_memory((const uint8_t*)data + spec.begin, spec.end - spec.begin, GPUGREP_LOC_HOST, pr, st, &spec);
+            });
+        }
+    }
+    return scan_memory((const uint8_t*)data, size, location, pr, stats);
+}
 }  // namespace gpugrep
 
 extern "C" {
@@ -1047,17 +1082,23 @@ int gpugrep_scan_buffer(const void* data, size_t size, int location, const char*
                         const unsigned int* pattern_ids, unsigned int elements, hs_event on_event, int buffer_size, int buffer_count,
                         unsigned long long max_match_count, void* stream, gpugrep_stats* stats) {
     gpugrep::Params pr{patterns, pattern_flags, pattern_ids, elements, on_event, buffer_size, buffer_count, max_match_count, stream};
-    if (location == GPUGREP_LOC_HOST) {
-        const std::vector<int> devices = gpugrep::shard_devices();
-        if (!devices.empty() && size >= 2 * gpugrep::min_shard_bytes() && pr.buffer_size >= 2) {
-            const size_t shards = std::min(devices.size(), size / gpugrep::min_shard_bytes());
-            const std::vector<size_t> bounds = gpugrep::buffer_bounds((const uint8_t*)data, size, shards);
-            return gpugrep::scan_sharded(devices, bounds, pr, stats, [&](size_t, const gpugrep::ShardSpec& spec, gpugrep_stats* st) {
-                return gpugrep::scan_memory((const uint8_t*)data + spec.begin, spec.end - spec.begin, GPUGREP_LOC_HOST, pr, st, &spec);
-            });
-        }
-    }
-    return gpugrep::scan_memory((const uint8_t*)data, size, location, pr, stats);
+    return gpugrep::scan_buffer(data, size, location, pr, stats);
+}
+
+int gpugrep_invert_scan_file(const char* file_name, const char* const* patterns, const unsigned int* pattern_flags, const unsigned int* pattern_ids,
+                             unsigned int elements, hs_event on_event, int buffer_size, int buffer_count, unsigned long long max_match_count,
+                             gpugrep_stats* stats) {
+    gpugrep::Params pr{patterns, pattern_flags, pattern_ids, elements, on_event, buffer_size, buffer_count, max_match_count, nullptr};
+    pr.invert = true;
+    return gpugrep::scan_path(file_name, pr, stats);
+}
+
+int gpugrep_invert_scan_buffer(const void* data, size_t size, int location, const char* const* patterns, const unsigned int* pattern_flags,
+                               const unsigned int* pattern_ids, unsigned int elements, hs_event on_event, int buffer_size, int buffer_count,
+                               unsigned long long max_match_count, void* stream, gpugrep_stats* stats) {
+    gpugrep::Params pr{patterns, pattern_flags, pattern_ids, elements, on_event, buffer_size, buffer_count, max_match_count, stream};
+    pr.invert = true;
+    return gpugrep::scan_buffer(data, size, location, pr, stats);
 }
 
 int gpugrep_match_ends(const void* data, size_t size, int location, const char* const* patterns, const unsigned int* pattern_flags,

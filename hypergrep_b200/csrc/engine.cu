@@ -8,6 +8,8 @@
 //           k_stream -> scan -> k_list_candidates [-> k_confirm] -> k_verify_smem | k_verify_local -> k_tile_offsets -> k_emit_nlm -> k_dedupe_records
 //   GENERAL (everything else, and the fallback when a fast-path capacity bound is hit):
 //           k_stream(no filter) -> scan -> k_newline_positions -> pseudo-line table -> k_match_pl_* -> scan -> emit
+// INVERTED scans (grep -v) select the lines without a match: the fast path adds a complement stage after the dedupe
+// (k_invert.cuh, run from slot_collect), the general path negates the per-line flags of k_match_pl_simple.
 // All byte offsets inside a segment are 32-bit (segments are < 4 GiB); line numbers are rebased on the host.
 // Device code lives in the .cuh files included below (one translation unit); this file holds the host side: device
 // tables, scan slots, the launch sequence of a segment and the collection of its results.
@@ -33,6 +35,7 @@
 #include "dfa_walk.cuh"
 #include "k_fast.cuh"
 #include "k_general.cuh"
+#include "k_invert.cuh"
 
 namespace gpugrep {
 
@@ -142,6 +145,7 @@ public:
     cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};   // 0/1: whole segment, 2/3: streaming kernel
     DevBuf d_input, d_meta, d_nlmask, d_gsum, d_prefix, d_sums, d_cand, d_res, d_recoff, d_recs, d_totals;
     DevBuf d_nlpos, d_npl, d_ploff, d_plstart, d_pllen, d_flags, d_counts, d_events, d_gather, d_gidx, d_hitinfo, d_survivors;
+    DevBuf d_linebits, d_invrecs;   // inverted fast path: matched-line bitmap, selected-line records
     PinBuf h_totals, h_recs, h_stage, h_gather, h_probe;
     // state of the in-flight segment
     const DeviceDb* ddb = nullptr;
@@ -150,10 +154,12 @@ public:
     int buffer_size = 0;
     bool fast = false;
     bool want_records = true;   // false: the caller only counts matches (no callback, no limit): skip the record D2H
+    bool invert = false;        // deliver the lines without a match (slot_set_invert)
     SegmentStats stats;
     bool in_use = false;
 
     int run_general(SegmentResult& out, std::string& error);
+    int run_complement(size_t nrec, size_t nlines, size_t selected, std::string& error);
 };
 
 int engine_select_device(int device, std::string& error) {
@@ -432,6 +438,7 @@ void engine_release_slot(ScanSlot* slot) {
 }
 
 void slot_set_want_records(ScanSlot* slot, bool want) { slot->want_records = want; }
+void slot_set_invert(ScanSlot* slot, bool invert) { slot->invert = invert; }
 
 uint8_t* slot_host_buffer(ScanSlot* slot, size_t capacity, std::string& error) {
     if (slot->h_stage.reserve(capacity + 64) != cudaSuccess) { error = "cudaHostAlloc failed for the staging buffer"; return nullptr; }
@@ -723,7 +730,7 @@ int ScanSlot::run_general(SegmentResult& out, std::string& error) {
     unsigned mgrid = (unsigned)((npl_total + 127) / 128);
     if (ddb->simple) {
         if (d_flags.reserve(npl_total) != cudaSuccess) { error = "cudaMalloc failed"; return 3; }
-        k_match_pl_simple<<<mgrid, 128, 0, st>>>(view, data, d_plstart.as<uint32_t>(), d_pllen.as<uint32_t>(), npl_total, d_flags.as<uint8_t>());
+        k_match_pl_simple<<<mgrid, 128, 0, st>>>(view, data, d_plstart.as<uint32_t>(), d_pllen.as<uint32_t>(), npl_total, d_flags.as<uint8_t>(), invert);
         stats.launches++;
         launch_scan(st, LoadU8{d_flags.as<uint8_t>()}, npl_total, d_recoff.as<unsigned long long>(), d_sums.as<unsigned long long>(), &dT->rec_total, stats);
         CUDA_TRY(cudaMemcpyAsync(hT, dT, sizeof(Totals), cudaMemcpyDeviceToHost, st));
@@ -773,6 +780,41 @@ int ScanSlot::run_general(SegmentResult& out, std::string& error) {
     return 0;
 }
 
+// Inverted fast path: records of the `selected` lines of the segment without a valid record among the first `nrec` of
+// d_recs, in line order, copied to h_recs.  One synchronisation (like run_general).
+int ScanSlot::run_complement(size_t nrec, size_t nlines, size_t selected, std::string& error) {
+    cudaStream_t st = stream;
+    Totals* dT = d_totals.as<Totals>();
+    const size_t nl_total = (size_t)(uint32_t)h_totals.as<Totals>()->meta_total;
+    const size_t nwords = (nlines + 31) / 32;
+    const size_t nb_scan = (nwords + kScanTile - 1) / kScanTile + 1;
+    // sized from the selected count, not from rec_cap: a text of very short lines selects up to one record per byte
+    if (d_linebits.reserve(nwords * 4) != cudaSuccess || d_recoff.reserve(nwords * 8) != cudaSuccess || d_sums.reserve(nb_scan * 8) != cudaSuccess ||
+        d_nlpos.reserve((nl_total + 1) * 4) != cudaSuccess || d_invrecs.reserve(selected * sizeof(LineRec)) != cudaSuccess) {
+        error = "cudaMalloc failed for the complement of an inverted scan"; return 3;
+    }
+    if (h_recs.reserve(selected * sizeof(LineRec)) != cudaSuccess) { error = "cudaHostAlloc failed"; return 3; }
+    uint32_t* bits = d_linebits.as<uint32_t>();
+    CUDA_TRY(cudaMemsetAsync(bits, 0, nwords * 4, st));
+    const unsigned sms = (unsigned)device_sms();
+    if (nrec) {
+        k_mark_lines<<<(unsigned)std::min<size_t>((nrec + 255) / 256, (size_t)sms * 8), 256, 0, st>>>(d_recs.as<LineRec>(), nrec, bits);
+        stats.launches++;
+    }
+    launch_scan(st, LoadPopc{bits}, nwords, d_recoff.as<unsigned long long>(), d_sums.as<unsigned long long>(), &dT->rec_total, stats);
+    k_newline_positions<<<(unsigned)((nblk * 32 + 255) / 256), 256, 0, st>>>(data, n, nblk, d_meta.as<unsigned long long>(), d_prefix.as<unsigned long long>(),
+                                                                           d_nlpos.as<uint32_t>(), d_nlmask.as<uint32_t>());
+    k_emit_unmarked<<<(unsigned)((nlines + 255) / 256), 256, 0, st>>>(d_nlpos.as<uint32_t>(), nl_total, n, nlines, bits, d_recoff.as<unsigned long long>(),
+                                                                     d_invrecs.as<LineRec>());
+    stats.launches += 2;
+    CUDA_TRY(cudaEventRecord(ev[1], st));
+    CUDA_TRY(cudaMemcpyAsync(h_recs.p, d_invrecs.p, selected * sizeof(LineRec), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaGetLastError());
+    stats.d2h_bytes += selected * sizeof(LineRec);
+    return 0;
+}
+
 int slot_collect(ScanSlot* s, SegmentResult& out, std::string& error, size_t split_above) {
     cudaStream_t st = s->stream;
     out = SegmentResult();
@@ -790,7 +832,16 @@ int slot_collect(ScanSlot* s, SegmentResult& out, std::string& error, size_t spl
             out.num_valid_recs = (size_t)hT->aux_total;
             const size_t nl_total = (size_t)(uint32_t)hT->meta_total;
             out.num_lines = nl_total + ((hT->last_byte & 0xff) != '\n' ? 1 : 0);
-            if (nrec && s->want_records) {
+            if (s->invert) {
+                // the valid records are the matched lines, one each: the complement has lines - valid records
+                const size_t selected = (size_t)out.num_lines - out.num_valid_recs;
+                if (selected && s->want_records) {
+                    int rc = s->run_complement(nrec, (size_t)out.num_lines, selected, error);
+                    if (rc) return rc;
+                }
+                nrec = selected;
+                out.num_valid_recs = selected;
+            } else if (nrec && s->want_records) {
                 if (s->h_recs.reserve(nrec * sizeof(LineRec)) != cudaSuccess) { error = "cudaHostAlloc failed"; return 3; }
                 CUDA_TRY(cudaMemcpyAsync(s->h_recs.p, s->d_recs.p, nrec * sizeof(LineRec), cudaMemcpyDeviceToHost, s->copy_stream));
                 CUDA_TRY(cudaStreamSynchronize(s->copy_stream));

@@ -79,6 +79,12 @@ int slot_submit(ScanSlot* slot, const DeviceDb& ddb, const DevicePrefilter* pf, 
 // Count-only callers (no callback, no match limit) need no records on the host: the record copy is skipped and
 // SegmentResult::lines stays null (num_valid_recs is still exact).  Call before slot_submit.
 void slot_set_want_records(ScanSlot* slot, bool want);
+// Inverted scan (grep -v): the segment's results are the pseudo-lines in which NO pattern reports, as LineRecs of a simple-mode
+// database (lines, num_line_recs, num_valid_recs; every record valid, kLineHasNul set conservatively).  num_lines is
+// unchanged.  Count-only (no records wanted) costs nothing beyond the normal scan: lines - matched.  Call before slot_submit.
+// Weak: a build of the host logic against a CPU stand-in of this engine that lacks inverted scans still links; the boundary
+// then fails inverted scans with 7 (there is no host-side complement).  engine.cu always defines it.
+__attribute__((weak)) void slot_set_invert(ScanSlot* slot, bool invert);
 // Wait for the segment and expose its results (valid until the next slot_submit on this slot).
 // Returns kSplitSegment (and no results) when the fast path hit one of its capacity bounds - a line too long for it, a
 // candidate or record overflow - in a segment of more than `split_above` bytes: the caller then scans the same bytes again

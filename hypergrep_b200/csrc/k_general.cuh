@@ -7,15 +7,17 @@ namespace gpugrep {
 // ------------------------------------------------------------------------------------------------------------
 // GENERAL PATH kernels
 // ------------------------------------------------------------------------------------------------------------
-// warp per 512-byte block: write the offset of every '\n' at its global rank
+// warp per 512-byte block: write the offset of every '\n' at its global rank.  `nlmask` (optional, the newline-chunk masks of
+// k_stream): only the 16-byte chunks that hold a newline are read.
 __global__ void __launch_bounds__(256) k_newline_positions(const uint8_t* __restrict__ data, size_t n, size_t nblk, const unsigned long long* __restrict__ meta,
-                                                           const unsigned long long* __restrict__ prefix, uint32_t* __restrict__ nlpos) {
+                                                           const unsigned long long* __restrict__ prefix, uint32_t* __restrict__ nlpos,
+                                                           const uint32_t* __restrict__ nlmask = nullptr) {
     const int lane = threadIdx.x & 31;
     size_t g = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (g >= nblk) return;
     size_t off = g * 512 + (size_t)lane * 16;
     uint32_t m = 0;
-    if (off < n) {
+    if (off < n && (!nlmask || ((nlmask[g] >> lane) & 1u))) {
         uint4 v = ld_chunk(data, off, n);
         m = newline_mask16(v);
         if (off + 16 > n) m &= (1u << (n - off)) - 1u;
@@ -69,11 +71,11 @@ __global__ void k_build_pseudo_lines(const uint32_t* __restrict__ nlpos, size_t 
 }
 
 __global__ void __launch_bounds__(128) k_match_pl_simple(DbView db, const uint8_t* __restrict__ data, const uint32_t* __restrict__ pl_start,
-                                                         const uint32_t* __restrict__ pl_len, size_t npl, uint8_t* __restrict__ flags) {
+                                                         const uint32_t* __restrict__ pl_len, size_t npl, uint8_t* __restrict__ flags, bool invert) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= npl) return;
     size_t st = pl_start[i];
-    flags[i] = block_matches<true>(db, data, st, st + pl_len[i]) ? 1 : 0;
+    flags[i] = block_matches<true>(db, data, st, st + pl_len[i]) != invert ? 1 : 0;   // invert: select the lines without a match
 }
 
 __global__ void k_emit_pl_simple(const uint32_t* __restrict__ pl_start, const uint32_t* __restrict__ pl_len, size_t npl, const uint8_t* __restrict__ flags,

@@ -147,11 +147,19 @@ def parallel_grep(  # pylint: disable=too-many-arguments,too-many-locals
     files_without_match: bool = False,
     files_with_matches: bool = False,
     quiet: bool = False,
+    invert_match: bool = False,
 ) -> int:
     """Scan files and print grep-formatted results (reference multiscanner.py:86-223).
 
     Returns the grep exit code: 2 if any file errored, else 1 if nothing matched, else 0.
+    ``invert_match`` (``-v``) selects the lines that no pattern matches; every other option then applies to those lines.
     """
+    if invert_match and only_matching:
+        # GNU grep -v -o: a selected line has no matching part, so nothing is printed; the exit code still says whether
+        # some line was selected.  -c / -t / -l / -L keep their output.
+        only_matching = False
+        if not (count_results or total_results or files_with_matches or files_without_match):
+            quiet = True
     if files_without_match or files_with_matches or quiet:
         max_match_count = 1  # these modes only need to know whether a file matches at all
     printer = _OrderedPrinter(
@@ -173,6 +181,7 @@ def parallel_grep(  # pylint: disable=too-many-arguments,too-many-locals
         "only_matching": only_matching,
         "no_messages": no_messages,
         "max_match_count": max_match_count,
+        "invert_match": invert_match,
     }
     workers = min(max(multiprocessing.cpu_count() - 1, 1), len(files))
     pool_type = ThreadPool if use_multithreading else multiprocessing.Pool
@@ -283,6 +292,8 @@ def parse_args(args: list | None = None) -> argparse.Namespace:
     matching.add_argument("-f", "--file", action="append", dest="pattern_files", metavar="file",
                           help="Obtain patterns from FILE, one per line; may be repeated and combined with -e.")
     matching.add_argument("-i", "--ignore-case", action="store_true", help="Perform case insensitive matching.")
+    matching.add_argument("-v", "--invert-match", action="store_true",
+                          help="Invert the sense of matching, to select non-matching lines.")
 
     output = parser.add_argument_group("General Output Control")
     output.add_argument("-c", "--count", action="store_true",
@@ -378,6 +389,7 @@ def main() -> None:
             quiet=args.quiet,
             files_without_match=args.files_without_match,
             files_with_matches=args.files_with_matches,
+            invert_match=args.invert_match,
         )
     )
 

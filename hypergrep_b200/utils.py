@@ -145,18 +145,26 @@ def scan(  # pylint: disable=too-many-arguments
     buffer_size: int = 262140,
     buffer_count: int = 16,
     max_match_count: int = 0,
+    invert_match: bool = False,
 ) -> int:
     """Scan one plain/gzip/zstd file on the GPU, delivering matched lines in batches (reference utils.py:292-358).
 
     ``callback(matches, count)`` receives up to ``buffer_count`` ``Result`` records per call, in file order,
     with 0-based ``line_number``.  Returns the engine's code: 0, or 1-7 (reference hyperscanner.c:25-33).
+    ``invert_match`` (``grep -v``) delivers the lines that no pattern matches instead, each with id 0, and
+    ``max_match_count`` then counts those lines.
     """
     pattern_array, flags_array, ids_array = prepare_patterns(patterns, flags=flags, ids=ids)
     c_callback = CALLBACK_TYPE(callback)
     lib = _get_hyperscanner_lib()
+    entry = _invert_entry(lib) if invert_match else None
     outcome = {"rc": 0}
 
     def _run() -> None:
+        if entry is not None:
+            outcome["rc"] = entry(path.encode(), pattern_array, flags_array, ids_array, len(pattern_array), c_callback, buffer_size,
+                                  buffer_count, max_match_count, None)
+            return
         outcome["rc"] = lib.hyperscan(
             path.encode(),
             pattern_array,
@@ -191,18 +199,41 @@ class _Stats(ctypes.Structure):
     ]
 
 
-def _count_matches(path: str, patterns: Sequence[str], flags: Sequence[int], max_match_count: int) -> tuple[int, int] | None:
+_FILE_ENTRY_ARGTYPES = [ctypes.c_char_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint, ctypes.c_void_p,
+                        ctypes.c_int, ctypes.c_int, ctypes.c_ulonglong, ctypes.c_void_p]
+
+
+def _invert_entry(lib: ctypes.CDLL):
+    """gpugrep_invert_scan_file of the loaded library.  Inverted matching has no CPU fallback: a library without the entry
+    point (a plain libhyperscanner.so through GPUGREP_LIBRARY) is an error."""
+    try:
+        entry = lib.gpugrep_invert_scan_file
+    except AttributeError as error:
+        raise NotImplementedError(
+            "invert_match needs gpugrep_invert_scan_file, which the loaded native library does not export "
+            f"({_library_path()}); there is no CPU fallback"
+        ) from error
+    entry.restype = ctypes.c_int
+    entry.argtypes = _FILE_ENTRY_ARGTYPES
+    return entry
+
+
+def _count_matches(path: str, patterns: Sequence[str], flags: Sequence[int], max_match_count: int,
+                   invert_match: bool = False) -> tuple[int, int] | None:
     """Count-only scan without a callback: the library counts on the device and copies no line back
     (gpugrep_scan_file with on_event = NULL).  Returns None if the loaded library has no such entry point (a plain
-    libhyperscanner.so), in which case the caller counts through the callback like the reference does."""
+    libhyperscanner.so), in which case the caller counts through the callback like the reference does.
+    ``invert_match`` counts the lines without a match (gpugrep_invert_scan_file); it has no such fallback."""
     lib = _get_hyperscanner_lib()
-    try:
-        entry = lib.gpugrep_scan_file
-    except AttributeError:
-        return None
-    entry.restype = ctypes.c_int
-    entry.argtypes = [ctypes.c_char_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint, ctypes.c_void_p,
-                      ctypes.c_int, ctypes.c_int, ctypes.c_ulonglong, ctypes.c_void_p]
+    if invert_match:
+        entry = _invert_entry(lib)
+    else:
+        try:
+            entry = lib.gpugrep_scan_file
+        except AttributeError:
+            return None
+        entry.restype = ctypes.c_int
+        entry.argtypes = _FILE_ENTRY_ARGTYPES
     pattern_array, flags_array, ids_array = prepare_patterns(patterns, flags=flags)
     stats = _Stats()
     outcome = {"rc": 0}
@@ -229,12 +260,15 @@ def grep(  # pylint: disable=too-many-arguments
     no_messages: bool = False,
     errors: str = "ignore",
     max_match_count: int = 0,
+    invert_match: bool = False,
 ) -> tuple[int | list[tuple[int, str]], int]:
     """grep-like collector on top of :func:`scan` (reference utils.py:147-231).
 
     Returns ``(results, return_code)`` where results is a count (``count_only``) or a list of
     ``(1-based line number, line text)``.  Missing files raise FileNotFoundError, directories ValueError,
     unless ``no_messages`` is set, in which case the code is RC_INVALID_FILE.
+    ``invert_match`` (``grep -v``) selects the lines that no pattern matches; ``max_match_count`` and the count then
+    refer to those lines, and ``only_matching`` gives ``[]`` (a line without a match has no matching parts).
     """
     python_patterns = [re.compile(pattern) for pattern in patterns]
     collected: list[tuple[int, str]] = []
@@ -251,6 +285,8 @@ def grep(  # pylint: disable=too-many-arguments
             raise ValueError("is a directory")
     if code:
         return (0 if count_only else collected), code
+    if invert_match and only_matching and not count_only:
+        return collected, code
 
     # `-o`: spans from the engine's match END offsets where that is exact (patterns of one fixed width whose syntax means the
     # same in Python's re; ASCII lines), re.finditer() as in the reference (utils.py:205-212) for everything else.
@@ -279,7 +315,7 @@ def grep(  # pylint: disable=too-many-arguments
     pattern_flags = _DEFAULT_FLAGS | (HS_FLAG_CASELESS if ignore_case else 0)
     if count_only:
         # SURVEY.md section 8(f)-2: counting needs no line copies and no Python frame per batch of 16 results
-        counted = _count_matches(file, patterns, [pattern_flags] * len(patterns), max_match_count)
+        counted = _count_matches(file, patterns, [pattern_flags] * len(patterns), max_match_count, invert_match)
         if counted is not None:
             return counted
     code = scan(
@@ -289,6 +325,7 @@ def grep(  # pylint: disable=too-many-arguments
         flags=[pattern_flags] * len(patterns),
         max_match_count=max_match_count,
         buffer_count=_GREP_BATCH,
+        invert_match=invert_match,
     )
     if only_matching:
         _fill_spans(groups, deferred, patterns, widths, python_patterns, errors)

@@ -110,6 +110,23 @@ GPUGREP_API int gpugrep_scan_file(const char* file_name, const char* const* patt
                       const unsigned int* pattern_ids, unsigned int elements, hs_event on_event, int buffer_size,
                       int buffer_count, unsigned long long max_match_count, gpugrep_stats* stats);
 
+/* ---- inverted matching (`grep -v`) -------------------------------------------------------------------------------
+ * Same arguments, inputs (plain / gzip / zstd files, host / pinned / device buffers, $GPUGREP_DEVICES sharding) and
+ * return codes as gpugrep_scan_file / gpugrep_scan_buffer, but the delivered records are the pseudo-lines in which NO
+ * pattern reports: for every input, their line numbers are {0 .. lines-1} minus those of the non-inverted scan.
+ * Each selected line is one record with id 0; `line` is the stripped text (leading NULs skipped, cut at the next NUL), so a
+ * pseudo-line of NUL bytes only is delivered as "".  The pattern set is compile-checked as given (4 exactly when
+ * hyperscan() returns 4); ids and SINGLEMATCH do not change which lines are selected.  max_match_count counts selected
+ * lines (the scan stops after the line on which the count reaches it), buffer_count batches them as in hyperscan(), and
+ * stats->matches is the number of selected lines.  on_event == NULL without a limit counts on the device. */
+GPUGREP_API int gpugrep_invert_scan_file(const char* file_name, const char* const* patterns, const unsigned int* pattern_flags,
+                             const unsigned int* pattern_ids, unsigned int elements, hs_event on_event, int buffer_size,
+                             int buffer_count, unsigned long long max_match_count, gpugrep_stats* stats);
+GPUGREP_API int gpugrep_invert_scan_buffer(const void* data, size_t size, int location, const char* const* patterns,
+                               const unsigned int* pattern_flags, const unsigned int* pattern_ids, unsigned int elements,
+                               hs_event on_event, int buffer_size, int buffer_count, unsigned long long max_match_count,
+                               void* stream, gpugrep_stats* stats);
+
 /* ---- match END offsets (SURVEY.md section 8f-4: spans for `grep -o`) --------------------------------------------
  * The reference gets the spans of `-o` by re-running Python's re.finditer() over every matched line (utils.py:205-212);
  * Hyperscan itself reports (id, end offset) per match and the reference drops the offset (hyperscanner.c:83-102).
