@@ -214,12 +214,12 @@ size_t gpugrep_db_copy_depth(const gpugrep_db* h, unsigned int group, uint8_t* d
     return d.size();
 }
 
-size_t gpugrep_db_copy_prefilter(const gpugrep_db* h, uint32_t* words, size_t cap_words, uint32_t* hash_mul) {
+size_t gpugrep_db_copy_prefilter(const gpugrep_db* h, uint32_t* words, size_t cap_words, uint32_t* bloom_mul) {
     if (!h || !h->db->prefilter.enabled) return 0;
     const auto& pf = h->db->prefilter;
     size_t n = std::min(cap_words, pf.bitmap.size());
     if (words) std::memcpy(words, pf.bitmap.data(), n * sizeof(uint32_t));
-    if (hash_mul) *hash_mul = pf.hash_mul;
+    if (bloom_mul) *bloom_mul = pf.bloom_mul;   // the bitmap's multiplier (a tuned table picks it), not the exact table's
     return n;
 }
 

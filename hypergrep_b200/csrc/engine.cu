@@ -342,9 +342,18 @@ std::shared_ptr<DevicePrefilter> engine_upload_prefilter(const Prefilter& pf, st
         while (rshift > 0 && (3 * slots * 4) << rshift > 200 * 1024) rshift--;   // two halves + alignment slack of one half
         const size_t copies = (size_t)1 << rshift;
         replicated.resize(2 * slots * copies);
-        for (size_t half = 0; half < 2; half++)
+        for (size_t half = 0; half < 2; half++) {
+            // An empty slot holds 0, which reads as a hit for the gram 0 ("\0\0\0\0": NUL runs and the zero padding after the
+            // end of a segment), and that gram always probes slot 0.  An empty slot 0 gets a filler key that hashes elsewhere.
+            uint32_t slot0 = pf.keys[half * slots];
+            if (slot0 == 0) {
+                const uint32_t mul = half == 0 ? pf.hash_mul : pf.hash_mul2;
+                slot0 = 1;
+                while (prefilter_hash(slot0, mul, pf.log2_slots) == 0) slot0++;
+            }
             for (size_t h = 0; h < slots; h++)
-                for (size_t r = 0; r < copies; r++) replicated[half * slots * copies + h * copies + r] = pf.keys[half * slots + h];
+                for (size_t r = 0; r < copies; r++) replicated[half * slots * copies + h * copies + r] = h == 0 ? slot0 : pf.keys[half * slots + h];
+        }
         out->pp.rshift = rshift;
         out->pp.half_bytes = (uint32_t)(slots * copies * 4);
         // byte offset of slot h, copy r: ((h << rshift) | r) * 4.  h = product >> (32 - log2_slots), hence:

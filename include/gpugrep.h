@@ -226,8 +226,12 @@ GPUGREP_API size_t gpugrep_db_copy_depth(const gpugrep_db* db, unsigned int grou
 /* Reports of accept set `accept` of `group`: writes up to cap (id, singlematch) pairs, returns the count. */
 GPUGREP_API int gpugrep_db_accept_reports(const gpugrep_db* db, unsigned int group, unsigned int accept, unsigned int* ids,
                               unsigned int* singlematch, unsigned int cap);
-/* Copies the prefilter bitmap ((1 << log2_bits) / 32 words); returns words copied, 0 if disabled. */
-GPUGREP_API size_t gpugrep_db_copy_prefilter(const gpugrep_db* db, uint32_t* words, size_t cap_words, uint32_t* hash_mul);
+/* Copies up to cap_words words of the bloom bitmap that the streaming kernel probes by default (nothing if words is NULL);
+ * returns min(cap_words, bitmap words), 0 if the prefilter is disabled.  The bitmap has words * 32 bits
+ * (prefilter_log2_bits reports the exact table's slots instead when that table exists).  *bloom_mul receives its
+ * multiplier: gram g (OR-ed with 0x20202020 when prefilter_fold) hits iff, with p = g * bloom_mul mod 2^32, bit (p & 7) of
+ * byte p >> (32 - (log2(words * 32) - 3)) is set. */
+GPUGREP_API size_t gpugrep_db_copy_prefilter(const gpugrep_db* db, uint32_t* words, size_t cap_words, uint32_t* bloom_mul);
 /* Copies up to cap exact prefilter grams (little-endian 4-byte windows); returns the total gram count. */
 GPUGREP_API size_t gpugrep_db_copy_grams(const gpugrep_db* db, uint32_t* out, size_t cap);
 /* Mixed sampling (prefilter_stride == 4 only): besides the table lookups at text offsets = 0 (mod 4), the streaming kernel

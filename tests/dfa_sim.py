@@ -186,20 +186,27 @@ def _is_word(b: int) -> bool:
     return (48 <= b <= 57) or (65 <= b <= 90) or (97 <= b <= 122) or b == 95
 
 
+def prefilter_flagged_chunks(db: "CompiledDb", data: bytes) -> set:
+    """16-byte chunks (index = offset >> 4) in which a sampled gram starting below len(data) is one of the exact grams
+    (bytes past the end read as NUL)."""
+    st = db.info.prefilter_stride
+    fold = 0x20202020 if db.info.prefilter_fold else 0
+    flagged = set()
+    for q in range(0, len(data), 2 if db.odd else st):
+        gram = int.from_bytes(data[q:q + 4].ljust(4, b"\0"), "little") | fold
+        if db.gram_hit(gram, q):
+            flagged.add(q >> 4)
+    return flagged
+
+
 def fast_path_matched_line_starts(db: "CompiledDb", data: bytes) -> set:
     """CPU model of the fast path (simple mode): gram hits flag 16-byte chunks; every flagged chunk is verified by a
     LOCAL DFA walk that starts `lookback` bytes before the chunk (or at the line start if that is nearer), treats NUL
     as end-of-data + restart, follows lines that start inside the chunk and stops once the automaton is idle past
     the chunk.  Lines containing NUL are re-checked exactly.  Returns the start offsets of the matched lines."""
     n = len(data)
-    st = db.info.prefilter_stride
-    fold = 0x20202020 if db.info.prefilter_fold else 0
     lookback = db.info.prefilter_lookback
-    flagged = set()
-    for q in range(0, n, 2 if db.odd else st):
-        gram = int.from_bytes(data[q:q + 4].ljust(4, b"\0"), "little") | fold
-        if db.gram_hit(gram, q):
-            flagged.add(q >> 4)
+    flagged = prefilter_flagged_chunks(db, data)
     marked = set()
     for c in sorted(flagged):
         o = c * 16
@@ -256,7 +263,7 @@ def fast_path_matched_line_starts(db: "CompiledDb", data: bytes) -> set:
                 continue
             # past the last sampled gram of the chunk the walk stops as soon as nothing that is still in progress can have begun at
             # or before that gram (automata.hpp Dfa::depth; the kernels test this once per word, the model per byte)
-            ifrom = o + (18 if db.odd else 20 - st)
+            ifrom = o + (18 if db.odd else 20 - db.info.prefilter_stride)
             if pos >= ifrom and (done_line or all(int(db.depths[k][states[k]]) < min(pos - ifrom + 4, 255) for k in range(len(db.groups)))):
                 break
             if done_line and pos >= o + 16:
