@@ -318,6 +318,7 @@ struct Job {
         stats.d2h_bytes += r.stats.d2h_bytes;
         stats.path |= r.stats.path;
         stats.segments++;
+        stats.nul_segments += r.stats.nul ? 1u : 0u;
         if (stop) return 0;
         int rc = db->simple ? deliver_simple(r, host, slot) : deliver_events(r, host, slot);
         line_base += r.num_lines;
@@ -964,6 +965,7 @@ int scan_sharded(const std::vector<int>& devices, const std::vector<size_t>& bou
         total.h2d_bytes += stats[g].h2d_bytes; total.d2h_bytes += stats[g].d2h_bytes; total.gpu_ms += stats[g].gpu_ms;
         total.stream_kernel_ms += stats[g].stream_kernel_ms; total.launches += stats[g].launches;
         total.stream_launches += stats[g].stream_launches; total.segments += stats[g].segments; total.path |= stats[g].path;
+        total.nul_segments += stats[g].nul_segments;
     }
     // ordered merge on the calling thread
     Deliverer out(pr.cb, effective_batch(pr));

@@ -34,12 +34,16 @@ struct DbView {
 
 constexpr uint32_t kInvalidLen = 0xffffffffu;   // LineRec.len of a record the host must drop (NUL re-check failed)
 constexpr uint32_t kHasNulBit = 0x80000000u;    // LineRec.len flag: the line contains NUL bytes (host applies the strip/cut rule)
+constexpr unsigned int kFallbackFlags = 7u;      // Totals::flags bits that send a fast-path segment to the general path
+constexpr unsigned int kSegmentNulFlag = 8u;     // Totals::flags bit: some byte of the segment is NUL
 
 struct Totals {
     unsigned long long meta_total;   // candidates << 32 | newlines
     unsigned long long rec_total;    // records to emit (fast path) / generic scan totals
     unsigned long long aux_total;
-    unsigned int flags;              // bit0: a 64 KiB super-block without newline; bit1: candidate overflow; bit2: record overflow
+    // bit0: a 64 KiB super-block without newline; bit1: candidate overflow; bit2: record overflow (bits 0-2 send the segment
+    // to the general path); bit3: the segment holds a NUL byte (k_stream)
+    unsigned int flags;
     unsigned int last_byte;
     unsigned int max_line;           // general path: longest line
     unsigned int survivors;          // fast path: candidates that k_confirm kept (length of the survivor list)

@@ -6,6 +6,7 @@
 // Two paths produce identical results:
 //   FAST    (simple mode + literal prefilter + no over-long lines):
 //           k_stream -> scan -> k_list_candidates [-> k_confirm] -> k_verify_smem | k_verify_local -> k_tile_offsets -> k_emit_nlm -> k_dedupe_records
+//           (count-only: k_emit_nlm<*, true> -> k_count_keys, no records)
 //   GENERAL (everything else, and the fallback when a fast-path capacity bound is hit):
 //           k_stream(no filter) -> scan -> k_newline_positions -> pseudo-line table -> k_match_pl_* -> scan -> emit
 // INVERTED scans (grep -v) select the lines without a match: the fast path adds a complement stage after the dedupe
@@ -153,7 +154,7 @@ public:
     size_t n = 0, nblk = 0, cand_cap = 0, rec_cap = 0;
     int buffer_size = 0;
     bool fast = false;
-    bool want_records = true;   // false: the caller only counts matches (no callback, no limit): skip the record D2H
+    bool want_records = true;   // false: the caller only counts matches (no callback, no limit): the fast path counts without records
     bool invert = false;        // deliver the lines without a match (slot_set_invert)
     SegmentStats stats;
     bool in_use = false;
@@ -480,32 +481,34 @@ static void launch_scan(cudaStream_t st, Load load, size_t n, unsigned long long
     stats.launches += 3;
 }
 
-template <int STRIDE, bool FOLD, int MODE, int NODD = 0>
+template <int STRIDE, bool FOLD, int MODE, int NODD, bool NUL>
 static cudaError_t launch_stream_t(cudaStream_t st, int grid, int block, size_t smem, const uint8_t* data, size_t n, unsigned long long* meta,
-                                   uint32_t* nlmask, unsigned long long* gsum, const DevicePrefilter* pf) {
+                                   uint32_t* nlmask, unsigned long long* gsum, const DevicePrefilter* pf,
+                                   unsigned int* flags) {
     if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(k_stream<STRIDE, FOLD, MODE, NODD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(k_stream<STRIDE, FOLD, MODE, NODD, NUL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
     }
-    k_stream<STRIDE, FOLD, MODE, NODD><<<grid, block, smem, st>>>(data, n, meta, nlmask, gsum, pf ? pf->d_table : nullptr, pf ? pf->table_words : 0,
-                                                            pf ? pf->pp : ProbeParams{});
+    k_stream<STRIDE, FOLD, MODE, NODD, NUL><<<grid, block, smem, st>>>(data, n, meta, nlmask, gsum, pf ? pf->d_table : nullptr, pf ? pf->table_words : 0,
+                                                            pf ? pf->pp : ProbeParams{}, flags);
     return cudaGetLastError();
 }
 
-template <int MODE>
+template <int MODE, bool NUL>
 static cudaError_t launch_stream_m(cudaStream_t st, int grid, int block, size_t smem, const uint8_t* data, size_t n, unsigned long long* meta,
-                                   uint32_t* nlmask, unsigned long long* gsum, const DevicePrefilter* pf) {
+                                   uint32_t* nlmask, unsigned long long* gsum, const DevicePrefilter* pf,
+                                   unsigned int* flags) {
     int key = pf->stride * 2 + (pf->fold ? 1 : 0);
     if (MODE == 2 && pf->stride == 4 && pf->nodd > 0)
-        return pf->fold ? launch_stream_t<4, true, MODE, 2>(st, grid, block, smem, data, n, meta, nlmask, gsum, pf)
-                        : launch_stream_t<4, false, MODE, 2>(st, grid, block, smem, data, n, meta, nlmask, gsum, pf);
+        return pf->fold ? launch_stream_t<4, true, MODE, 2, NUL>(st, grid, block, smem, data, n, meta, nlmask, gsum, pf, flags)
+                        : launch_stream_t<4, false, MODE, 2, NUL>(st, grid, block, smem, data, n, meta, nlmask, gsum, pf, flags);
     switch (key) {
-        case 8: return launch_stream_t<4, false, MODE>(st, grid, block, smem, data, n, meta, nlmask, gsum, pf);
-        case 9: return launch_stream_t<4, true, MODE>(st, grid, block, smem, data, n, meta, nlmask, gsum, pf);
-        case 4: return launch_stream_t<2, false, MODE>(st, grid, block, smem, data, n, meta, nlmask, gsum, pf);
-        case 5: return launch_stream_t<2, true, MODE>(st, grid, block, smem, data, n, meta, nlmask, gsum, pf);
-        case 2: return launch_stream_t<1, false, MODE>(st, grid, block, smem, data, n, meta, nlmask, gsum, pf);
-        default: return launch_stream_t<1, true, MODE>(st, grid, block, smem, data, n, meta, nlmask, gsum, pf);
+        case 8: return launch_stream_t<4, false, MODE, 0, NUL>(st, grid, block, smem, data, n, meta, nlmask, gsum, pf, flags);
+        case 9: return launch_stream_t<4, true, MODE, 0, NUL>(st, grid, block, smem, data, n, meta, nlmask, gsum, pf, flags);
+        case 4: return launch_stream_t<2, false, MODE, 0, NUL>(st, grid, block, smem, data, n, meta, nlmask, gsum, pf, flags);
+        case 5: return launch_stream_t<2, true, MODE, 0, NUL>(st, grid, block, smem, data, n, meta, nlmask, gsum, pf, flags);
+        case 2: return launch_stream_t<1, false, MODE, 0, NUL>(st, grid, block, smem, data, n, meta, nlmask, gsum, pf, flags);
+        default: return launch_stream_t<1, true, MODE, 0, NUL>(st, grid, block, smem, data, n, meta, nlmask, gsum, pf, flags);
     }
 }
 
@@ -613,9 +616,14 @@ int slot_submit(ScanSlot* s, const DeviceDb& ddb, const DevicePrefilter* pf, con
     CUDA_TRY(cudaMemsetAsync(gsum + (ngroups ? ngroups - 1 : 0), 0, 16, st));
     CUDA_TRY(cudaEventRecord(s->ev[2], st));
     cudaError_t le;
-    if (!s->fast) le = launch_stream_t<4, false, 0>(st, grid, block, 0, s->data, n, meta, nlmask, gsum, nullptr);
-    else if (pf->mode == 1) le = launch_stream_m<1>(st, grid, block, smem, s->data, n, meta, nlmask, gsum, pf);
-    else le = launch_stream_m<2>(st, grid, block, smem, s->data, n, meta, nlmask, gsum, pf);
+    // the NUL test (Totals::flags bit 3) only serves count-only scans (k_emit_nlm<*, true>)
+    const bool nul_test = !s->want_records;
+    if (!s->fast) le = nul_test ? launch_stream_t<4, false, 0, 0, true>(st, grid, block, 0, s->data, n, meta, nlmask, gsum, nullptr, &dT->flags)
+                                : launch_stream_t<4, false, 0, 0, false>(st, grid, block, 0, s->data, n, meta, nlmask, gsum, nullptr, &dT->flags);
+    else if (pf->mode == 1) le = nul_test ? launch_stream_m<1, true>(st, grid, block, smem, s->data, n, meta, nlmask, gsum, pf, &dT->flags)
+                                          : launch_stream_m<1, false>(st, grid, block, smem, s->data, n, meta, nlmask, gsum, pf, &dT->flags);
+    else le = nul_test ? launch_stream_m<2, true>(st, grid, block, smem, s->data, n, meta, nlmask, gsum, pf, &dT->flags)
+                       : launch_stream_m<2, false>(st, grid, block, smem, s->data, n, meta, nlmask, gsum, pf, &dT->flags);
     if (le != cudaSuccess) { error = std::string("k_stream launch: ") + cudaGetErrorString(le); return 7; }
     CUDA_TRY(cudaEventRecord(s->ev[3], st));
     s->stats.launches++;
@@ -672,13 +680,22 @@ int slot_submit(ScanSlot* s, const DeviceDb& ddb, const DevicePrefilter* pf, con
                                           survivors, dT, s->d_res.as<uint32_t>(), tile_records);
         }
         k_tile_offsets<<<1, 1024, 0, st>>>(tile_records, &dT->meta_total, s->cand_cap, &dT->rec_total);
-        auto emit_kernel = ddb.nnfa > 0 ? k_emit_nlm<true> : k_emit_nlm<false>;
+        // Without records (count-only scans) the emit kernel writes one 4-byte key per record into the record buffer, and
+        // k_count_keys counts the distinct lines.  Either way a segment with more records than fit falls back to the general
+        // path (flags bit 2), so that the count never depends on the capacity.
+        const bool count_only = !s->want_records;
+        auto emit_kernel = ddb.nnfa > 0 ? (count_only ? k_emit_nlm<true, true> : k_emit_nlm<true, false>)
+                                        : (count_only ? k_emit_nlm<false, true> : k_emit_nlm<false, false>);
+        const size_t out_cap = count_only ? s->rec_cap * sizeof(LineRec) / sizeof(uint32_t) : s->rec_cap;
         const unsigned emit_per_sm = blocks_per_sm(emit_kernel, kEmitThreads);
         emit_kernel<<<(unsigned)std::min<size_t>((s->cand_cap + kEmitTile - 1) / kEmitTile, (size_t)emit_per_sm * sms), kEmitThreads, 0, st>>>(
             view, s->data, n, s->d_cand.as<uint32_t>(), s->d_res.as<uint32_t>(), tile_records, meta, prefix, nlmask, &dT->meta_total,
-            s->cand_cap, s->d_recs.as<LineRec>(), s->rec_cap, dT);
-        k_dedupe_records<<<(unsigned)std::min<size_t>((s->rec_cap + 255) / 256, (size_t)sms * 4), 256, 0, st>>>(s->d_recs.as<LineRec>(), s->rec_cap, dT);
-        s->stats.launches += 5;   // list, verify, tile offsets, emit, dedupe
+            s->cand_cap, s->d_recs.as<LineRec>(), s->d_recs.as<uint32_t>(), out_cap, dT);
+        if (count_only)
+            k_count_keys<<<(unsigned)std::min<size_t>((out_cap + 255) / 256, (size_t)sms * 4), 256, 0, st>>>(s->d_recs.as<uint32_t>(), out_cap, dT);
+        else
+            k_dedupe_records<<<(unsigned)std::min<size_t>((s->rec_cap + 255) / 256, (size_t)sms * 4), 256, 0, st>>>(s->d_recs.as<LineRec>(), s->rec_cap, dT);
+        s->stats.launches += 5;   // list, verify, tile offsets, emit, dedupe / key count
         CUDA_TRY(cudaEventRecord(s->ev[1], st));
     }
     CUDA_TRY(cudaMemcpyAsync(&dT->last_byte, s->data + n - 1, 1, cudaMemcpyDeviceToDevice, st));
@@ -832,10 +849,11 @@ int slot_collect(ScanSlot* s, SegmentResult& out, std::string& error, size_t spl
     s->stats.d2h_bytes += sizeof(Totals);
     if (s->n == 0) { out.stats = s->stats; return 0; }
     Totals* hT = s->h_totals.as<Totals>();
+    s->stats.nul = (hT->flags & kSegmentNulFlag) != 0;
     bool done = false;
     if (s->fast) {
         s->stats.candidates = hT->meta_total >> 32;
-        if (hT->flags == 0) {
+        if ((hT->flags & kFallbackFlags) == 0) {
             s->stats.path |= 1;
             size_t nrec = (size_t)hT->rec_total;   // includes records marked kInvalidLen (repeats of a line, failed NUL re-checks)
             out.num_valid_recs = (size_t)hT->aux_total;

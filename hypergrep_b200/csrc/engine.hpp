@@ -35,6 +35,7 @@ struct SegmentStats {
     unsigned long long candidates = 0;
     unsigned long long h2d_bytes = 0, d2h_bytes = 0;
     unsigned path = 0;   // bit0 fast path, bit1 general path
+    bool nul = false;    // the streaming kernel found a NUL byte in the segment (it tests in count-only scans only)
 };
 
 struct SegmentResult {
@@ -76,8 +77,9 @@ uint8_t* slot_host_buffer(ScanSlot* slot, size_t capacity, std::string& error);
 //  pf: gram table for the fast path, or nullptr (general path).
 int slot_submit(ScanSlot* slot, const DeviceDb& ddb, const DevicePrefilter* pf, const uint8_t* host_data, const uint8_t* dev_data, size_t n,
                 int buffer_size, void* user_stream, std::string& error);
-// Count-only callers (no callback, no match limit) need no records on the host: the record copy is skipped and
-// SegmentResult::lines stays null (num_valid_recs is still exact).  Call before slot_submit.
+// Count-only callers (no callback, no match limit) need no records on the host: the fast path counts the matched lines on
+// the device without building records, SegmentResult::lines stays null and num_valid_recs is exact (num_line_recs is then
+// the number of marked lines, repeats included).  Call before slot_submit.
 void slot_set_want_records(ScanSlot* slot, bool want);
 // Inverted scan (grep -v): the segment's results are the pseudo-lines in which NO pattern reports, as LineRecs of a simple-mode
 // database (lines, num_line_recs, num_valid_recs; every record valid, kLineHasNul set conservatively).  num_lines is

@@ -577,13 +577,39 @@ __device__ bool warp_nul_scan(const uint8_t* __restrict__ data, size_t n, uint32
     return false;
 }
 
+// Count-only identity of a line that is cheaper than its start: the chunk c that holds the newline in front of the line and
+// the rank r of that newline among the newlines of c counted from the last one (r = 0: the last), as c * 16 + 15 - r;
+// kNoNewlineKey for the first line of the segment.  Two records of one line get the same key, records of different lines
+// different keys, and the key of the line that contains an aligned chunk start o comes from nlmask words alone.
+constexpr uint32_t kNoNewlineKey = 0xfffffffeu;   // (chunk * 16 + 15 stays below it: segments are < 4 GiB - 1 KiB)
+__device__ uint32_t nlm_line_key(const uint32_t* __restrict__ nlmask, uint32_t o) {
+    const uint32_t c = o >> 4;
+    uint32_t b = c >> 5;
+    uint32_t w = nlmask[b] & ((1u << (c & 31u)) - 1u);   // chunks of this block below c
+    while (true) {
+        if (w) return (b * 32u + (31u - __clz(w))) * 16u + 15u;
+        if (b == 0) return kNoNewlineKey;
+        if (b >= 4) {   // four mask words per step, as nlm_line_start
+            const uint32_t w3 = nlmask[b - 1], w2 = nlmask[b - 2], w1 = nlmask[b - 3], w0 = nlmask[b - 4];
+            if (w3) { b -= 1; w = w3; } else if (w2) { b -= 2; w = w2; } else if (w1) { b -= 3; w = w1; } else { b -= 4; w = w0; }
+        } else {
+            b--;
+            w = nlmask[b];
+        }
+    }
+}
+
 constexpr uint32_t kNulBound = 512;
 // Records of one marked candidate chunk per lane; whole warps call it (`live`: this lane has a candidate).
-template <bool WITH_NFA>
+// `nul_free` (count-only scans): k_stream found no NUL byte in the segment, so no line needs the NUL scan and the exact re-check.
+// COUNT_ONLY: instead of a LineRec, one 32-bit key per record goes to keys[at] (kInvalidLen: failed NUL re-check), from
+// which k_count_keys counts the distinct valid lines; no line numbers.  In a NUL-free segment the key is nlm_line_key
+// (no line extents at all), else the line start (the extents are needed for the re-check anyway).
+template <bool WITH_NFA, bool COUNT_ONLY>
 __device__ uint32_t emit_lane_nlm(const DbView& db, const uint8_t* __restrict__ data, size_t n, const uint32_t* __restrict__ cand,
                                   const uint32_t* __restrict__ marks, const unsigned long long* __restrict__ meta,
                                   const unsigned long long* __restrict__ prefix, const uint32_t* __restrict__ nlmask, uint32_t nblk, bool live, size_t i,
-                                  size_t at, LineRec* __restrict__ recs, size_t rec_cap, Totals* totals) {
+                                  size_t at, LineRec* __restrict__ recs, uint32_t* __restrict__ keys, size_t rec_cap, bool nul_free, Totals* totals) {
     const uint32_t lane = threadIdx.x & 31;
     uint32_t valid = 0;
     uint32_t mask = live ? marks[i] : 0u;
@@ -592,6 +618,31 @@ __device__ uint32_t emit_lane_nlm(const DbView& db, const uint8_t* __restrict__ 
     if (live && ((nlmask[o >> 9] >> ((o >> 4) & 31u)) & 1u)) nlm = newline_mask16(ld_chunk(data, o, n));
     uint32_t st = 0;
     bool first = true;   // still on line 0 of the chunk (the line that contains byte o)
+    if (COUNT_ONLY && nul_free) {
+        // key of line j > 0 of the chunk: c * 16 + 15 - (newlines of the chunk behind the one in front of the line)
+        const uint32_t key_base = (o >> 4) * 16u + 15u;
+        while (mask != 0) {
+            while (!(mask & 1u)) {   // lines of the chunk that are not marked
+                if (!nlm) { mask = 0; break; }
+                nlm &= nlm - 1;
+                first = false;
+                mask >>= 1;
+            }
+            if (mask == 0) break;
+            const uint32_t key = first ? nlm_line_key(nlmask, o) : key_base - __popc(nlm);
+            valid++;
+            if (at < rec_cap) keys[at] = key;
+            else atomicOr(&totals->flags, 4u);
+            at++;
+            if (!nlm) mask = 0;
+            else {
+                nlm &= nlm - 1;
+                first = false;
+                mask >>= 1;
+            }
+        }
+        return valid;
+    }
     while (__any_sync(0xffffffffu, mask != 0)) {
         while (mask != 0 && !(mask & 1u)) {   // lines of the chunk that are not marked
             if (!nlm) { mask = 0; break; }
@@ -608,7 +659,7 @@ __device__ uint32_t emit_lane_nlm(const DbView& db, const uint8_t* __restrict__ 
             en = nlm ? o + __ffs(nlm) : nlm_line_end(data, n, nlmask, nblk, o + 16u < (uint32_t)n ? o + 16u : (uint32_t)n - 1u);
             // (nlm == 0 here means: no newline at or after st inside the chunk, so the line ends beyond it; if the chunk is
             //  the last one, the search starts at the last byte and returns n)
-            settled = nul_scan_bounded(data, n, st, en, kNulBound, &has_nul, &resume);
+            if (!nul_free) settled = nul_scan_bounded(data, n, st, en, kNulBound, &has_nul, &resume);
         }
         for (uint32_t pend = __ballot_sync(0xffffffffu, work && !settled); pend; pend &= pend - 1) {
             const int src = __ffs(pend) - 1;
@@ -618,9 +669,14 @@ __device__ uint32_t emit_lane_nlm(const DbView& db, const uint8_t* __restrict__ 
         if (work) {
             if (ok && has_nul) ok = block_matches<false>(db, data, st, en) || (WITH_NFA && block_matches_nfa(db, data, st, en));
             valid += ok ? 1u : 0u;
-            const uint32_t line_no = nlm_line_number(data, meta, prefix, nlmask, st);
-            if (at < rec_cap) recs[at] = LineRec{line_no, st, ok ? ((en - st) | (has_nul ? kHasNulBit : 0u)) : kInvalidLen};
-            else atomicOr(&totals->flags, 4u);
+            if (COUNT_ONLY) {
+                if (at < rec_cap) keys[at] = ok ? st : kInvalidLen;
+                else atomicOr(&totals->flags, 4u);
+            } else {
+                const uint32_t line_no = nlm_line_number(data, meta, prefix, nlmask, st);
+                if (at < rec_cap) recs[at] = LineRec{line_no, st, ok ? ((en - st) | (has_nul ? kHasNulBit : 0u)) : kInvalidLen};
+                else atomicOr(&totals->flags, 4u);
+            }
             at++;
             if (!nlm) mask = 0;
             else {
@@ -634,15 +690,18 @@ __device__ uint32_t emit_lane_nlm(const DbView& db, const uint8_t* __restrict__ 
     return valid;
 }
 
-template <bool WITH_NFA>   // the database holds NFA-fallback patterns: lines with NUL bytes are re-checked with them too (1 KiB of local memory)
+// COUNT_ONLY (the caller wants no records: grep -c, count-only scans): keys for k_count_keys instead of records (see
+// emit_lane_nlm); `recs` is unused and `rec_cap` is the capacity of `keys`.
+template <bool WITH_NFA, bool COUNT_ONLY>   // WITH_NFA: the database holds NFA-fallback patterns: lines with NUL bytes are re-checked with them too (1 KiB of local memory)
 __global__ void __launch_bounds__(kEmitThreads, 6) k_emit_nlm(DbView db, const uint8_t* __restrict__ data, size_t n, const uint32_t* __restrict__ cand,
                                                            const uint32_t* __restrict__ marks, const uint32_t* __restrict__ tile_offsets,
                                                            const unsigned long long* __restrict__ meta, const unsigned long long* __restrict__ prefix,
                                                            const uint32_t* __restrict__ nlmask, const unsigned long long* meta_total, size_t cap,
-                                                           LineRec* __restrict__ recs, size_t rec_cap, Totals* totals) {
+                                                           LineRec* __restrict__ recs, uint32_t* __restrict__ keys, size_t rec_cap, Totals* totals) {
     __shared__ uint32_t q_cand[kEmitQueue], q_at[kEmitQueue];
     __shared__ unsigned long long s_warp[kEmitThreads / 32], s_total;
     const uint32_t nblk = (uint32_t)((n + 511) >> 9);
+    const bool nul_free = COUNT_ONLY && !(totals->flags & kSegmentNulFlag);   // (k_stream tests for NUL bytes in count-only scans only)
     uint32_t valid = 0;
     uint32_t head = 0, queued = 0;   // the same in every thread of the block
     size_t ncand = (size_t)(*meta_total >> 32);
@@ -681,7 +740,8 @@ __global__ void __launch_bounds__(kEmitThreads, 6) k_emit_nlm(DbView db, const u
         __syncthreads();
         while (queued >= (uint32_t)kEmitThreads) {
             const uint32_t k = (head + threadIdx.x) & (kEmitQueue - 1);
-            valid += emit_lane_nlm<WITH_NFA>(db, data, n, cand, marks, meta, prefix, nlmask, nblk, true, q_cand[k], q_at[k], recs, rec_cap, totals);
+            valid += emit_lane_nlm<WITH_NFA, COUNT_ONLY>(db, data, n, cand, marks, meta, prefix, nlmask, nblk, true, q_cand[k], q_at[k], recs, keys, rec_cap,
+                                                                 nul_free, totals);
             head += kEmitThreads;
             queued -= kEmitThreads;
         }
@@ -694,9 +754,10 @@ __global__ void __launch_bounds__(kEmitThreads, 6) k_emit_nlm(DbView db, const u
         const uint32_t j = (threadIdx.x >> 5) + kWarps * (threadIdx.x & 31);
         const uint32_t k = (head + j) & (kEmitQueue - 1);
         const bool live = j < queued;
-        valid += emit_lane_nlm<WITH_NFA>(db, data, n, cand, marks, meta, prefix, nlmask, nblk, live, live ? q_cand[k] : 0, live ? q_at[k] : 0, recs, rec_cap, totals);
+        valid += emit_lane_nlm<WITH_NFA, COUNT_ONLY>(db, data, n, cand, marks, meta, prefix, nlmask, nblk, live, live ? q_cand[k] : 0, live ? q_at[k] : 0,
+                                                             recs, keys, rec_cap, nul_free, totals);
     }
-    (void)valid;   // the unique valid records are counted by k_dedupe_records
+    (void)valid;   // the unique valid records are counted by k_dedupe_records / k_count_keys
 }
 
 // The same line can be marked by several candidate chunks that intersect it.  Their records are ADJACENT in the record
@@ -712,6 +773,20 @@ __global__ void __launch_bounds__(256) k_dedupe_records(LineRec* __restrict__ re
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < nrec; i += (size_t)gridDim.x * blockDim.x) {
         if (i > 0 && recs[i].start == recs[i - 1].start) recs[i].len = kInvalidLen;
         else if (recs[i].len != kInvalidLen) valid++;
+    }
+    valid = __reduce_add_sync(0xffffffffu, valid);
+    if ((threadIdx.x & 31) == 0 && valid) atomicAdd(&totals->aux_total, (unsigned long long)valid);
+}
+
+// Count-only counterpart of k_dedupe_records over the keys of k_emit_nlm<*, true>: the valid keys that differ from their
+// predecessor (the records of one line are adjacent, see above) are the distinct matched lines -> aux_total.
+__global__ void __launch_bounds__(256) k_count_keys(const uint32_t* __restrict__ keys, size_t cap, Totals* totals) {
+    size_t nkeys = (size_t)totals->rec_total;
+    if (nkeys > cap) nkeys = cap;
+    uint32_t valid = 0;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < nkeys; i += (size_t)gridDim.x * blockDim.x) {
+        const uint32_t key = keys[i];
+        if (key != kInvalidLen && (i == 0 || key != keys[i - 1])) valid++;
     }
     valid = __reduce_add_sync(0xffffffffu, valid);
     if ((threadIdx.x & 31) == 0 && valid) atomicAdd(&totals->aux_total, (unsigned long long)valid);

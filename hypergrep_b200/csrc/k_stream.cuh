@@ -12,6 +12,10 @@ namespace gpugrep {
 // STRIDE: sample every STRIDE-th byte position (4, 2, 1).  MODE: 0 no prefilter, 1 exact keys, 2 bloom byte table.
 // Second output: nlmask[block] = ballot(lanes whose 16-byte chunk holds at least one '\n'); the emit kernel finds line
 // extents and line numbers from these words instead of searching the text again.
+// NUL: third output, Totals::flags bit 3 when some byte in [0, n) is NUL.  The count-only emit kernel then needs no line
+// extents and no per-line NUL scans in a segment without one (log text has none).  One sticky register per thread, one
+// vote per warp at the end.  Only count-only scans test: at stride 4 the test costs the kernel 7 % (0.457 -> 0.491 ms per
+// 2 GiB for configs[0], B200), more than the NUL scans it saves a scan with records.
 // Algorithmic traffic: 1 byte read per input byte + 12 bytes written per 512.
 // ------------------------------------------------------------------------------------------------------------
 // Gram lookups of one 16-byte chunk.  MODE 1: two-choice table of exact 32-bit keys; the table is replicated
@@ -90,6 +94,19 @@ __device__ __forceinline__ uint32_t newline_count16_fma(const uint4& v, uint32_t
     return __popcll(acc);
 }
 
+// NUL test of one 16-byte chunk, OR-ed into a sticky word: bit 7 of some byte of acc ends up set iff some word held a zero
+// byte (haszero4 without its final mask).  Per word one subtraction, which ptxas can place on the FMA pipe, and one
+// three-input logic op: the ALU pipe is the one this kernel saturates first.
+__device__ __forceinline__ void nul_accumulate(const uint4& v, uint32_t& acc) {
+    const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+        uint32_t t;
+        asm("mad.lo.u32 %0, %1, 1, 0xfefefeff;" : "=r"(t) : "r"(w[i]));   // w - 0x01010101
+        asm("lop3.b32 %0, %1, %2, %0, 0xBA;" : "+r"(acc) : "r"(t), "r"(w[i]));   // acc | (t & ~w)
+    }
+}
+
 constexpr int kStreamU = 4;   // 512-byte blocks per warp step
 
 // Per-warp constants of the streaming kernel.
@@ -101,10 +118,10 @@ struct StreamRegs {
 // (Tried and dropped, profiles/README.md: a CONFIRM variant in which a lane whose chunk passes the bloom table confirms it
 // right here with the exact tables of confirm.cuh - for the 10,000-pattern set this kernel went from 0.31 to 2.5 ms per GiB:
 // the warp runs the confirmation code, global lookups and all, in nearly every chunk step with a handful of lanes busy.)
-template <int STRIDE, bool FOLD, int MODE, int NODD>
+template <int STRIDE, bool FOLD, int MODE, int NODD, bool NUL>
 __device__ __forceinline__ void stream_group(const uint4 (&v)[kStreamU], uint32_t g0, const uint8_t* __restrict__ data, size_t n,
                                              unsigned long long* __restrict__ meta, uint32_t* __restrict__ nlmask, unsigned long long* __restrict__ gsum,
-                                             const uint32_t* __restrict__ s_tab, const ProbeParams& pp, const StreamRegs& r) {
+                                             const uint32_t* __restrict__ s_tab, const ProbeParams& pp, const StreamRegs& r, uint32_t& nul) {
     constexpr int U = kStreamU;
     const uint32_t lane = r.lane;
     uint32_t after = 0;   // first word after the group (only lane 31 needs it, for grams that straddle the end)
@@ -119,6 +136,7 @@ __device__ __forceinline__ void stream_group(const uint4 (&v)[kStreamU], uint32_
 #pragma unroll
         for (int u = 0; u < U; u++) {
             c[u] = newline_count16_fma(v[u], r.cnl, r.c80);
+            if (NUL) nul_accumulate(v[u], nul);
             nlm[u] = __ballot_sync(0xffffffffu, c[u] != 0u);
             uint32_t nx = 0;
             if (MODE != 0 && (STRIDE < 4 || NODD > 0)) {
@@ -145,10 +163,11 @@ __device__ __forceinline__ void stream_group(const uint4 (&v)[kStreamU], uint32_
     }
 }
 
-template <int STRIDE, bool FOLD, int MODE, int NODD>
+template <int STRIDE, bool FOLD, int MODE, int NODD, bool NUL>
 __global__ void __launch_bounds__(1024) k_stream(const uint8_t* __restrict__ data, size_t n, unsigned long long* __restrict__ meta,
                                                  uint32_t* __restrict__ nlmask, unsigned long long* __restrict__ gsum,
-                                                 const uint32_t* __restrict__ table, int table_words, ProbeParams pp) {
+                                                 const uint32_t* __restrict__ table, int table_words, ProbeParams pp,
+                                                 unsigned int* __restrict__ flags) {
     extern __shared__ __align__(16) uint32_t s_raw[];
     // exact tables are placed at an address aligned to the size of one half (see probe_chunk); the launch reserves the slack
     uint32_t* s_tab = s_raw;
@@ -180,6 +199,7 @@ __global__ void __launch_bounds__(1024) k_stream(const uint8_t* __restrict__ dat
     const uint32_t nblk = (uint32_t)((n + 511) >> 9);
     const uint32_t nfull = (uint32_t)(n >> 9);   // blocks that lie entirely inside [0, n)
     const uint32_t step = nwarps * U;
+    uint32_t nul = 0;   // sticky NUL test (nul_accumulate) of the full blocks
 
     // ---- main loop: groups of U full blocks, no bounds checks on the data loads
     // The loads of the NEXT group are issued before the current group is processed (twice the bytes in flight per warp:
@@ -199,12 +219,13 @@ __global__ void __launch_bounds__(1024) k_stream(const uint8_t* __restrict__ dat
 #pragma unroll
             for (int u = 0; u < U; u++) ahead[u] = ld_stream16(lane_data + ((size_t)g1 << 9) + u * 512);
         }
-        stream_group<STRIDE, FOLD, MODE, NODD>(v, g0, data, n, meta, nlmask, gsum, s_tab, pp, r);
+        stream_group<STRIDE, FOLD, MODE, NODD, NUL>(v, g0, data, n, meta, nlmask, gsum, s_tab, pp, r, nul);
     }
 
     // ---- tail: the last (< U) full blocks and the partial block, one block per warp step, bounds-checked; the totals of
     // that last, partial group are added up by its first warp
     const uint32_t tail0 = (nfull / U) * U;
+    bool tail_nul = false;
     for (uint32_t g = tail0 + warp; g < nblk; g += nwarps) {
         size_t off = ((size_t)g << 9) + (size_t)lane * 16;
         uint4 v = off < n ? ld_chunk(data, off, n) : make_uint4(0, 0, 0, 0);
@@ -219,6 +240,11 @@ __global__ void __launch_bounds__(1024) k_stream(const uint8_t* __restrict__ dat
         uint32_t cnt = newline_count16_fma(v, r.cnl, r.c80);
         bool hit = probe_chunk<STRIDE, FOLD, MODE, NODD>(v, nx, s_tab, pp, r.c1, r.c2);
         if (off >= n) hit = false;   // chunks that start at or beyond n can never be candidates
+        // the zero padding at and beyond n is not text: only the bytes below n count in the NUL test
+        if (NUL) {
+            const uint32_t inside = off >= n ? 0u : (off + 16 > n ? (1u << (uint32_t)(n - off)) - 1u : 0xffffu);
+            tail_nul |= (byte_mask16(v, 0u) & inside) != 0u;
+        }
         uint32_t mask = __ballot_sync(0xffffffffu, hit);
         uint32_t nl = __ballot_sync(0xffffffffu, cnt != 0u);
         uint32_t total = __reduce_add_sync(0xffffffffu, cnt);
@@ -229,6 +255,7 @@ __global__ void __launch_bounds__(1024) k_stream(const uint8_t* __restrict__ dat
             atomicAdd(&gsum[tail0 / U], ((unsigned long long)__popc(mask) << 32) | total);
         }
     }
+    if (NUL && __any_sync(0xffffffffu, (nul & 0x80808080u) != 0u || tail_nul) && lane == 0) atomicOr(flags, kSegmentNulFlag);
 }
 
 }  // namespace gpugrep

@@ -195,7 +195,7 @@ class _Stats(ctypes.Structure):
         ("candidates", ctypes.c_ulonglong), ("h2d_bytes", ctypes.c_ulonglong), ("d2h_bytes", ctypes.c_ulonglong),
         ("gpu_ms", ctypes.c_double), ("stream_kernel_ms", ctypes.c_double), ("wall_ms", ctypes.c_double),
         ("launches", ctypes.c_uint), ("stream_launches", ctypes.c_uint), ("segments", ctypes.c_uint), ("path", ctypes.c_uint),
-        ("split_segments", ctypes.c_uint), ("reserved", ctypes.c_uint),
+        ("split_segments", ctypes.c_uint), ("nul_segments", ctypes.c_uint),
     ]
 
 

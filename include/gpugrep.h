@@ -88,7 +88,7 @@ typedef struct gpugrep_stats {
     unsigned int segments;             /* device segments processed                                        */
     unsigned int path;                 /* bit 0: prefilter fast path used; bit 1: general line-table path used */
     unsigned int split_segments;       /* large segments that hit a fast-path bound and were scanned again in 64 MiB pieces */
-    unsigned int reserved;
+    unsigned int nul_segments;         /* segments with a NUL byte (count-only scans test for them)        */
 } gpugrep_stats;
 
 #define GPUGREP_LOC_HOST 0   /* data is host memory (pinned memory is copied directly, pageable is staged) */
