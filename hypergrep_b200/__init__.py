@@ -5,6 +5,7 @@ functions, constants and ctypes types, backed by ``lib/libgpugrep.so`` instead o
 """
 
 from hypergrep_b200.utils import CALLBACK_TYPE
+from hypergrep_b200.utils import CONTEXT_ID
 from hypergrep_b200.utils import HS_FLAG_CASELESS
 from hypergrep_b200.utils import HS_FLAG_DOTALL
 from hypergrep_b200.utils import HS_FLAG_MULTILINE
@@ -20,6 +21,7 @@ from hypergrep_b200.utils import scan
 __version__ = "0.1.0"
 __all__ = [
     "CALLBACK_TYPE",
+    "CONTEXT_ID",
     "HS_FLAG_CASELESS",
     "HS_FLAG_DOTALL",
     "HS_FLAG_MULTILINE",

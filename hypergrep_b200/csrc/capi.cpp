@@ -17,6 +17,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <condition_variable>
+#include <deque>
 #include <functional>
 #include <list>
 #include <mutex>
@@ -113,16 +114,13 @@ public:
     // collecting deliverer of a shard worker: results are stored, not called back
     explicit Deliverer(ShardResults* collect) : cb_(nullptr), cap_(1), collect_(collect) {}
     // `bytes`/`len`: the pseudo-line as it sits in the file.  The delivered text is what the reference strcpy()s:
-    // leading NULs skipped, cut at the next NUL (hyperscanner.c:205-214, :92).
-    void emit(unsigned id, unsigned long long line_number, const uint8_t* bytes, size_t len, bool may_have_nul = true) {
-        count_++;
+    // leading NULs skipped, cut at the next NUL (hyperscanner.c:205-214, :92).  `counted`: false for context lines, which
+    // count() leaves out.
+    void emit(unsigned id, unsigned long long line_number, const uint8_t* bytes, size_t len, bool may_have_nul = true, bool counted = true) {
+        if (counted) count_++;
         if (!cb_ && !collect_) return;
         size_t a = 0, b = len;
-        if (may_have_nul) {
-            while (a < len && bytes[a] == 0) a++;
-            const void* z = std::memchr(bytes + a, 0, len - a);
-            if (z) b = (size_t)((const uint8_t*)z - bytes);
-        }
+        if (may_have_nul) strip(bytes, len, a, b);
         if (collect_) {
             collect_->records.push_back(ShardRecord{id, line_number, collect_->text.size()});
             collect_->text.insert(collect_->text.end(), (const char*)bytes + a, (const char*)bytes + b);
@@ -159,6 +157,14 @@ public:
     void emit_text(unsigned id, unsigned long long line_number, const char* text) {
         emit(id, line_number, (const uint8_t*)text, std::strlen(text), false);
     }
+    // the delivered text of a pseudo-line is [a, b)
+    static void strip(const uint8_t* bytes, size_t len, size_t& a, size_t& b) {
+        a = 0;
+        b = len;
+        while (a < len && bytes[a] == 0) a++;
+        const void* z = std::memchr(bytes + a, 0, len - a);
+        if (z) b = (size_t)((const uint8_t*)z - bytes);
+    }
 private:
     static constexpr size_t kBlock = (size_t)1 << 20;
     char* place(size_t bytes) {
@@ -180,6 +186,60 @@ private:
     std::vector<hyperscanner_result_t> results_;
     std::vector<std::vector<char>> blocks_;
     size_t block_ = 0, used_ = 0;
+};
+
+// Context lines (grep -A/-B/-C) on the delivering thread.  It is fed, in file order, the selected lines and the context
+// candidates of the engine: a superset of the context lines (the output lines of each segment and the segment's edge
+// lines, see slot_set_context).  It delivers each output line once, selected lines with id 0 and context lines with
+// GPUGREP_CONTEXT_ID.  It applies max_match_count to the selected lines; after the line that reaches the limit, the next
+// `after` lines still go out, all as context.  `tag_only` (the shard workers of a scan over several GPUs): every record is
+// passed on, tagged, for the merge to filter; only the limit applies.
+class ContextFilter {
+public:
+    ContextFilter(Deliverer* out, uint32_t before, uint32_t after, unsigned long long max_match, bool tag_only)
+        : out_(out), before_(before), after_(after), max_(max_match), tag_only_(tag_only) {}
+    // false: the limit has been reached and `line` lies past the trailing context: nothing more will be delivered
+    bool feed(bool selected, unsigned long long line, const uint8_t* bytes, size_t len, bool may_have_nul) {
+        if (limit_reached()) {
+            if (line - last_ > after_) return false;
+            out_->emit(GPUGREP_CONTEXT_ID, line, bytes, len, may_have_nul, false);
+            return true;
+        }
+        if (selected) {
+            for (const Held& h : held_)
+                if (line - h.line <= before_) out_->emit(GPUGREP_CONTEXT_ID, h.line, (const uint8_t*)h.text.data(), h.text.size(), false, false);
+            held_.clear();
+            out_->emit(0, line, bytes, len, may_have_nul);
+            last_ = line;
+            any_ = true;
+            selected_++;
+        } else if (tag_only_ || (any_ && line - last_ <= after_)) {
+            out_->emit(GPUGREP_CONTEXT_ID, line, bytes, len, may_have_nul, false);
+        } else if (before_) {
+            // held until a selected line within `before` lines follows; at most `before` lines can be wanted
+            size_t a = 0, b = len;
+            if (may_have_nul) Deliverer::strip(bytes, len, a, b);
+            held_.push_back(Held{line, std::string((const char*)bytes + a, b - a)});
+            if (held_.size() > before_) held_.pop_front();
+        }
+        return true;
+    }
+    // the limit has been reached and every line from `next_line` on lies past the trailing context
+    bool finished(unsigned long long next_line) const { return limit_reached() && next_line - last_ > after_; }
+
+private:
+    bool limit_reached() const { return max_ > 0 && selected_ >= max_; }
+    struct Held {
+        unsigned long long line;
+        std::string text;   // stripped
+    };
+    Deliverer* out_;
+    uint32_t before_, after_;
+    unsigned long long max_;
+    bool tag_only_;
+    bool any_ = false;
+    unsigned long long last_ = 0, selected_ = 0;
+    std::deque<Held> held_;
 };
 
 constexpr size_t kSampleBytes = 512 << 10;   // head of the input used to tune the prefilter windows
@@ -261,6 +321,7 @@ struct Job {
     int buffer_size = 0;
     unsigned long long max_match = 0;
     Deliverer* out = nullptr;
+    ContextFilter* context = nullptr;   // scans with context lines: every record goes through it (it applies max_match)
     unsigned long long line_base = 0;
     bool stop = false;
     gpugrep_stats stats{};
@@ -340,7 +401,7 @@ struct Job {
             }
         }
         size_t take = count;
-        if (max_match > 0) {
+        if (max_match > 0 && !context) {
             unsigned long long room = max_match > out->count() ? max_match - out->count() : 0;
             if ((unsigned long long)take >= room) { take = (size_t)room; stop = true; }
         }
@@ -365,8 +426,16 @@ struct Job {
                 __builtin_prefetch(ahead + 128);
             }
             const uint8_t* bytes = host ? host + lr.start : gathered.data() + goff[i];
-            out->emit(db->simple_id, line_base + lr.line, bytes, lr.len & kLineLenMask, fast_rec ? (lr.len & kLineHasNul) != 0 : true);
+            const bool may_have_nul = fast_rec ? (lr.len & kLineHasNul) != 0 : true;
+            if (!context) {
+                out->emit(db->simple_id, line_base + lr.line, bytes, lr.len & kLineLenMask, may_have_nul);
+            } else if (!context->feed((lr.len & kLineContext) == 0, line_base + lr.line, bytes, lr.len & kLineLenMask, may_have_nul)) {
+                stop = true;
+                break;
+            }
         }
+        // the reader goes on past the limit while trailing context is owed
+        if (context && context->finished(line_base + r.num_lines)) stop = true;
         return 0;
     }
 
@@ -440,6 +509,10 @@ struct Params {
     void* user_stream;
     EndsSink* ends = nullptr;   // gpugrep_match_ends(): end offsets instead of lines
     bool invert = false;        // gpugrep_invert_scan_*(): deliver the pseudo-lines in which no pattern reports
+    bool context_scan = false;  // gpugrep_context_scan_*(): lines around the selected ones too
+    uint32_t before = 0, after = 0;
+    // the context stage runs only when lines are delivered (count-only scans ignore context)
+    bool context() const { return context_scan && cb != nullptr && (before || after); }
 };
 
 // Largest prefix of [p, p+have) that ends on a pseudo-line boundary; 0 if none exists yet.
@@ -458,11 +531,14 @@ size_t cut_point(const uint8_t* p, size_t have, bool final, size_t limit) {
 void set_invert(ScanSlot* slot, bool invert) {
     if (slot_set_invert) slot_set_invert(slot, invert);
 }
+void set_context(ScanSlot* slot, const Params& pr) {
+    if (slot_set_context) slot_set_context(slot, pr.context() ? pr.before : 0u, pr.context() ? pr.after : 0u);
+}
 
 int setup_job(const Params& pr, Job& job, Deliverer& out, unsigned long long weight = 0) {
     int rc = 0;
     job.db = cached_database(pr.patterns, pr.flags, pr.ids, pr.elements, rc, job.error);
-    if (job.db && pr.invert) {
+    if (job.db && (pr.invert || pr.context_scan)) {
         // Which lines match does not depend on ids or SINGLEMATCH: once the set compiles as given, it is scanned as "every
         // pattern SINGLEMATCH, one id 0" (simple mode, so multi-id sets take the fast path too), CASELESS/DOTALL/MULTILINE kept.
         std::vector<unsigned> flags(pr.elements), ids(pr.elements, 0u);
@@ -475,6 +551,7 @@ int setup_job(const Params& pr, Job& job, Deliverer& out, unsigned long long wei
     }
     if (pr.buffer_size < 2) { job.error = "buffer_size must be at least 2"; return GPUGREP_SCAN; }
     if (pr.invert && !slot_set_invert) { job.error = "this build of the engine has no inverted scan"; return GPUGREP_SCAN; }
+    if (pr.context_scan && !slot_set_context) { job.error = "this build of the engine has no context lines"; return GPUGREP_SCAN; }
     job.device_weight = weight;
     job.device = pick_device(weight, &job.device_charged);
     if (engine_select_device(job.device, job.error) != 0) {
@@ -536,6 +613,8 @@ int scan_file(const char* path, const Params& pr, gpugrep_stats* stats_out, cons
     }
     int rc = setup_job(pr, job, out, weight);
     if (rc) { set_last_error(job.error); return rc; }
+    ContextFilter context(&out, pr.before, pr.after, pr.max_match, shard != nullptr);
+    if (pr.context()) job.context = &context;
     std::string err;
     auto src = shard ? open_plain_range(path, shard->begin, shard->end, err) : open_byte_source(path, err);
     if (!src) { set_last_error(err); return GPUGREP_GZ_OPEN; }
@@ -583,6 +662,7 @@ int scan_file(const char* path, const Params& pr, gpugrep_stats* stats_out, cons
     for (ScanSlot* sl : slots) {
         slot_set_want_records(sl, !count_only);
         set_invert(sl, pr.invert);
+        set_context(sl, pr);
     }
     SegmentQueue q;
     for (int i = 0; i < kSlots; i++) q.free_slots.push_back(i);
@@ -730,6 +810,8 @@ int scan_memory(const uint8_t* data, size_t size, int location, const Params& pr
     Job job;
     int rc = setup_job(pr, job, out, size);
     if (rc) { set_last_error(job.error); return rc; }
+    ContextFilter context(&out, pr.before, pr.after, pr.max_match, shard != nullptr);
+    if (pr.context()) job.context = &context;
     std::string err;
     const size_t limit = clamp_limit(pr.buffer_size);
     const bool on_device = location == GPUGREP_LOC_DEVICE;
@@ -748,6 +830,7 @@ int scan_memory(const uint8_t* data, size_t size, int location, const Params& pr
     for (ScanSlot* sl : slots) {
         slot_set_want_records(sl, !count_only);
         set_invert(sl, pr.invert);
+        set_context(sl, pr);
     }
     const uint8_t* seg_host[2] = {nullptr, nullptr};
     const uint8_t* seg_dev[2] = {nullptr, nullptr};
@@ -969,11 +1052,21 @@ int scan_sharded(const std::vector<int>& devices, const std::vector<size_t>& bou
     }
     // ordered merge on the calling thread
     Deliverer out(pr.cb, effective_batch(pr));
+    // context lines: the shards pass on every candidate (id GPUGREP_CONTEXT_ID), and the merge filters them, so that a
+    // window may reach across a shard boundary
+    ContextFilter context(&out, pr.before, pr.after, pr.max_match, false);
     unsigned long long line_base = 0;
     bool stop = false;
     for (size_t g = 0; g < G && !stop; g++) {
         if (count_only) {
             out.emit_count_only(stats[g].matches);
+        } else if (pr.context()) {
+            const auto& recs = results[g].records;
+            for (size_t i = 0; i < recs.size() && !stop; i++) {
+                const char* text = results[g].text.data() + recs[i].offset;
+                stop = !context.feed(recs[i].id != GPUGREP_CONTEXT_ID, line_base + recs[i].line, (const uint8_t*)text, std::strlen(text), false);
+            }
+            if (context.finished(line_base + stats[g].lines)) stop = true;
         } else {
             const auto& recs = results[g].records;
             for (size_t i = 0; i < recs.size() && !stop;) {
@@ -1100,6 +1193,29 @@ int gpugrep_invert_scan_buffer(const void* data, size_t size, int location, cons
                                unsigned long long max_match_count, void* stream, gpugrep_stats* stats) {
     gpugrep::Params pr{patterns, pattern_flags, pattern_ids, elements, on_event, buffer_size, buffer_count, max_match_count, stream};
     pr.invert = true;
+    return gpugrep::scan_buffer(data, size, location, pr, stats);
+}
+
+int gpugrep_context_scan_file(const char* file_name, const char* const* patterns, const unsigned int* pattern_flags, const unsigned int* pattern_ids,
+                              unsigned int elements, hs_event on_event, int buffer_size, int buffer_count, unsigned long long max_match_count,
+                              unsigned int before, unsigned int after, int invert, gpugrep_stats* stats) {
+    gpugrep::Params pr{patterns, pattern_flags, pattern_ids, elements, on_event, buffer_size, buffer_count, max_match_count, nullptr};
+    pr.invert = invert != 0;
+    pr.context_scan = true;
+    pr.before = before;
+    pr.after = after;
+    return gpugrep::scan_path(file_name, pr, stats);
+}
+
+int gpugrep_context_scan_buffer(const void* data, size_t size, int location, const char* const* patterns, const unsigned int* pattern_flags,
+                                const unsigned int* pattern_ids, unsigned int elements, hs_event on_event, int buffer_size, int buffer_count,
+                                unsigned long long max_match_count, unsigned int before, unsigned int after, int invert, void* stream,
+                                gpugrep_stats* stats) {
+    gpugrep::Params pr{patterns, pattern_flags, pattern_ids, elements, on_event, buffer_size, buffer_count, max_match_count, stream};
+    pr.invert = invert != 0;
+    pr.context_scan = true;
+    pr.before = before;
+    pr.after = after;
     return gpugrep::scan_buffer(data, size, location, pr, stats);
 }
 

@@ -11,6 +11,8 @@
 //           k_stream(no filter) -> scan -> k_newline_positions -> pseudo-line table -> k_match_pl_* -> scan -> emit
 // INVERTED scans (grep -v) select the lines without a match: the fast path adds a complement stage after the dedupe
 // (k_invert.cuh, run from slot_collect), the general path negates the per-line flags of k_match_pl_simple.
+// CONTEXT lines (grep -A/-B/-C, scans with records): a window test over the prefix count of the selected lines picks the
+// output lines of a segment (k_context.cuh, after the dedupe on the fast path, after k_match_pl_simple on the general path).
 // All byte offsets inside a segment are 32-bit (segments are < 4 GiB); line numbers are rebased on the host.
 // Device code lives in the .cuh files included below (one translation unit); this file holds the host side: device
 // tables, scan slots, the launch sequence of a segment and the collection of its results.
@@ -37,6 +39,7 @@
 #include "k_fast.cuh"
 #include "k_general.cuh"
 #include "k_invert.cuh"
+#include "k_context.cuh"
 
 namespace gpugrep {
 
@@ -146,7 +149,8 @@ public:
     cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};   // 0/1: whole segment, 2/3: streaming kernel
     DevBuf d_input, d_meta, d_nlmask, d_gsum, d_prefix, d_sums, d_cand, d_res, d_recoff, d_recs, d_totals;
     DevBuf d_nlpos, d_npl, d_ploff, d_plstart, d_pllen, d_flags, d_counts, d_events, d_gather, d_gidx, d_hitinfo, d_survivors;
-    DevBuf d_linebits, d_invrecs;   // inverted fast path: matched-line bitmap, selected-line records
+    DevBuf d_linebits, d_invrecs;   // inverted fast path: matched-line bitmap, selected-line records (context lines: output records)
+    DevBuf d_outbits, d_outoff;     // context lines: output-line bitmap (general path: flags) and its prefix
     PinBuf h_totals, h_recs, h_stage, h_gather, h_probe;
     // state of the in-flight segment
     const DeviceDb* ddb = nullptr;
@@ -156,11 +160,14 @@ public:
     bool fast = false;
     bool want_records = true;   // false: the caller only counts matches (no callback, no limit): the fast path counts without records
     bool invert = false;        // deliver the lines without a match (slot_set_invert)
+    uint32_t ctx_before = 0, ctx_after = 0;   // context lines (slot_set_context)
     SegmentStats stats;
     bool in_use = false;
 
     int run_general(SegmentResult& out, std::string& error);
     int run_complement(size_t nrec, size_t nlines, size_t selected, std::string& error);
+    int run_context(size_t nrec, size_t nlines, size_t selected, size_t& count, std::string& error);
+    bool context() const { return want_records && (ctx_before || ctx_after); }
 };
 
 int engine_select_device(int device, std::string& error) {
@@ -449,6 +456,10 @@ void engine_release_slot(ScanSlot* slot) {
 
 void slot_set_want_records(ScanSlot* slot, bool want) { slot->want_records = want; }
 void slot_set_invert(ScanSlot* slot, bool invert) { slot->invert = invert; }
+void slot_set_context(ScanSlot* slot, uint32_t before, uint32_t after) {
+    slot->ctx_before = before;
+    slot->ctx_after = after;
+}
 
 uint8_t* slot_host_buffer(ScanSlot* slot, size_t capacity, std::string& error) {
     if (slot->h_stage.reserve(capacity + 64) != cudaSuccess) { error = "cudaHostAlloc failed for the staging buffer"; return nullptr; }
@@ -759,14 +770,28 @@ int ScanSlot::run_general(SegmentResult& out, std::string& error) {
         k_match_pl_simple<<<mgrid, 128, 0, st>>>(view, data, d_plstart.as<uint32_t>(), d_pllen.as<uint32_t>(), npl_total, d_flags.as<uint8_t>(), invert);
         stats.launches++;
         launch_scan(st, LoadU8{d_flags.as<uint8_t>()}, npl_total, d_recoff.as<unsigned long long>(), d_sums.as<unsigned long long>(), &dT->rec_total, stats);
+        // context lines: the output flags from the window test over the prefix of the selected flags, and their prefix
+        const bool ctx = context();
+        if (ctx) {
+            if (d_outbits.reserve(npl_total) != cudaSuccess || d_outoff.reserve(npl_total * 8) != cudaSuccess) { error = "cudaMalloc failed"; return 3; }
+            k_context_flags<<<(unsigned)((npl_total + 255) / 256), 256, 0, st>>>(d_recoff.as<unsigned long long>(), &dT->rec_total, npl_total, ctx_before,
+                                                                                   ctx_after, d_outbits.as<uint8_t>());
+            stats.launches++;
+            launch_scan(st, LoadU8{d_outbits.as<uint8_t>()}, npl_total, d_outoff.as<unsigned long long>(), d_sums.as<unsigned long long>(), &dT->aux_total, stats);
+        }
         CUDA_TRY(cudaMemcpyAsync(hT, dT, sizeof(Totals), cudaMemcpyDeviceToHost, st));
         CUDA_TRY(cudaStreamSynchronize(st));
-        size_t nrec = (size_t)hT->rec_total;
+        size_t nrec = (size_t)(ctx ? hT->aux_total : hT->rec_total);
         if (nrec) {
             if (d_recs.reserve(nrec * sizeof(LineRec)) != cudaSuccess) { error = "cudaMalloc failed"; return 3; }
             if (h_recs.reserve(nrec * sizeof(LineRec)) != cudaSuccess) { error = "cudaHostAlloc failed"; return 3; }
-            k_emit_pl_simple<<<(unsigned)((npl_total + 255) / 256), 256, 0, st>>>(d_plstart.as<uint32_t>(), d_pllen.as<uint32_t>(), npl_total,
-                                                                                    d_flags.as<uint8_t>(), d_recoff.as<unsigned long long>(), d_recs.as<LineRec>());
+            if (ctx)
+                k_emit_pl_context<<<(unsigned)((npl_total + 255) / 256), 256, 0, st>>>(d_plstart.as<uint32_t>(), d_pllen.as<uint32_t>(), npl_total,
+                                                                                         d_flags.as<uint8_t>(), d_outbits.as<uint8_t>(),
+                                                                                         d_outoff.as<unsigned long long>(), d_recs.as<LineRec>());
+            else
+                k_emit_pl_simple<<<(unsigned)((npl_total + 255) / 256), 256, 0, st>>>(d_plstart.as<uint32_t>(), d_pllen.as<uint32_t>(), npl_total,
+                                                                                        d_flags.as<uint8_t>(), d_recoff.as<unsigned long long>(), d_recs.as<LineRec>());
             stats.launches++;
             CUDA_TRY(cudaEventRecord(ev[1], st));
             CUDA_TRY(cudaMemcpyAsync(h_recs.p, d_recs.p, nrec * sizeof(LineRec), cudaMemcpyDeviceToHost, st));
@@ -841,6 +866,54 @@ int ScanSlot::run_complement(size_t nrec, size_t nlines, size_t selected, std::s
     return 0;
 }
 
+// Fast path with context lines: the `count` output records of the segment (k_context.cuh), in line order, copied to h_recs.
+// `selected`: lines selected (valid records, or with invert the lines without one).  The output count is only known on
+// the device; the buffers are sized from a bound on it (every selected line outputs at most A+B+1 lines, the edges at
+// most A+B more, and no segment more than its lines), so that the stage needs one synchronisation, like run_complement.
+int ScanSlot::run_context(size_t nrec, size_t nlines, size_t selected, size_t& count, std::string& error) {
+    cudaStream_t st = stream;
+    Totals* dT = d_totals.as<Totals>();
+    Totals* hT = h_totals.as<Totals>();
+    const size_t nl_total = (size_t)(uint32_t)hT->meta_total;
+    const size_t nwords = (nlines + 31) / 32;
+    const size_t nb_scan = (nwords + kScanTile - 1) / kScanTile + 1;
+    const unsigned __int128 window = (unsigned __int128)ctx_before + ctx_after + 1;
+    const unsigned __int128 edges = (unsigned __int128)std::min<size_t>(ctx_before, nlines) + std::min<size_t>(ctx_after, nlines);
+    const size_t bound = (size_t)std::min<unsigned __int128>(nlines, window * selected + edges);
+    if (d_linebits.reserve(nwords * 4) != cudaSuccess || d_outbits.reserve(nwords * 4) != cudaSuccess || d_recoff.reserve(nwords * 8) != cudaSuccess ||
+        d_outoff.reserve(nwords * 8) != cudaSuccess || d_sums.reserve(nb_scan * 8) != cudaSuccess || d_nlpos.reserve((nl_total + 1) * 4) != cudaSuccess ||
+        d_invrecs.reserve(bound * sizeof(LineRec)) != cudaSuccess) {
+        error = "cudaMalloc failed for the context lines of a scan"; return 3;
+    }
+    if (h_recs.reserve(bound * sizeof(LineRec)) != cudaSuccess) { error = "cudaHostAlloc failed"; return 3; }
+    uint32_t* bits = d_linebits.as<uint32_t>();
+    uint32_t* out_bits = d_outbits.as<uint32_t>();
+    CUDA_TRY(cudaMemsetAsync(bits, 0, nwords * 4, st));
+    const unsigned sms = (unsigned)device_sms();
+    if (nrec) {
+        k_mark_lines<<<(unsigned)std::min<size_t>((nrec + 255) / 256, (size_t)sms * 8), 256, 0, st>>>(d_recs.as<LineRec>(), nrec, bits);
+        stats.launches++;
+    }
+    launch_scan(st, LoadSelectedPopc{bits, nlines, invert}, nwords, d_recoff.as<unsigned long long>(), d_sums.as<unsigned long long>(), &dT->rec_total, stats);
+    const unsigned line_grid = (unsigned)((nwords * 32 + 255) / 256);
+    k_context_bits<<<line_grid, 256, 0, st>>>(bits, nlines, invert, d_recoff.as<unsigned long long>(), &dT->rec_total, ctx_before, ctx_after, out_bits);
+    launch_scan(st, LoadPopc{out_bits}, nwords, d_outoff.as<unsigned long long>(), d_sums.as<unsigned long long>(), &dT->aux_total, stats);
+    k_newline_positions<<<(unsigned)((nblk * 32 + 255) / 256), 256, 0, st>>>(data, n, nblk, d_meta.as<unsigned long long>(), d_prefix.as<unsigned long long>(),
+                                                                           d_nlpos.as<uint32_t>(), d_nlmask.as<uint32_t>());
+    k_emit_context<<<line_grid, 256, 0, st>>>(d_nlpos.as<uint32_t>(), nl_total, n, nlines, bits, invert, out_bits, d_outoff.as<unsigned long long>(),
+                                              d_invrecs.as<LineRec>());
+    stats.launches += 3;
+    CUDA_TRY(cudaEventRecord(ev[1], st));
+    CUDA_TRY(cudaMemcpyAsync(&hT->aux_total, &dT->aux_total, sizeof(hT->aux_total), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(h_recs.p, d_invrecs.p, bound * sizeof(LineRec), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaGetLastError());
+    count = (size_t)hT->aux_total;
+    if (count > bound) { error = "context lines: more output lines than the bound allows"; return 7; }
+    stats.d2h_bytes += bound * sizeof(LineRec) + sizeof(hT->aux_total);
+    return 0;
+}
+
 int slot_collect(ScanSlot* s, SegmentResult& out, std::string& error, size_t split_above) {
     cudaStream_t st = s->stream;
     out = SegmentResult();
@@ -859,7 +932,14 @@ int slot_collect(ScanSlot* s, SegmentResult& out, std::string& error, size_t spl
             out.num_valid_recs = (size_t)hT->aux_total;
             const size_t nl_total = (size_t)(uint32_t)hT->meta_total;
             out.num_lines = nl_total + ((hT->last_byte & 0xff) != '\n' ? 1 : 0);
-            if (s->invert) {
+            if (s->context()) {
+                const size_t selected = s->invert ? (size_t)out.num_lines - out.num_valid_recs : out.num_valid_recs;
+                size_t count = 0;
+                int rc = s->run_context(nrec, (size_t)out.num_lines, selected, count, error);
+                if (rc) return rc;
+                nrec = count;
+                out.num_valid_recs = count;
+            } else if (s->invert) {
                 // the valid records are the matched lines, one each: the complement has lines - valid records
                 const size_t selected = (size_t)out.num_lines - out.num_valid_recs;
                 if (selected && s->want_records) {

@@ -16,10 +16,13 @@ namespace gpugrep {
 struct LineRec {
     uint32_t line;    // pseudo-line index inside the segment
     uint32_t start;   // byte offset of the pseudo-line inside the segment
-    uint32_t len;     // bytes, trailing '\n' included when present; bit 31 (fast path only): the line contains NUL bytes
+    uint32_t len;     // bytes, trailing '\n' included when present; bit 31 (fast path only): the line contains NUL bytes;
+                      // bit 30 (scans with context lines): an output line that is not selected
 };
-constexpr uint32_t kLineLenMask = 0x7fffffffu;
+// (fast-path lines are shorter than 128 KiB and pseudo-lines at most 2^29 bytes: bit 30 is free)
+constexpr uint32_t kLineLenMask = 0x3fffffffu;
 constexpr uint32_t kLineHasNul = 0x80000000u;
+constexpr uint32_t kLineContext = 0x40000000u;
 constexpr uint32_t kLineInvalid = 0xffffffffu;   // fast path: repeat of a line already reported, or a failed NUL re-check
 
 // One automaton report (general mode): some accept set fired at `end` inside pseudo-line `line`.
@@ -87,6 +90,13 @@ void slot_set_want_records(ScanSlot* slot, bool want);
 // Weak: a build of the host logic against a CPU stand-in of this engine that lacks inverted scans still links; the boundary
 // then fails inverted scans with 7 (there is no host-side complement).  engine.cu always defines it.
 __attribute__((weak)) void slot_set_invert(ScanSlot* slot, bool invert);
+// Context lines (grep -A/-B/-C), for scans that want records: the segment's results are, in line order, every output line
+// whose selected line (matched, or with invert unmatched) lies in the segment - within `after` lines after or `before`
+// lines before it - plus the segment's first `after` and last `before` lines, the candidates for the selected lines of
+// the neighbouring segments.  Records of lines that are not selected carry kLineContext; every record is valid.
+// before == after == 0: no context stage.  Call before slot_submit.  Weak like slot_set_invert (a build without it fails
+// context scans with 7).
+__attribute__((weak)) void slot_set_context(ScanSlot* slot, uint32_t before, uint32_t after);
 // Wait for the segment and expose its results (valid until the next slot_submit on this slot).
 // Returns kSplitSegment (and no results) when the fast path hit one of its capacity bounds - a line too long for it, a
 // candidate or record overflow - in a segment of more than `split_above` bytes: the caller then scans the same bytes again

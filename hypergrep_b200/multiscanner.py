@@ -85,6 +85,7 @@ class _OrderedPrinter:  # pylint: disable=too-many-instance-attributes
         self.total = 0
         self.matched = False
         self.errored = False
+        self.printed = False   # some line has been printed (a group separator goes before the next group)
 
     def __call__(self, tagged: tuple[int, Any]) -> None:
         index, outcome = tagged
@@ -125,7 +126,11 @@ class _OrderedPrinter:  # pylint: disable=too-many-instance-attributes
             print(f"{name}:{found}" if opt["with_file_name"] else f"{found}")
         else:
             try:
-                print_results(found, name, with_file_name=opt["with_file_name"], with_line_number=opt["with_line_number"])
+                if opt["context"]:
+                    self.printed = print_context_results(found, name, opt["with_file_name"], opt["with_line_number"], opt["group_separator"],
+                                                         opt["group_span"], self.printed)
+                else:
+                    print_results(found, name, with_file_name=opt["with_file_name"], with_line_number=opt["with_line_number"])
             except BrokenPipeError:
                 pass  # e.g. piped into `head`; keep draining the pool
         self._advance()
@@ -148,11 +153,19 @@ def parallel_grep(  # pylint: disable=too-many-arguments,too-many-locals
     files_with_matches: bool = False,
     quiet: bool = False,
     invert_match: bool = False,
+    before_context: int | None = None,
+    after_context: int | None = None,
+    group_separator: str | None = "--",
 ) -> int:
     """Scan files and print grep-formatted results (reference multiscanner.py:86-223).
 
     Returns the grep exit code: 2 if any file errored, else 1 if nothing matched, else 0.
     ``invert_match`` (``-v``) selects the lines that no pattern matches; every other option then applies to those lines.
+    ``before_context`` / ``after_context`` (``-B`` / ``-A``) print the lines around each selected line, as GNU grep does,
+    with ``group_separator`` (None: none) before each group that does not continue the previous output; as in GNU grep, a
+    width of 0 still separates the groups, and None (the default) prints no context output at all.  -c, -t, -l, -L and
+    -q ignore them; with -o only the matched parts are printed, and a separator goes between two selected lines whose gap
+    exceeds ``before_context + after_context`` lines.
     """
     if invert_match and only_matching:
         # GNU grep -v -o: a selected line has no matching part, so nothing is printed; the exit code still says whether
@@ -162,6 +175,10 @@ def parallel_grep(  # pylint: disable=too-many-arguments,too-many-locals
             quiet = True
     if files_without_match or files_with_matches or quiet:
         max_match_count = 1  # these modes only need to know whether a file matches at all
+    context = before_context is not None or after_context is not None
+    if count_results or total_results or files_without_match or files_with_matches or quiet:
+        context = False
+    before_context, after_context = (before_context or 0, after_context or 0) if context else (0, 0)
     printer = _OrderedPrinter(
         files,
         {
@@ -173,6 +190,10 @@ def parallel_grep(  # pylint: disable=too-many-arguments,too-many-locals
             "files_without_match": files_without_match,
             "files_with_matches": files_with_matches,
             "quiet": quiet,
+            "context": context,
+            "group_separator": group_separator,
+            # printed lines continue a group when they are adjacent; with -o, selected lines whose windows touch
+            "group_span": before_context + after_context + 1 if only_matching else 1,
         },
     )
     grep_kwargs = {
@@ -182,6 +203,9 @@ def parallel_grep(  # pylint: disable=too-many-arguments,too-many-locals
         "no_messages": no_messages,
         "max_match_count": max_match_count,
         "invert_match": invert_match,
+        # (-o prints matched parts only: the grouping of the selected lines is all the printer needs)
+        "before_context": 0 if only_matching else before_context,
+        "after_context": 0 if only_matching else after_context,
     }
     workers = min(max(multiprocessing.cpu_count() - 1, 1), len(files))
     pool_type = ThreadPool if use_multithreading else multiprocessing.Pool
@@ -209,6 +233,26 @@ def print_results(results: list, file_name: str, with_file_name: bool = False, w
         sys.stdout.write("".join(f"{prefix}{number}:{text}" for number, text in results))
     else:
         sys.stdout.write("".join(f"{prefix}{text}" for _, text in results))
+
+
+def print_context_results(  # pylint: disable=too-many-arguments
+    results: list, file_name: str, with_file_name: bool, with_line_number: bool, separator: str | None, span: int, printed: bool
+) -> bool:
+    """Print the results of a scan with context lines as GNU grep does: selected lines as ``name:12:text``, context lines as
+    ``name-12-text``, and ``separator`` before each group that does not continue the previous output (``printed``: some
+    line has been printed before, by any file).  A result continues the group when its line number is at most ``span``
+    after the previous one.  ``results``: ``(number, text, is_context)``, or ``(number, part)`` with -o.  Returns ``printed``."""
+    out = []
+    previous = None
+    for entry in results:
+        number, text = entry[0], entry[1]
+        mark = "-" if len(entry) > 2 and entry[2] else ":"
+        if (previous is None or number - previous > span) and printed and separator is not None:
+            out.append(f"{separator}\n")
+        previous, printed = number, True
+        out.append((f"{file_name}{mark}" if with_file_name else "") + (f"{number}{mark}" if with_line_number else "") + text)
+    sys.stdout.write("".join(out))
+    return printed
 
 
 def read_stdin() -> Iterator[str]:
@@ -323,6 +367,18 @@ def parse_args(args: list | None = None) -> argparse.Namespace:
     selection.add_argument("-a", "--text", action="store_true",
                            help="Accepted for grep compatibility; files are always processed as bytes.")
 
+    context = parser.add_argument_group("Context Line Control")
+    context.add_argument("-A", "--after-context", type=int, metavar="NUM", default=None,
+                         help="Print NUM lines of trailing context after matching lines.")
+    context.add_argument("-B", "--before-context", type=int, metavar="NUM", default=None,
+                         help="Print NUM lines of leading context before matching lines.")
+    context.add_argument("-C", "--context", type=int, metavar="NUM", default=None,
+                         help="Print NUM lines of output context (-A and -B take precedence).")
+    context.add_argument("--group-separator", metavar="SEP", default="--",
+                         help="Print SEP on a line between groups of context lines (default: --).")
+    context.add_argument("--no-group-separator", dest="group_separator", action="store_const", const=None,
+                         help="Do not print a separator between groups of context lines.")
+
     extra = parser.add_argument_group("Unique arguments to hyperscanner")
     extra.add_argument("-t", "--total", action="store_true",
                        help="Suppress normal output; print a count of matching lines across all input files.")
@@ -358,6 +414,14 @@ def main() -> None:
         raise SystemExit(2) from error
     if args.gnu_regexp and args.regexp != "pcre":
         patterns = to_gnu_regular_expressions(patterns)
+    after_context = args.after_context if args.after_context is not None else args.context
+    before_context = args.before_context if args.before_context is not None else args.context
+    if after_context is not None or before_context is not None:   # (one given: the other is 0)
+        after_context, before_context = after_context or 0, before_context or 0
+    for value in (args.after_context, args.before_context, args.context):
+        if value is not None and value < 0:
+            print(f"hyperscanner: {value}: invalid context length argument")
+            raise SystemExit(2)
 
     files = get_argparse_files(args) or list(read_stdin())
     if args.sort_files:
@@ -390,6 +454,9 @@ def main() -> None:
             files_without_match=args.files_without_match,
             files_with_matches=args.files_with_matches,
             invert_match=args.invert_match,
+            before_context=before_context,
+            after_context=after_context,
+            group_separator=args.group_separator,
         )
     )
 

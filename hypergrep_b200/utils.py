@@ -24,6 +24,9 @@ _DEFAULT_FLAGS = HS_FLAG_DOTALL | HS_FLAG_MULTILINE | HS_FLAG_SINGLEMATCH
 RC_INVALID_FILE = 101
 _RC_INTERRUPTED = 130
 
+# Result.id of a context line (scan()/grep() with before_context / after_context; GPUGREP_CONTEXT_ID in include/gpugrep.h).
+CONTEXT_ID = 0xFFFFFFFF
+
 _LIB_NAME = "libgpugrep.so"
 _lock = threading.Lock()
 _state: dict = {"lib": None, "libzstd": None, "libhs": None}
@@ -146,6 +149,8 @@ def scan(  # pylint: disable=too-many-arguments
     buffer_count: int = 16,
     max_match_count: int = 0,
     invert_match: bool = False,
+    before_context: int = 0,
+    after_context: int = 0,
 ) -> int:
     """Scan one plain/gzip/zstd file on the GPU, delivering matched lines in batches (reference utils.py:292-358).
 
@@ -153,14 +158,23 @@ def scan(  # pylint: disable=too-many-arguments
     with 0-based ``line_number``.  Returns the engine's code: 0, or 1-7 (reference hyperscanner.c:25-33).
     ``invert_match`` (``grep -v``) delivers the lines that no pattern matches instead, each with id 0, and
     ``max_match_count`` then counts those lines.
+    ``before_context`` / ``after_context`` (``grep -B`` / ``-A``) also deliver the lines that lie up to that many lines
+    before / after a selected line, with id ``CONTEXT_ID``; selected lines then carry id 0.  ``max_match_count`` counts
+    selected lines, and the ``after_context`` lines behind the one that reaches it are still delivered, as context.
     """
+    _check_context(before_context, after_context)
     pattern_array, flags_array, ids_array = prepare_patterns(patterns, flags=flags, ids=ids)
     c_callback = CALLBACK_TYPE(callback)
     lib = _get_hyperscanner_lib()
-    entry = _invert_entry(lib) if invert_match else None
+    context = before_context > 0 or after_context > 0
+    entry = _context_entry(lib) if context else (_invert_entry(lib) if invert_match else None)
     outcome = {"rc": 0}
 
     def _run() -> None:
+        if context:
+            outcome["rc"] = entry(path.encode(), pattern_array, flags_array, ids_array, len(pattern_array), c_callback, buffer_size,
+                                  buffer_count, max_match_count, before_context, after_context, int(invert_match), None)
+            return
         if entry is not None:
             outcome["rc"] = entry(path.encode(), pattern_array, flags_array, ids_array, len(pattern_array), c_callback, buffer_size,
                                   buffer_count, max_match_count, None)
@@ -218,6 +232,28 @@ def _invert_entry(lib: ctypes.CDLL):
     return entry
 
 
+def _check_context(before_context: int, after_context: int) -> None:
+    if before_context < 0 or after_context < 0:
+        raise ValueError(f"context line counts must not be negative (before_context={before_context}, after_context={after_context})")
+    if before_context > 0xFFFFFFFF or after_context > 0xFFFFFFFF:
+        raise ValueError("context line counts must fit in 32 bits")
+
+
+def _context_entry(lib: ctypes.CDLL):
+    """gpugrep_context_scan_file of the loaded library.  Context lines have no CPU fallback: a library without the entry
+    point (a plain libhyperscanner.so through GPUGREP_LIBRARY) is an error."""
+    try:
+        entry = lib.gpugrep_context_scan_file
+    except AttributeError as error:
+        raise NotImplementedError(
+            "before_context / after_context need gpugrep_context_scan_file, which the loaded native library does not export "
+            f"({_library_path()}); there is no CPU fallback"
+        ) from error
+    entry.restype = ctypes.c_int
+    entry.argtypes = _FILE_ENTRY_ARGTYPES[:9] + [ctypes.c_uint, ctypes.c_uint, ctypes.c_int, ctypes.c_void_p]
+    return entry
+
+
 def _count_matches(path: str, patterns: Sequence[str], flags: Sequence[int], max_match_count: int,
                    invert_match: bool = False) -> tuple[int, int] | None:
     """Count-only scan without a callback: the library counts on the device and copies no line back
@@ -261,7 +297,9 @@ def grep(  # pylint: disable=too-many-arguments
     errors: str = "ignore",
     max_match_count: int = 0,
     invert_match: bool = False,
-) -> tuple[int | list[tuple[int, str]], int]:
+    before_context: int = 0,
+    after_context: int = 0,
+) -> tuple[int | list[tuple[int, str]] | list[tuple[int, str, bool]], int]:
     """grep-like collector on top of :func:`scan` (reference utils.py:147-231).
 
     Returns ``(results, return_code)`` where results is a count (``count_only``) or a list of
@@ -269,7 +307,12 @@ def grep(  # pylint: disable=too-many-arguments
     unless ``no_messages`` is set, in which case the code is RC_INVALID_FILE.
     ``invert_match`` (``grep -v``) selects the lines that no pattern matches; ``max_match_count`` and the count then
     refer to those lines, and ``only_matching`` gives ``[]`` (a line without a match has no matching parts).
+    ``before_context`` / ``after_context`` (``grep -B`` / ``-A``) add the lines up to that many lines before / after each
+    selected line; results are then ``(line number, line text, is_context)``.  ``count_only`` and ``only_matching`` ignore
+    context.  Negative counts raise ValueError.
     """
+    _check_context(before_context, after_context)
+    context = (before_context > 0 or after_context > 0) and not (count_only or only_matching)
     python_patterns = [re.compile(pattern) for pattern in patterns]
     collected: list[tuple[int, str]] = []
     counter = [0]
@@ -309,6 +352,8 @@ def grep(  # pylint: disable=too-many-arguments
                     continue
                 text = raw.decode(errors=errors)
                 groups.append([(record.line_number + 1, f"{part.group()}\n") for part in python_patterns[record.id].finditer(text)])
+            elif context:
+                collected.append((record.line_number + 1, raw.decode(errors=errors), record.id == CONTEXT_ID))
             else:
                 collected.append((record.line_number + 1, raw.decode(errors=errors)))
 
@@ -326,6 +371,8 @@ def grep(  # pylint: disable=too-many-arguments
         max_match_count=max_match_count,
         buffer_count=_GREP_BATCH,
         invert_match=invert_match,
+        before_context=before_context if context else 0,
+        after_context=after_context if context else 0,
     )
     if only_matching:
         _fill_spans(groups, deferred, patterns, widths, python_patterns, errors)

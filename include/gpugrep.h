@@ -127,6 +127,28 @@ GPUGREP_API int gpugrep_invert_scan_buffer(const void* data, size_t size, int lo
                                hs_event on_event, int buffer_size, int buffer_count, unsigned long long max_match_count,
                                void* stream, gpugrep_stats* stats);
 
+/* ---- context lines (`grep -A/-B/-C`) -----------------------------------------------------------------------------
+ * Same inputs and return codes as gpugrep_scan_file / gpugrep_scan_buffer.  The selected lines are the matched pseudo-lines,
+ * or with `invert` != 0 those in which no pattern reports (as gpugrep_invert_scan_*).  A pseudo-line is delivered if it is
+ * selected, or lies within `after` lines after or `before` lines before a selected line (a context line).  Records come in
+ * line order, one per delivered line: selected lines with id 0, context lines with id GPUGREP_CONTEXT_ID; `line` is the
+ * stripped text (a pseudo-line of NUL bytes only is ""), and a caller sees a new group wherever line_number jumps.
+ * The pattern set is compile-checked as given, then scanned as "every pattern SINGLEMATCH, one id".  max_match_count counts
+ * selected lines; after the line that reaches it, the next `after` lines are still delivered, all as context (even lines
+ * that would match), then the scan stops.  Batches are full batches of buffer_count records, context lines included
+ * (clamped to max_match_count when that is smaller), then the remainder.  stats->matches counts selected lines.
+ * With before == after == 0 the records equal those of gpugrep_scan_* with every id 0 (or gpugrep_invert_scan_*).
+ * on_event == NULL counts selected lines and ignores context.  A build of the engine without context lines returns 7. */
+#define GPUGREP_CONTEXT_ID 0xFFFFFFFFu
+GPUGREP_API int gpugrep_context_scan_file(const char* file_name, const char* const* patterns, const unsigned int* pattern_flags,
+                              const unsigned int* pattern_ids, unsigned int elements, hs_event on_event, int buffer_size,
+                              int buffer_count, unsigned long long max_match_count, unsigned int before, unsigned int after,
+                              int invert, gpugrep_stats* stats);
+GPUGREP_API int gpugrep_context_scan_buffer(const void* data, size_t size, int location, const char* const* patterns,
+                                const unsigned int* pattern_flags, const unsigned int* pattern_ids, unsigned int elements,
+                                hs_event on_event, int buffer_size, int buffer_count, unsigned long long max_match_count,
+                                unsigned int before, unsigned int after, int invert, void* stream, gpugrep_stats* stats);
+
 /* ---- match END offsets (SURVEY.md section 8f-4: spans for `grep -o`) --------------------------------------------
  * The reference gets the spans of `-o` by re-running Python's re.finditer() over every matched line (utils.py:205-212);
  * Hyperscan itself reports (id, end offset) per match and the reference drops the offset (hyperscanner.c:83-102).
