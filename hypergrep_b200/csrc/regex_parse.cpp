@@ -202,8 +202,15 @@ private:
             case 'H': out = ~set_hspace(); return EscKind::Set;
             case 'V': out = ~set_vspace(); return EscKind::Set;
             case 'v': out = set_vspace(); return EscKind::Set;
-            case 'N': if (in_class) { fail("\\N is not supported in a class"); return EscKind::Error; }
-                      out = ~ByteSet::of('\n'); return EscKind::Set;
+            case 'N': {
+                if (in_class) { fail("\\N is not supported in a class"); return EscKind::Error; }
+                // \N{U+hh..} names a code point (UTF mode only); any other '{' after \N must open a quantifier
+                int mn, mx;
+                const size_t at = i_;
+                if (!eof() && peek() == '{' && !try_braces(mn, mx)) { fail("\\N{ is not a quantifier (\\N{U+..} needs UTF mode)"); return EscKind::Error; }
+                i_ = at;
+                out = ~ByteSet::of('\n'); return EscKind::Set;
+            }
             case 'n': out = ByteSet::of('\n'); is_single = true; return EscKind::Set;
             case 'r': out = ByteSet::of('\r'); is_single = true; return EscKind::Set;
             case 't': out = ByteSet::of('\t'); is_single = true; return EscKind::Set;
@@ -216,7 +223,7 @@ private:
                 if (eof()) { fail("\\c at end of pattern"); return EscKind::Error; }
                 unsigned char x = peek(); i_++;
                 if (x >= 'a' && x <= 'z') x -= 32;
-                if (x > 127) { fail("\\c must be followed by an ASCII character"); return EscKind::Error; }
+                if (x < 32 || x > 126) { fail("\\c must be followed by a printable ASCII character"); return EscKind::Error; }
                 out = ByteSet::of(x ^ 0x40); is_single = true; return EscKind::Set;
             }
             case 'x': {
@@ -249,7 +256,7 @@ private:
         }
         if (c >= '1' && c <= '9') {
             if (!in_class) { fail("back-references are not supported"); return EscKind::Error; }
-            if (c >= '8') { fail("invalid escape in class"); return EscKind::Error; }
+            if (c >= '8') { out = ByteSet::of(c); is_single = true; return EscKind::Set; }   // [\8]: the digit itself
             unsigned v = c - '0'; int nd = 1;
             while (nd < 3 && !eof() && peek() >= '0' && peek() <= '7') { v = v * 8 + (peek() - '0'); nd++; i_++; }
             out = ByteSet::of(v & 255); is_single = true; return EscKind::Set;
@@ -292,6 +299,9 @@ private:
         return true;
     }
 
+    // '-' at i_ that is not the last character of the class
+    bool dash_starts_range() const { return !eof() && peek() == '-' && i_ + 1 < s_.size() && peek(1) != ']'; }
+
     NodePtr parse_class(const Flags& f) {
         // i_ is just past '['
         bool negate = false;
@@ -319,6 +329,7 @@ private:
                     item = ps;
                     i_ = close + 2;
                     acc |= item; have_prev = false;
+                    if (dash_starts_range()) { fail("invalid range in character class"); return nullptr; }
                     continue;
                 }
                 // no closing :] -> literal '['
@@ -338,7 +349,11 @@ private:
                 }
                 if (k != EscKind::Set) { fail("invalid escape in class"); return nullptr; }
                 if (is_single) { single = true; for (unsigned b = 0; b < 256; b++) if (es.test(b)) single_val = b; }
-                else { acc |= es; have_prev = false; continue; }
+                else {
+                    // a class escape (\d, \h, ...) can bound no range: PCRE2 faults "[\d-z]" where Perl only warns
+                    if (dash_starts_range()) { fail("invalid range in character class"); return nullptr; }
+                    acc |= es; have_prev = false; continue;
+                }
             } else {
                 i_++; single = true; single_val = c;
             }
@@ -357,9 +372,10 @@ private:
                         EscKind k = parse_escape(true, f, es, ak, is_single);
                         if (k == EscKind::Error) return nullptr;
                         if (k == EscKind::Set && is_single) { for (unsigned b = 0; b < 256; b++) if (es.test(b)) hi = b; hi_ok = true; }
-                        else { i_ = save; }  // "a-\d": '-' is literal; re-parse from '-'
-                    } else if (d == '[' && (peek(1) == ':')) {
-                        i_ = save;
+                        else if (k == EscKind::Set) { fail("invalid range in character class"); return nullptr; }   // "a-\d"
+                        else { i_ = save; }   // "a-\Q..": '-' is literal; re-parse from '-'
+                    } else if (d == '[' && peek(1) == ':' && s_.find(":]", i_ + 2) != std::string::npos) {
+                        fail("invalid range in character class"); return nullptr;   // "a-[:digit:]"
                     } else {
                         i_++; hi = d; hi_ok = true;
                     }

@@ -61,12 +61,12 @@ def _gram_bytes(g: int) -> bytes:
     return int(g).to_bytes(4, "little")
 
 
-def k1_text(n: int, grams: np.ndarray, seed: int) -> bytes:
+def k1_text(n: int, grams: np.ndarray, seed: int, background: np.ndarray = fpc.BACKGROUND) -> bytes:
     """Background that no gram of the set occurs in, lines of 20-300 bytes, and grams of the set planted one per 16-byte
     chunk at most: one per 512-byte block at offset 53*j + 509 (every offset mod 512 and mod 16 over 512 blocks) and one in
     the last six bytes of each block (grams that run into the next block, the next group of four, the next warp's step)."""
     r = np.random.default_rng(seed)
-    buf = fpc.BACKGROUND[r.integers(0, fpc.BACKGROUND.size, n)]
+    buf = background[r.integers(0, background.size, n)]
     nl = np.cumsum(r.integers(20, 300, n // 20 + 2))
     buf[nl[nl < n]] = 10
     j = np.arange((n + 511) // 512, dtype=np.int64)
