@@ -854,6 +854,8 @@ int scan_memory(const uint8_t* data, size_t size, int location, const Params& pr
     // Collect segment `idx` and deliver its results.  A large segment in which the fast path hit one of its bounds (a line
     // too long for it, a candidate / record overflow) is not sent down the general path as a whole: the same bytes are
     // scanned again in 64 MiB pieces on this slot, one after the other, and only the piece with the problem pays for it.
+    // A general-path segment with more match events than one segment holds is cut the same way (device-resident input
+    // comes in segments of up to 2 GiB; a 64 MiB piece is what host input gets anyway).
     constexpr size_t kSplitAbove = (size_t)128 << 20, kSplitPiece = (size_t)64 << 20;
     auto finish = [&](int idx) -> int {
         SegmentResult res;

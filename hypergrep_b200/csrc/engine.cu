@@ -164,7 +164,7 @@ public:
     SegmentStats stats;
     bool in_use = false;
 
-    int run_general(SegmentResult& out, std::string& error);
+    int run_general(SegmentResult& out, std::string& error, size_t split_above);
     int run_complement(size_t nrec, size_t nlines, size_t selected, std::string& error);
     int run_context(size_t nrec, size_t nlines, size_t selected, size_t& count, std::string& error);
     bool context() const { return want_records && (ctx_before || ctx_after); }
@@ -716,7 +716,7 @@ int slot_submit(ScanSlot* s, const DeviceDb& ddb, const DevicePrefilter* pf, con
     return 0;
 }
 
-int ScanSlot::run_general(SegmentResult& out, std::string& error) {
+int ScanSlot::run_general(SegmentResult& out, std::string& error, size_t split_above) {
     cudaStream_t st = stream;
     Totals* dT = d_totals.as<Totals>();
     Totals* hT = h_totals.as<Totals>();
@@ -810,7 +810,12 @@ int ScanSlot::run_general(SegmentResult& out, std::string& error) {
         CUDA_TRY(cudaMemcpyAsync(hT, dT, sizeof(Totals), cudaMemcpyDeviceToHost, st));
         CUDA_TRY(cudaStreamSynchronize(st));
         size_t nev = (size_t)hT->rec_total;
-        if (nev > ((size_t)1 << 27)) { error = "too many match events in one segment (non-SINGLEMATCH pattern matching nearly every byte?)"; return 7; }
+        if (nev > ((size_t)1 << 27)) {
+            // a large segment is scanned again in smaller pieces, each under the bound unless its own text is that dense
+            if (split_above && n > split_above) return kSplitSegment;
+            error = "too many match events in one segment (non-SINGLEMATCH pattern matching nearly every byte?)";
+            return 7;
+        }
         if (nev) {
             if (d_events.reserve(nev * sizeof(EventRec)) != cudaSuccess) { error = "cudaMalloc failed"; return 3; }
             if (h_recs.reserve(nev * sizeof(EventRec)) != cudaSuccess) { error = "cudaHostAlloc failed"; return 3; }
@@ -961,7 +966,8 @@ int slot_collect(ScanSlot* s, SegmentResult& out, std::string& error, size_t spl
     }
     if (!done) {
         if (s->fast && split_above && s->n > split_above) { out.stats = s->stats; return kSplitSegment; }
-        int rc = s->run_general(out, error);
+        int rc = s->run_general(out, error, split_above);
+        if (rc == kSplitSegment) out.stats = s->stats;
         if (rc) return rc;
     }
     float ms = 0;

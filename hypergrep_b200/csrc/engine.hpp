@@ -100,8 +100,9 @@ __attribute__((weak)) void slot_set_context(ScanSlot* slot, uint32_t before, uin
 // Wait for the segment and expose its results (valid until the next slot_submit on this slot).
 // Returns kSplitSegment (and no results) when the fast path hit one of its capacity bounds - a line too long for it, a
 // candidate or record overflow - in a segment of more than `split_above` bytes: the caller then scans the same bytes again
-// in smaller segments, so that only the piece with the problem takes the (much slower) general path.  split_above == 0:
-// never ask, take the general path for the whole segment.
+// in smaller segments, so that only the piece with the problem takes the (much slower) general path.  The general path
+// asks the same when such a segment has more match events than it can hold (2^27).  split_above == 0: never ask, take
+// the general path for the whole segment (and fail with 7 over the event bound).
 constexpr int kSplitSegment = -2;
 int slot_collect(ScanSlot* slot, SegmentResult& out, std::string& error, size_t split_above = 0);
 

@@ -311,6 +311,46 @@ static int ev_cmp(const void* a, const void* b) {
     return 0;
 }
 
+/* Every (end, id) at which a match of a pattern of `db` ends in the block, in hs_scan order (by end, then id), each pair
+   once: every start offset is tried with an anchored DFA match, whose ovector lists all match ends from that start.
+   *out is malloc()ed (free() it); returns 0 or PORT_SCAN. */
+static int port_block_ends(port_db_t* db, const char* line, size_t len, port_ev_t** out, size_t* out_n) {
+    size_t cap = 64, nev = 0;
+    port_ev_t* ev = (port_ev_t*)malloc(cap * sizeof(*ev));
+    uint32_t ovn = (uint32_t)(len + 2);
+    p2_md* md = P2.md_create(ovn, NULL);
+    size_t wsn = 4096 + 64 * len;
+    int* ws = (int*)malloc(wsn * sizeof(int));
+    unsigned char* seen = (unsigned char*)malloc(len + 1);
+    for (unsigned i = 0; i < db->n; i++) {
+        memset(seen, 0, len + 1);
+        for (size_t s = 0; s < len; s++) {
+            int rc = P2.dfa_match(db->code[i], (const unsigned char*)line, len, s, P2_ANCHORED, md, NULL, ws, wsn);
+            if (rc == P2_ERROR_NOMATCH) continue;
+            if (rc < 0) { fprintf(stderr, "oracle: pcre2_dfa_match error %d\n", rc); free(ev); free(ws); free(seen); P2.md_free(md); return PORT_SCAN; }
+            size_t* ov = P2.ovector(md);
+            int cnt = rc == 0 ? (int)ovn : rc;
+            for (int k = 0; k < cnt; k++) {
+                size_t e = ov[2 * k + 1];
+                if (e == s) continue; /* zero-width matches are not reports (the simple path passes PCRE2_NOTEMPTY) */
+                seen[e] = 1;
+            }
+        }
+        for (size_t e = 1; e <= len; e++) if (seen[e]) {
+            if (nev == cap) { cap *= 2; ev = (port_ev_t*)realloc(ev, cap * sizeof(*ev)); }
+            ev[nev].end = e; ev[nev].id = db->ids[i]; nev++;
+        }
+    }
+    free(ws); free(seen); P2.md_free(md);
+    qsort(ev, nev, sizeof(*ev), ev_cmp);
+    size_t u = 0;   /* one report per (id, end) */
+    for (size_t k = 0; k < nev; k++)
+        if (!u || ev[k].end != ev[u - 1].end || ev[k].id != ev[u - 1].id) ev[u++] = ev[k];
+    *out = ev;
+    *out_n = u;
+    return 0;
+}
+
 /* stand-in for hs_scan(db, line, strlen(line), ...) at hyperscanner.c:217 */
 static int port_scan_block(port_db_t* db, port_state_t* st, const char* line, size_t len) {
     if (len == 0) return 0;
@@ -339,36 +379,11 @@ static int port_scan_block(port_db_t* db, port_state_t* st, const char* line, si
         return 0;
     }
     /* general mode: all (id, end) reports */
-    size_t cap = 64, nev = 0;
-    port_ev_t* ev = (port_ev_t*)malloc(cap * sizeof(*ev));
-    uint32_t ovn = (uint32_t)(len + 2);
-    p2_md* md = P2.md_create(ovn, NULL);
-    size_t wsn = 4096 + 64 * len;
-    int* ws = (int*)malloc(wsn * sizeof(int));
-    unsigned char* seen = (unsigned char*)malloc(len + 1);
-    for (unsigned i = 0; i < db->n; i++) {
-        memset(seen, 0, len + 1);
-        for (size_t s = 0; s < len; s++) {
-            int rc = P2.dfa_match(db->code[i], (const unsigned char*)line, len, s, P2_ANCHORED, md, NULL, ws, wsn);
-            if (rc == P2_ERROR_NOMATCH) continue;
-            if (rc < 0) { fprintf(stderr, "oracle: pcre2_dfa_match error %d\n", rc); free(ev); free(ws); free(seen); P2.md_free(md); return PORT_SCAN; }
-            size_t* ov = P2.ovector(md);
-            int cnt = rc == 0 ? (int)ovn : rc;
-            for (int k = 0; k < cnt; k++) {
-                size_t e = ov[2 * k + 1];
-                if (e == s) continue; /* zero-width matches are not reports (the simple path passes PCRE2_NOTEMPTY) */
-                seen[e] = 1;
-            }
-        }
-        for (size_t e = 1; e <= len; e++) if (seen[e]) {
-            if (nev == cap) { cap *= 2; ev = (port_ev_t*)realloc(ev, cap * sizeof(*ev)); }
-            ev[nev].end = e; ev[nev].id = db->ids[i]; nev++;
-        }
-    }
-    qsort(ev, nev, sizeof(*ev), ev_cmp);
-    /* dedupe (id,end); SINGLEMATCH ids fire once per block */
+    port_ev_t* ev = NULL;
+    size_t nev = 0;
+    if (port_block_ends(db, line, len, &ev, &nev) != 0) return PORT_SCAN;
+    /* SINGLEMATCH ids fire once per block */
     for (size_t k = 0; k < nev; k++) {
-        if (k && ev[k].end == ev[k - 1].end && ev[k].id == ev[k - 1].id) continue;
         int sm = 0;
         for (unsigned i = 0; i < db->n; i++) if (db->ids[i] == ev[k].id) { sm = (db->flags[i] & HS_FLAG_SINGLEMATCH) != 0; break; }
         if (sm) {
@@ -378,7 +393,7 @@ static int port_scan_block(port_db_t* db, port_state_t* st, const char* line, si
         }
         port_emit(st, ev[k].id);
     }
-    free(ev); free(ws); free(seen); P2.md_free(md);
+    free(ev);
     return 0;
 }
 
@@ -566,5 +581,42 @@ int oracle_lines_buffer(const char* text, size_t n, const char* const* patterns,
     *out_matches = st.match_count; *out_lines = st.line_number;
     g_sink = NULL;
     free(buf); free(slot.line); port_db_free(db);
+    return ret;
+}
+
+/* ---- test extension: what gpugrep_match_ends() promises (include/gpugrep.h), from the same pseudo-lines, strip rule and
+ * hs_scan order as the scans above: one (line, id, end) per match end, SINGLEMATCH cleared, `end` counted from the start
+ * of the scanned block.  At most `capacity` records are written to `out`; *count is the number found. ---- */
+typedef struct { unsigned long long line_number; unsigned int id; unsigned int end; } port_match_end_t;
+int oracle_ends_buffer(const char* text, size_t n, const char* const* patterns, const unsigned int* flags, const unsigned int* ids,
+                       unsigned elements, int buffer_size, port_match_end_t* out, unsigned long long capacity, unsigned long long* count) {
+    unsigned* cleared = (unsigned*)malloc((elements ? elements : 1) * sizeof(unsigned));
+    for (unsigned i = 0; i < elements; i++) cleared[i] = (flags ? flags[i] : 0u) & ~HS_FLAG_SINGLEMATCH;
+    port_db_t* db = port_compile(patterns, cleared, ids, elements);
+    free(cleared);
+    if (!db) return PORT_DB;
+    char* buf = (char*)calloc((size_t)buffer_size + 1, 1);
+    unsigned long long line_number = 0, found = 0;
+    size_t pos = 0; int ret = 0;
+    while (pos < n) {
+        size_t lim = (size_t)buffer_size - 1;
+        size_t avail = n - pos < lim ? n - pos : lim;
+        const char* nl = (const char*)memchr(text + pos, '\n', avail);
+        size_t k = nl ? (size_t)(nl - (text + pos)) + 1 : avail;
+        memcpy(buf, text + pos, k); buf[k] = 0; pos += k;
+        const char* line = port_strip(buf, buffer_size);
+        size_t len = strlen(line);
+        if (len) {
+            port_ev_t* ev = NULL;
+            size_t nev = 0;
+            if ((ret = port_block_ends(db, line, len, &ev, &nev)) != 0) break;
+            for (size_t e = 0; e < nev; e++, found++)
+                if (found < capacity) { out[found].line_number = line_number; out[found].id = ev[e].id; out[found].end = (unsigned)ev[e].end; }
+            free(ev);
+        }
+        line_number++;
+    }
+    *count = found;
+    free(buf); port_db_free(db);
     return ret;
 }

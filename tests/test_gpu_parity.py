@@ -443,7 +443,7 @@ def _oracle_records_threaded(oracle_lib, data: bytes, patterns, flags, threads: 
 
 
 def test_ten_thousand_caseless_patterns_full_set(gpu_lib, oracle_lib):
-    """configs[4] at its named size: ALL 10,000 caseless template patterns (many DFA groups, group gating, a candidate
+    """configs[4] at its named size: ALL 10,000 caseless template patterns (4 DFA groups, group gating, a candidate
     list close to its capacity) over 64 MiB of 2-16 KiB JSON-ish lines, records compared with the oracle (every matched
     line number and its bytes).  The oracle runs sharded over the host cores."""
     import os
