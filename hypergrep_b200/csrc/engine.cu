@@ -19,6 +19,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <atomic>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -95,6 +96,31 @@ int device_sms() {
 }
 // k_verify_smem: table + class map per block, two blocks per SM (227 KiB of shared memory)
 constexpr size_t kMaxSharedTableBytes = (size_t)112 << 10;
+
+// A kernel's dynamic shared-memory limit (cudaFuncAttributeMaxDynamicSharedMemorySize) belongs to the process and the
+// device, not to one launch.  Scans run concurrently on host threads with different table sizes, so a scan that set a
+// smaller limit would make another scan's larger launch fail.  The limit of each kernel is therefore only ever raised:
+// one SmemLimit per kernel function (a static at its one launch site) holds the largest value set on each device.
+constexpr int kMaxDevices = 64;
+struct SmemLimit {
+    std::atomic<int> bytes[kMaxDevices] = {};
+};
+std::mutex g_smem_mu;
+
+template <class Kernel>
+cudaError_t raise_smem_limit(SmemLimit& limit, Kernel kernel, size_t smem) {
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return e;
+    if (dev < 0 || dev >= kMaxDevices) return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    std::atomic<int>& cur = limit.bytes[dev];
+    if ((size_t)cur.load(std::memory_order_acquire) >= smem) return cudaSuccess;
+    std::lock_guard<std::mutex> lk(g_smem_mu);
+    if ((size_t)cur.load(std::memory_order_relaxed) >= smem) return cudaSuccess;
+    e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e == cudaSuccess) cur.store((int)smem, std::memory_order_release);
+    return e;
+}
 
 }  // namespace
 
@@ -497,7 +523,8 @@ static cudaError_t launch_stream_t(cudaStream_t st, int grid, int block, size_t 
                                    uint32_t* nlmask, unsigned long long* gsum, const DevicePrefilter* pf,
                                    unsigned int* flags) {
     if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(k_stream<STRIDE, FOLD, MODE, NODD, NUL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        static SmemLimit limit;
+        cudaError_t e = raise_smem_limit(limit, k_stream<STRIDE, FOLD, MODE, NODD, NUL>, smem);
         if (e != cudaSuccess) return e;
     }
     k_stream<STRIDE, FOLD, MODE, NODD, NUL><<<grid, block, smem, st>>>(data, n, meta, nlmask, gsum, pf ? pf->d_table : nullptr, pf ? pf->table_words : 0,
@@ -665,11 +692,15 @@ int slot_submit(ScanSlot* s, const DeviceDb& ddb, const DevicePrefilter* pf, con
                 error = "cudaMalloc failed for candidate scratch"; return 3;
             }
             const size_t csmem = (size_t)pf->table_words * 4;
-            CUDA_TRY(cudaFuncSetAttribute(k_confirm, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)csmem));
+            static SmemLimit confirm_limit;
+            CUDA_TRY(raise_smem_limit(confirm_limit, k_confirm, csmem));
             const unsigned cgrid = (unsigned)std::min<size_t>((s->cand_cap + kConfirmThreads - 1) / kConfirmThreads, sms);
             k_confirm<<<cgrid, kConfirmThreads, csmem, st>>>(s->data, n, s->d_cand.as<uint32_t>(), &dT->meta_total, s->cand_cap, pf->d_table, pf->table_words,
                                                              pf->pp, rp, s->d_hitinfo.as<unsigned long long>(), s->d_res.as<uint32_t>(),
                                                              s->d_survivors.as<uint32_t>(), dT);
+            // (checked before anything that reads its output is queued)
+            le = cudaGetLastError();
+            if (le != cudaSuccess) { error = std::string("k_confirm launch: ") + cudaGetErrorString(le); return 7; }
             hitinfo = s->d_hitinfo.as<unsigned long long>();
             survivors = s->d_survivors.as<uint32_t>();
             s->stats.launches++;
@@ -678,7 +709,8 @@ int slot_submit(ScanSlot* s, const DeviceDb& ddb, const DevicePrefilter* pf, con
         const bool v1 = vsel && std::strcmp(vsel, "v1") == 0;
         if (!v1 && ddb.smem_table_bytes && hitinfo == nullptr && pf->lookback <= 64u) {
             const size_t vsmem = 256 + ddb.smem_table_bytes;
-            CUDA_TRY(cudaFuncSetAttribute(k_verify_smem, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)vsmem));
+            static SmemLimit verify_limit;
+            CUDA_TRY(raise_smem_limit(verify_limit, k_verify_smem, vsmem));
             const unsigned per_sm = blocks_per_sm(k_verify_smem, kVerifySmemThreads, vsmem);
             unsigned vgrid = (unsigned)std::min<size_t>((s->cand_cap + kVerifySmemThreads - 1) / kVerifySmemThreads, (size_t)per_sm * sms);
             k_verify_smem<<<vgrid, kVerifySmemThreads, vsmem, st>>>(view, s->data, n, s->d_cand.as<uint32_t>(), &dT->meta_total, s->cand_cap, pf->lookback,
@@ -690,6 +722,8 @@ int slot_submit(ScanSlot* s, const DeviceDb& ddb, const DevicePrefilter* pf, con
             kernel<<<vgrid, 128, 0, st>>>(view, s->data, n, s->d_cand.as<uint32_t>(), &dT->meta_total, s->cand_cap, pf->lookback, idle_span, hitinfo,
                                           survivors, dT, s->d_res.as<uint32_t>(), tile_records);
         }
+        le = cudaGetLastError();
+        if (le != cudaSuccess) { error = std::string("verification kernel launch: ") + cudaGetErrorString(le); return 7; }
         k_tile_offsets<<<1, 1024, 0, st>>>(tile_records, &dT->meta_total, s->cand_cap, &dT->rec_total);
         // Without records (count-only scans) the emit kernel writes one 4-byte key per record into the record buffer, and
         // k_count_keys counts the distinct lines.  Either way a segment with more records than fit falls back to the general
