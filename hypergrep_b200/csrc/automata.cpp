@@ -16,6 +16,7 @@ namespace {
 struct NfaBuilder {
     Nfa& nfa;
     size_t max_insts;
+    bool lazy = false;   // honour Node::lazy (span programs only)
     bool overflow = false;
     std::map<ByteSet, int> set_ids;
 
@@ -61,19 +62,20 @@ struct NfaBuilder {
             case NodeKind::Repeat: {
                 const Node& c = *n.kids[0];
                 int cur;
+                const bool swap = lazy && n.lazy;   // prefer leaving the repeat
                 if (n.max < 0) {
                     int loop = add(NfaInst::Split, -1, -1, 0);
                     int body = emit(c, loop);
                     if (overflow) return 0;
-                    nfa.prog[loop].x = body;
-                    nfa.prog[loop].y = next;
+                    nfa.prog[loop].x = swap ? next : body;
+                    nfa.prog[loop].y = swap ? body : next;
                     cur = (n.min == 0) ? loop : body;
                     for (int k = 1; k < n.min; k++) cur = emit(c, cur);
                 } else {
                     cur = next;
                     for (int k = 0; k < n.max - n.min; k++) {
                         int b = emit(c, cur);
-                        cur = add(NfaInst::Split, b, next, 0);
+                        cur = swap ? add(NfaInst::Split, next, b, 0) : add(NfaInst::Split, b, next, 0);
                         if (overflow) return 0;
                     }
                     for (int k = 0; k < n.min; k++) cur = emit(c, cur);
@@ -87,8 +89,8 @@ struct NfaBuilder {
 
 }  // namespace
 
-bool nfa_add_pattern(Nfa& nfa, const Node& ast, int index, size_t max_insts) {
-    NfaBuilder b{nfa, max_insts};
+bool nfa_add_pattern(Nfa& nfa, const Node& ast, int index, size_t max_insts, bool lazy) {
+    NfaBuilder b{nfa, max_insts, lazy};
     for (size_t i = 0; i < nfa.sets.size(); i++) b.set_ids.emplace(nfa.sets[i], (int)i);
     size_t mark_prog = nfa.prog.size(), mark_sets = nfa.sets.size();
     int m = b.add(NfaInst::Match, -1, -1, index);

@@ -31,8 +31,10 @@ struct Nfa {
 };
 
 // Append pattern `ast` as pattern number `index` of the group.  Returns false if the program would exceed
-// `max_insts` (bounded repeats are expanded by copying).
-bool nfa_add_pattern(Nfa& nfa, const Node& ast, int index, size_t max_insts);
+// `max_insts` (bounded repeats are expanded by copying).  Every Split lists the branch a backtracking matcher tries first
+// as x: the earlier alternative, and for a repeat the greedy choice, or with `lazy` the lazy choice of a repeat marked so
+// (the span program, pike_vm.hpp).  The automata do not depend on the order, and are built without `lazy`.
+bool nfa_add_pattern(Nfa& nfa, const Node& ast, int index, size_t max_insts, bool lazy = false);
 
 struct Dfa {
     // alphabet

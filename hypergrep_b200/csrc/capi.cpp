@@ -30,6 +30,7 @@
 #include "database.hpp"
 #include "engine.hpp"
 #include "ingest.hpp"
+#include "pike_vm.hpp"
 
 namespace gpugrep {
 void set_last_error(const std::string& e);
@@ -106,6 +107,13 @@ struct EndsSink {
     size_t count = 0;
 };
 
+// Sink of gpugrep_match_spans(): (line, start, end) records.
+struct SpansSink {
+    gpugrep_match_span* out;
+    size_t capacity;
+    size_t count = 0;
+};
+
 class Deliverer {
 public:
     Deliverer(hs_event cb, int buffer_count) : cb_(cb), cap_(std::max(1, buffer_count)) {
@@ -145,6 +153,13 @@ public:
         if (ends_->count < ends_->capacity) ends_->out[ends_->count] = gpugrep_match_end{line_number, id, end};
         ends_->count++;
     }
+    void set_spans(SpansSink* sink) { spans_ = sink; }
+    bool wants_spans() const { return spans_ != nullptr; }
+    void emit_span(unsigned long long line_number, unsigned start, unsigned end) {
+        count_++;
+        if (spans_->count < spans_->capacity) spans_->out[spans_->count] = gpugrep_match_span{line_number, start, end};
+        spans_->count++;
+    }
     void flush() {
         if (cb_ && fill_ > 0) cb_(results_.data(), fill_);
         fill_ = 0;
@@ -181,6 +196,7 @@ private:
     int cap_;
     ShardResults* collect_ = nullptr;
     EndsSink* ends_ = nullptr;
+    SpansSink* spans_ = nullptr;
     int fill_ = 0;
     unsigned long long count_ = 0;
     std::vector<hyperscanner_result_t> results_;
@@ -381,7 +397,7 @@ struct Job {
         stats.segments++;
         stats.nul_segments += r.stats.nul ? 1u : 0u;
         if (stop) return 0;
-        int rc = db->simple ? deliver_simple(r, host, slot) : deliver_events(r, host, slot);
+        int rc = out->wants_spans() ? deliver_spans(r) : (db->simple ? deliver_simple(r, host, slot) : deliver_events(r, host, slot));
         line_base += r.num_lines;
         return rc;
     }
@@ -440,6 +456,11 @@ struct Job {
     }
 
     std::vector<LineRec> unique_;
+
+    int deliver_spans(const SegmentResult& r) {
+        for (size_t i = 0; i < r.num_spans; i++) out->emit_span(line_base + r.spans[i].line, r.spans[i].start, r.spans[i].end);
+        return 0;
+    }
 
     int deliver_events(const SegmentResult& r, const uint8_t* host, ScanSlot* slot) {
         // events arrive grouped by pseudo-line in file order; inside a line they are grouped by DFA group
@@ -508,6 +529,8 @@ struct Params {
     unsigned long long max_match;
     void* user_stream;
     EndsSink* ends = nullptr;   // gpugrep_match_ends(): end offsets instead of lines
+    SpansSink* spans = nullptr;             // gpugrep_match_spans(): match spans of `span_program` instead of lines
+    const PikeProgram* span_program = nullptr;
     bool invert = false;        // gpugrep_invert_scan_*(): deliver the pseudo-lines in which no pattern reports
     bool context_scan = false;  // gpugrep_context_scan_*(): lines around the selected ones too
     uint32_t before = 0, after = 0;
@@ -534,6 +557,9 @@ void set_invert(ScanSlot* slot, bool invert) {
 void set_context(ScanSlot* slot, const Params& pr) {
     if (slot_set_context) slot_set_context(slot, pr.context() ? pr.before : 0u, pr.context() ? pr.after : 0u);
 }
+void set_spans(ScanSlot* slot, const Params& pr) {
+    if (slot_set_spans) slot_set_spans(slot, pr.span_program);
+}
 
 int setup_job(const Params& pr, Job& job, Deliverer& out, unsigned long long weight = 0) {
     int rc = 0;
@@ -552,6 +578,7 @@ int setup_job(const Params& pr, Job& job, Deliverer& out, unsigned long long wei
     if (pr.buffer_size < 2) { job.error = "buffer_size must be at least 2"; return GPUGREP_SCAN; }
     if (pr.invert && !slot_set_invert) { job.error = "this build of the engine has no inverted scan"; return GPUGREP_SCAN; }
     if (pr.context_scan && !slot_set_context) { job.error = "this build of the engine has no context lines"; return GPUGREP_SCAN; }
+    if (pr.span_program && !slot_set_spans) { job.error = "this build of the engine has no span stage"; return GPUGREP_SCAN; }
     job.device_weight = weight;
     job.device = pick_device(weight, &job.device_charged);
     if (engine_select_device(job.device, job.error) != 0) {
@@ -663,6 +690,7 @@ int scan_file(const char* path, const Params& pr, gpugrep_stats* stats_out, cons
         slot_set_want_records(sl, !count_only);
         set_invert(sl, pr.invert);
         set_context(sl, pr);
+        set_spans(sl, pr);
     }
     SegmentQueue q;
     for (int i = 0; i < kSlots; i++) q.free_slots.push_back(i);
@@ -804,6 +832,7 @@ int scan_memory(const uint8_t* data, size_t size, int location, const Params& pr
     double t0 = now_ms();
     Deliverer own(pr.cb, effective_batch(pr));
     own.set_ends(pr.ends);
+    own.set_spans(pr.spans);
     Deliverer collecting(shard ? shard->collect : nullptr);
     Deliverer counting(nullptr, 1);
     Deliverer& out = !shard ? own : (shard->count_only ? counting : collecting);
@@ -831,6 +860,7 @@ int scan_memory(const uint8_t* data, size_t size, int location, const Params& pr
         slot_set_want_records(sl, !count_only);
         set_invert(sl, pr.invert);
         set_context(sl, pr);
+        set_spans(sl, pr);
     }
     const uint8_t* seg_host[2] = {nullptr, nullptr};
     const uint8_t* seg_dev[2] = {nullptr, nullptr};
@@ -1229,6 +1259,25 @@ int gpugrep_match_ends(const void* data, size_t size, int location, const char* 
     for (unsigned i = 0; i < elements; i++) flags[i] = (pattern_flags ? pattern_flags[i] : 0u) & ~8u;
     gpugrep::EndsSink sink{out, out ? capacity : 0};
     gpugrep::Params pr{patterns, flags.data(), pattern_ids, elements, nullptr, buffer_size, 1, 0, nullptr, &sink};
+    const int rc = gpugrep::scan_memory((const uint8_t*)data, size, location, pr, stats);
+    if (count) *count = sink.count;
+    return rc;
+}
+
+int gpugrep_match_spans(const void* data, size_t size, int location, const char* pattern, int buffer_size, gpugrep_match_span* out,
+                        size_t capacity, size_t* count, gpugrep_stats* stats) {
+    if (count) *count = 0;
+    gpugrep::PikeProgram program;
+    if (!gpugrep::build_pike_program(pattern, program)) {
+        gpugrep::set_last_error("the pattern is not accepted by gpugrep_span_exact");
+        return GPUGREP_DB;
+    }
+    // compiled like the reference's re.compile(pattern): no flags (the automata only check that the pattern compiles)
+    const unsigned flags = 0, id = 0;
+    gpugrep::SpansSink sink{out, out ? capacity : 0};
+    gpugrep::Params pr{&pattern, &flags, &id, 1, nullptr, buffer_size, 1, 0, nullptr};
+    pr.spans = &sink;
+    pr.span_program = &program;
     const int rc = gpugrep::scan_memory((const uint8_t*)data, size, location, pr, stats);
     if (count) *count = sink.count;
     return rc;

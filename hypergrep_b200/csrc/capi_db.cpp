@@ -7,7 +7,9 @@
 #include <string>
 
 #include "../../include/gpugrep.h"
+#include "automata.hpp"
 #include "database.hpp"
+#include "pike_vm.hpp"
 #include "regex.hpp"
 
 namespace gpugrep {
@@ -96,7 +98,122 @@ bool same_meaning_in_python(const std::string& p) {
     return !in_class;
 }
 
+// Lexical screen of the span route: the syntax of same_meaning_in_python plus the quantifiers * + ? {m} {m,} {m,n} and their
+// lazy forms.  Python reads {,n} as {0,n} where this compiler reads a literal; a quantifier after a quantifier is an error
+// in Python (or possessive, from 3.11 on); Python's str \s includes 0x1C-0x1F; $, inline flags and POSIX classes differ too.
+bool spans_mean_the_same_in_python(const std::string& p) {
+    bool in_class = false;
+    bool can_repeat = false;   // the previous item is an atom a quantifier may follow
+    for (size_t i = 0; i < p.size(); i++) {
+        const unsigned char c = (unsigned char)p[i];
+        if (c < 0x20 || c > 0x7e) return false;
+        if (c == '\\') {
+            if (i + 1 >= p.size()) return false;
+            const unsigned char e = (unsigned char)p[++i];
+            if (e == 'x') {   // exactly two hex digits in Python
+                if (i + 2 >= p.size() || !std::isxdigit((unsigned char)p[i + 1]) || !std::isxdigit((unsigned char)p[i + 2])) return false;
+                i += 2;
+            } else if (std::isalnum(e)) {
+                if (in_class ? std::strchr("dDwWntrf", e) == nullptr : std::strchr("dDwWbBAntrf", e) == nullptr) return false;
+            }
+            if (!in_class) can_repeat = !(e == 'b' || e == 'B' || e == 'A');
+            continue;
+        }
+        if (in_class) {
+            if (c == '[') return false;                  // POSIX classes / nested sets
+            if (c == ']' && !(p[i - 1] == '[' || (p[i - 1] == '^' && i >= 2 && p[i - 2] == '['))) { in_class = false; can_repeat = true; }
+            continue;
+        }
+        size_t quantifier_end = 0;   // index of the last byte of a quantifier at i, 0 if none
+        switch (c) {
+            case '[': in_class = true; break;
+            case '(':
+                if (i + 1 < p.size() && p[i + 1] == '?') {   // only (?:
+                    if (i + 2 >= p.size() || p[i + 2] != ':') return false;
+                    i += 2;
+                }
+                can_repeat = false;
+                continue;
+            case ')': can_repeat = true; continue;
+            case '|': case '^': can_repeat = false; continue;
+            case '*': case '+': case '?': quantifier_end = i; break;
+            case '{': {   // {m} {m,} {m,n}
+                size_t j = i + 1;
+                while (j < p.size() && std::isdigit((unsigned char)p[j])) j++;
+                if (j == i + 1) return false;
+                if (j < p.size() && p[j] == ',') {
+                    j++;
+                    while (j < p.size() && std::isdigit((unsigned char)p[j])) j++;
+                }
+                if (j >= p.size() || p[j] != '}') return false;
+                quantifier_end = j;
+                break;
+            }
+            case '}': return false;
+            case '$': return false;
+            default: can_repeat = true; continue;
+        }
+        if (c == '[') continue;
+        if (!can_repeat) return false;
+        i = quantifier_end;
+        if (i + 1 < p.size() && p[i + 1] == '?') i++;   // lazy
+        if (i + 1 < p.size() && (p[i + 1] == '*' || p[i + 1] == '+' || p[i + 1] == '?' || p[i + 1] == '{')) return false;
+        can_repeat = false;
+    }
+    return !in_class;
+}
+
+// pike_vm.hpp cannot include regex.hpp (device code): its assertion codes are the AssertKind values
+static_assert(kPikeBeginBuffer == (uint32_t)AssertKind::BeginBuffer && kPikeWordBoundary == (uint32_t)AssertKind::WordBoundary &&
+                  kPikeNotWordBoundary == (uint32_t)AssertKind::NotWordBoundary,
+              "pike_vm.hpp assertion codes must equal regex.hpp AssertKind values");
+
+// A node that can match without consuming a byte (assertions count as empty).
+bool nullable(const Node& n) { return matches_empty_buffer(n); }
+
+bool repeats_consume(const Node& n) {
+    if (n.kind == NodeKind::Repeat && (n.kids.empty() || nullable(*n.kids[0]))) return false;
+    for (const NodePtr& k : n.kids)
+        if (!repeats_consume(*k)) return false;
+    return true;
+}
+
+// The span program of a screened pattern, or false.
+bool span_program(const std::string& text, PikeProgram& out) {
+    if (!spans_mean_the_same_in_python(text)) return false;
+    ParseResult parsed = parse_regex(text, 0);
+    if (!parsed.root || nullable(*parsed.root) || !repeats_consume(*parsed.root)) return false;
+    Nfa nfa;
+    if (!nfa_add_pattern(nfa, *parsed.root, 0, (size_t)kPikeMaxInsts, /*lazy=*/true)) return false;
+    if (nfa.sets.size() > 256) return false;
+    out.insts.clear();
+    out.sets.clear();
+    for (const NfaInst& in : nfa.prog) {
+        switch (in.op) {
+            case NfaInst::Byte: out.insts.push_back(pike_inst(kPikeByte, (uint32_t)in.arg, (uint32_t)in.x, 0)); break;
+            case NfaInst::Split: out.insts.push_back(pike_inst(kPikeSplit, 0, (uint32_t)in.x, (uint32_t)in.y)); break;
+            case NfaInst::Match: out.insts.push_back(pike_inst(kPikeMatch, 0, 0, 0)); break;
+            case NfaInst::Assert: {
+                const AssertKind k = (AssertKind)in.arg;
+                if (k != AssertKind::BeginBuffer && k != AssertKind::WordBoundary && k != AssertKind::NotWordBoundary) return false;
+                out.insts.push_back(pike_inst(kPikeAssert, (uint32_t)in.arg, (uint32_t)in.x, 0));
+                break;
+            }
+        }
+    }
+    for (const ByteSet& s : nfa.sets)
+        for (int w = 0; w < 4; w++) {
+            out.sets.push_back((uint32_t)s.w[w]);
+            out.sets.push_back((uint32_t)(s.w[w] >> 32));
+        }
+    out.start = nfa.starts[0];
+    return true;
+}
+
 }  // namespace
+
+bool build_pike_program(const char* pattern, PikeProgram& out) { return pattern && span_program(pattern, out); }
+
 }  // namespace gpugrep
 
 struct gpugrep_db {
@@ -127,6 +244,11 @@ int gpugrep_span_width(const char* pattern) {
     if (!parsed.root) return -1;
     const int width = gpugrep::fixed_width(*parsed.root);
     return width > 0 ? width : -1;
+}
+
+int gpugrep_span_exact(const char* pattern) {
+    gpugrep::PikeProgram program;
+    return gpugrep::build_pike_program(pattern, program) ? 1 : 0;
 }
 
 const char* gpugrep_last_error(void) { return gpugrep::g_last_error.c_str(); }

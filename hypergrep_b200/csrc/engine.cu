@@ -11,6 +11,8 @@
 //           k_stream(no filter) -> scan -> k_newline_positions -> pseudo-line table -> k_match_pl_* -> scan -> emit
 // INVERTED scans (grep -v) select the lines without a match: the fast path adds a complement stage after the dedupe
 // (k_invert.cuh, run from slot_collect), the general path negates the per-line flags of k_match_pl_simple.
+// SPANS (grep -o, slot_set_spans): the general path up to the pseudo-line table, then k_spans (count) -> scan -> k_spans (write)
+// instead of the automata (k_spans.cuh).
 // CONTEXT lines (grep -A/-B/-C, scans with records): a window test over the prefix count of the selected lines picks the
 // output lines of a segment (k_context.cuh, after the dedupe on the fast path, after k_match_pl_simple on the general path).
 // All byte offsets inside a segment are 32-bit (segments are < 4 GiB); line numbers are rebased on the host.
@@ -41,6 +43,7 @@
 #include "k_general.cuh"
 #include "k_invert.cuh"
 #include "k_context.cuh"
+#include "k_spans.cuh"
 
 namespace gpugrep {
 
@@ -177,6 +180,7 @@ public:
     DevBuf d_nlpos, d_npl, d_ploff, d_plstart, d_pllen, d_flags, d_counts, d_events, d_gather, d_gidx, d_hitinfo, d_survivors;
     DevBuf d_linebits, d_invrecs;   // inverted fast path: matched-line bitmap, selected-line records (context lines: output records)
     DevBuf d_outbits, d_outoff;     // context lines: output-line bitmap (general path: flags) and its prefix
+    DevBuf d_pike;                  // span stage: the program and its byte sets
     PinBuf h_totals, h_recs, h_stage, h_gather, h_probe;
     // state of the in-flight segment
     const DeviceDb* ddb = nullptr;
@@ -187,10 +191,12 @@ public:
     bool want_records = true;   // false: the caller only counts matches (no callback, no limit): the fast path counts without records
     bool invert = false;        // deliver the lines without a match (slot_set_invert)
     uint32_t ctx_before = 0, ctx_after = 0;   // context lines (slot_set_context)
+    const PikeProgram* pike = nullptr;        // span stage (slot_set_spans)
     SegmentStats stats;
     bool in_use = false;
 
     int run_general(SegmentResult& out, std::string& error, size_t split_above);
+    int run_spans(SegmentResult& out, size_t npl_total, std::string& error, size_t split_above);
     int run_complement(size_t nrec, size_t nlines, size_t selected, std::string& error);
     int run_context(size_t nrec, size_t nlines, size_t selected, size_t& count, std::string& error);
     bool context() const { return want_records && (ctx_before || ctx_after); }
@@ -482,6 +488,7 @@ void engine_release_slot(ScanSlot* slot) {
 
 void slot_set_want_records(ScanSlot* slot, bool want) { slot->want_records = want; }
 void slot_set_invert(ScanSlot* slot, bool invert) { slot->invert = invert; }
+void slot_set_spans(ScanSlot* slot, const PikeProgram* program) { slot->pike = program; }
 void slot_set_context(ScanSlot* slot, uint32_t before, uint32_t after) {
     slot->ctx_before = before;
     slot->ctx_after = after;
@@ -568,7 +575,7 @@ int slot_submit(ScanSlot* s, const DeviceDb& ddb, const DevicePrefilter* pf, con
         while (super_bytes * 4 <= (size_t)buffer_size && super_bytes < 65536) super_bytes *= 2;   // 2*super-1 <= buffer_size-1
     }
     // (NFA-fallback patterns ride the fast path when the exact gram table is there: it tells which candidates they own)
-    s->fast = ddb.simple && pf != nullptr && super_bytes >= 2048 && std::getenv("GPUGREP_FORCE_GENERAL") == nullptr &&
+    s->fast = s->pike == nullptr && ddb.simple && pf != nullptr && super_bytes >= 2048 && std::getenv("GPUGREP_FORCE_GENERAL") == nullptr &&
               (ddb.nnfa == 0 || (pf->mode == 2 && pf->d_confirm != nullptr && std::getenv("GPUGREP_NFA_GENERAL") == nullptr));
 
     if (host_data) {
@@ -798,6 +805,7 @@ int ScanSlot::run_general(SegmentResult& out, std::string& error, size_t split_a
     DbView view{ddb->d_groups, ddb->ngroups, ddb->d_nfas, ddb->nnfa};
     size_t nb_scan = (npl_total + kScanTile - 1) / kScanTile + 1;
     if (d_sums.reserve(nb_scan * 8) != cudaSuccess || d_recoff.reserve(npl_total * 8) != cudaSuccess) { error = "cudaMalloc failed"; return 3; }
+    if (pike) return run_spans(out, npl_total, error, split_above);
     unsigned mgrid = (unsigned)((npl_total + 127) / 128);
     if (ddb->simple) {
         if (d_flags.reserve(npl_total) != cudaSuccess) { error = "cudaMalloc failed"; return 3; }
@@ -867,6 +875,51 @@ int ScanSlot::run_general(SegmentResult& out, std::string& error, size_t split_a
         out.num_events = nev;
     }
     CUDA_TRY(cudaGetLastError());
+    return 0;
+}
+
+// Span stage: the spans of every pseudo-line of the table (d_plstart / d_pllen), in line order, copied to h_recs.
+int ScanSlot::run_spans(SegmentResult& out, size_t npl_total, std::string& error, size_t split_above) {
+    cudaStream_t st = stream;
+    Totals* dT = d_totals.as<Totals>();
+    Totals* hT = h_totals.as<Totals>();
+    const int ninst = (int)pike->insts.size(), nsets = (int)(pike->sets.size() / 8);
+    const size_t words = pike->insts.size() + pike->sets.size();
+    if (d_pike.reserve(words * 4) != cudaSuccess || d_counts.reserve(npl_total * 4) != cudaSuccess) { error = "cudaMalloc failed"; return 3; }
+    uint32_t* prog = d_pike.as<uint32_t>();
+    CUDA_TRY(cudaMemcpyAsync(prog, pike->insts.data(), pike->insts.size() * 4, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(prog + ninst, pike->sets.data(), pike->sets.size() * 4, cudaMemcpyHostToDevice, st));
+    stats.h2d_bytes += words * 4;
+    const size_t smem = words * 4;   // at most 128 instructions and 256 sets: 8.5 KiB
+    const unsigned grid = (unsigned)((npl_total + 127) / 128);
+    k_spans<<<grid, 128, smem, st>>>(prog, ninst, nsets, pike->start, data, d_plstart.as<uint32_t>(), d_pllen.as<uint32_t>(), npl_total,
+                                     d_counts.as<uint32_t>(), nullptr, nullptr);
+    stats.launches++;
+    launch_scan(st, LoadU32{d_counts.as<uint32_t>()}, npl_total, d_recoff.as<unsigned long long>(), d_sums.as<unsigned long long>(), &dT->rec_total, stats);
+    CUDA_TRY(cudaMemcpyAsync(hT, dT, sizeof(Totals), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    const size_t nspan = (size_t)hT->rec_total;
+    if (nspan > ((size_t)1 << 27)) {
+        if (split_above && n > split_above) return kSplitSegment;
+        error = "too many match spans in one segment";
+        return 7;
+    }
+    if (nspan) {
+        if (d_events.reserve(nspan * sizeof(SpanRec)) != cudaSuccess) { error = "cudaMalloc failed"; return 3; }
+        if (h_recs.reserve(nspan * sizeof(SpanRec)) != cudaSuccess) { error = "cudaHostAlloc failed"; return 3; }
+        k_spans<<<grid, 128, smem, st>>>(prog, ninst, nsets, pike->start, data, d_plstart.as<uint32_t>(), d_pllen.as<uint32_t>(), npl_total,
+                                         d_counts.as<uint32_t>(), d_recoff.as<unsigned long long>(), d_events.as<SpanRec>());
+        stats.launches++;
+        CUDA_TRY(cudaEventRecord(ev[1], st));
+        CUDA_TRY(cudaMemcpyAsync(h_recs.p, d_events.p, nspan * sizeof(SpanRec), cudaMemcpyDeviceToHost, st));
+        stats.d2h_bytes += nspan * sizeof(SpanRec);
+    } else {
+        CUDA_TRY(cudaEventRecord(ev[1], st));
+    }
+    CUDA_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaGetLastError());
+    out.spans = h_recs.as<SpanRec>();
+    out.num_spans = nspan;
     return 0;
 }
 

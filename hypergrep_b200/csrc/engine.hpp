@@ -32,6 +32,12 @@ struct EventRec {
     uint32_t report;   // index into Database::report_begin flattened over groups (DeviceDb::accept_base)
 };
 
+// One match span (slot_set_spans): [start, end) relative to the scanned block of pseudo-line `line` (after leading-NUL
+// stripping); start == end == kSpanOverBudget (pike_vm.hpp) marks a line whose search ran over its step budget.
+struct SpanRec {
+    uint32_t line, start, end;
+};
+
 struct SegmentStats {
     double gpu_ms = 0, stream_ms = 0;
     unsigned launches = 0, stream_launches = 0;
@@ -48,9 +54,12 @@ struct SegmentResult {
     size_t num_valid_recs = 0;        // fast path: records whose len is not kLineInvalid (the others must be skipped)
     const EventRec* events = nullptr; // general mode, grouped by line in file order
     size_t num_events = 0;
+    const SpanRec* spans = nullptr;   // span stage (slot_set_spans): by line, then start
+    size_t num_spans = 0;
     SegmentStats stats;
 };
 
+struct PikeProgram;       // span program of one pattern (pike_vm.hpp)
 struct DeviceDb;          // device-resident DFA tables of one Database on one device
 struct DevicePrefilter;   // device-resident gram table of one (sample-tuned) Prefilter
 class ScanSlot;    // stream + scratch + pinned result buffers for one in-flight segment
@@ -97,6 +106,11 @@ __attribute__((weak)) void slot_set_invert(ScanSlot* slot, bool invert);
 // before == after == 0: no context stage.  Call before slot_submit.  Weak like slot_set_invert (a build without it fails
 // context scans with 7).
 __attribute__((weak)) void slot_set_context(ScanSlot* slot, uint32_t before, uint32_t after);
+// Span stage (grep -o, gpugrep_match_spans): the segment takes the general path, and its results are the leftmost-first
+// match spans of `program` in every pseudo-line (SegmentResult::spans) instead of lines or events; null switches it off.
+// `program` stays valid until slot_collect returns.  Call before slot_submit.  Weak like slot_set_invert (a build without it
+// fails span scans with 7).
+__attribute__((weak)) void slot_set_spans(ScanSlot* slot, const PikeProgram* program);
 // Wait for the segment and expose its results (valid until the next slot_submit on this slot).
 // Returns kSplitSegment (and no results) when the fast path hit one of its capacity bounds - a line too long for it, a
 // candidate or record overflow - in a segment of more than `split_above` bytes: the caller then scans the same bytes again

@@ -51,6 +51,7 @@ struct Node {
     ByteSet set;                 // Set
     std::vector<NodePtr> kids;   // Concat / Alt / Repeat(1 kid)
     int min = 0, max = 0;        // Repeat; max < 0 = unbounded
+    bool lazy = false;           // Repeat written with a lazy `?` (same language; only the span program's Split order differs)
     AssertKind assert_kind = AssertKind::BeginBuffer;
 };
 

@@ -151,12 +151,14 @@ private:
             if (!quantifiable) { fail("quantifier does not follow a repeatable item"); return nullptr; }
             if (mx >= 0 && mn > mx) { fail("numbers out of order in {} quantifier"); return nullptr; }
             if (mn > 32767 || mx > 32767) { fail("bounded repeat is too large"); return nullptr; }
-            if (!eof() && peek() == '?') i_++;                     // lazy: same language
+            bool lazy = false;
+            if (!eof() && peek() == '?') { i_++; lazy = true; }   // lazy: same language, recorded for the span program
             else if (!eof() && peek() == '+') { fail("possessive quantifiers are not supported"); return nullptr; }
             if (mx == 0) { atom = mk(NodeKind::Empty); }
             else if (!(mn == 1 && mx == 1)) {
                 auto rep = mk(NodeKind::Repeat);
                 rep->min = mn; rep->max = mx;
+                rep->lazy = lazy;
                 rep->kids.push_back(std::move(atom));
                 atom = std::move(rep);
             }

@@ -7,7 +7,9 @@ CUDA engine: there is no Python/CPU matching fallback, and loading fails loudly 
 
 from __future__ import annotations
 
+import bisect
 import ctypes
+import itertools
 import os
 import re
 import threading
@@ -331,24 +333,32 @@ def grep(  # pylint: disable=too-many-arguments
     if invert_match and only_matching and not count_only:
         return collected, code
 
-    # `-o`: spans from the engine's match END offsets where that is exact (patterns of one fixed width whose syntax means the
-    # same in Python's re; ASCII lines), re.finditer() as in the reference (utils.py:205-212) for everything else.
+    # `-o`: spans from the engine where that is exact (ASCII lines; patterns of one fixed width whose syntax means the same in
+    # Python's re take the match END offsets, other patterns that pass the span screen the leftmost-first match spans),
+    # re.finditer() as in the reference (utils.py:205-212) for everything else.
     widths = _span_widths(patterns) if only_matching else None
-    groups: list[list[tuple[int, str]]] = []      # one entry per record, in record order
-    deferred: list[tuple[int, int, bytes]] = []   # (index into groups, pattern id, line bytes)
+    exact = (_span_exact(patterns) or [False] * len(patterns)) if widths is not None else None
+    groups: list[list[tuple[int, str]]] = []      # one entry per record (or per batch of span-route records), in record order
+    deferred: list[tuple[int, int, bytes]] = []   # fixed-width route: (index into groups, pattern id, line bytes)
+    span_lines = _SpanLines(widths, exact) if widths is not None else None
 
     def _on_batch(matches: ctypes.Array, count: int) -> None:
         if count_only:
             counter[0] += count
+            return
+        if span_lines is not None and span_lines.take_batch(matches, count, groups):
             return
         for position in range(count):
             record = matches[position]
             raw = record.line
             if only_matching:
                 # Same quirk as the reference (utils.py:205-212): record.id is the user id, not the pattern index.
-                if widths is not None and widths[record.id] > 0 and raw.isascii() and raw.endswith(b"\n"):
-                    deferred.append((len(groups), record.id, raw))
-                    groups.append([(record.line_number + 1, "")])
+                if widths is not None and (widths[record.id] > 0 or exact[record.id]) and raw.isascii() and raw.endswith(b"\n"):
+                    if widths[record.id] > 0:
+                        deferred.append((len(groups), record.id, raw))
+                        groups.append([(record.line_number + 1, "")])
+                    else:
+                        span_lines.add(record.id, [record.line_number], [raw], groups)
                     continue
                 text = raw.decode(errors=errors)
                 groups.append([(record.line_number + 1, f"{part.group()}\n") for part in python_patterns[record.id].finditer(text)])
@@ -375,7 +385,7 @@ def grep(  # pylint: disable=too-many-arguments
         after_context=after_context if context else 0,
     )
     if only_matching:
-        _fill_spans(groups, deferred, patterns, widths, python_patterns, errors)
+        _fill_spans(groups, deferred, patterns, widths, python_patterns, errors, span_lines)
         collected = [entry for group in groups for entry in group]
     return (counter[0] if count_only else collected), code
 
@@ -400,14 +410,141 @@ def _span_widths(patterns: Sequence[str]) -> list[int] | None:
     return [width(pattern.encode()) for pattern in patterns]
 
 
+class _MatchSpan(ctypes.Structure):
+    """gpugrep_match_span (include/gpugrep.h)."""
+
+    _fields_ = [("line_number", ctypes.c_ulonglong), ("start", ctypes.c_uint), ("end", ctypes.c_uint)]
+
+
+_SPAN_OVER_BUDGET = 0xFFFFFFFF
+
+
+def _span_exact(patterns: Sequence[str]) -> list[bool] | None:
+    """Per pattern: True if the engine's leftmost-first match spans equal re.finditer() (gpugrep_span_exact), or None if the
+    loaded library cannot compute spans."""
+    lib = _get_hyperscanner_lib()
+    try:
+        exact = lib.gpugrep_span_exact
+        lib.gpugrep_match_spans  # pylint: disable=pointless-statement
+    except AttributeError:
+        return None
+    exact.restype = ctypes.c_int
+    exact.argtypes = [ctypes.c_char_p]
+    return [exact(pattern.encode()) == 1 for pattern in patterns]
+
+
+class _SpanLines:
+    """The records of the span route, per pattern id: ASCII lines ending in '\\n' of variable-width patterns that pass
+    gpugrep_span_exact.  Whole batches are taken without a Python step per record: ids, line numbers and line pointers are
+    read as three strided slices of the batch, and one isascii() / newline count over the joined lines checks the batch."""
+
+    def __init__(self, widths: list[int], exact: list[bool]):
+        self.routed = [width <= 0 and bool(ok) for width, ok in zip(widths, exact)]
+        self.lines: dict[int, list] = {}   # pattern id -> [joined chunks, line numbers, line bytes, (output list, first, count)]
+
+    def __len__(self) -> int:
+        return sum(len(entry[1]) for entry in self.lines.values())
+
+    def add(self, pattern_id: int, numbers: list[int], raws: list[bytes], groups: list, blob: bytes | None = None) -> None:
+        entry = self.lines.setdefault(pattern_id, [[], [], [], []])
+        out: list = []
+        groups.append(out)   # filled by fill() with the entries of these lines
+        entry[3].append((out, len(entry[1]), len(numbers)))
+        entry[0].append(blob if blob is not None else b"".join(raws))
+        entry[1].extend(numbers)
+        entry[2].extend(raws)
+
+    def take_batch(self, matches, count: int, groups: list) -> bool:
+        """Takes the whole batch if every record belongs to one routed pattern and every line is ASCII and ends in '\\n'."""
+        if count <= 0 or not any(self.routed):
+            return False
+        base = ctypes.cast(matches, ctypes.c_void_p).value   # hyperscanner_result_t: id @0, line_number @8, line @16
+        ids = (ctypes.c_uint * (6 * count)).from_address(base)[0::6]
+        pattern_id = ids[0]
+        if pattern_id >= len(self.routed) or not self.routed[pattern_id] or ids.count(pattern_id) != count:
+            return False
+        raws = (ctypes.c_char_p * (3 * count)).from_address(base)[2::3]
+        blob = b"".join(raws)
+        # (a delivered line holds at most one '\\n', its last byte)
+        if not blob.isascii() or blob.count(b"\n") != count:
+            return False
+        self.add(pattern_id, (ctypes.c_ulonglong * (3 * count)).from_address(base)[1::3], raws, groups, blob)
+        return True
+
+    def fill(self, patterns: Sequence[str], python_patterns: list, errors: str) -> None:
+        for pattern_id, (chunks, numbers, raws, segments) in self.lines.items():
+            entries, first_line = _span_entries(b"".join(chunks), numbers, raws, patterns[pattern_id], python_patterns[pattern_id], errors)
+            for out, first, count in segments:
+                lo = bisect.bisect_left(first_line, first)
+                out.extend(entries[lo:bisect.bisect_left(first_line, first + count, lo)])
+
+
+def _span_entries(text: bytes, numbers: list[int], raws: list[bytes], pattern: str, python_pattern, errors: str):
+    """The `-o` entries (line number, part + '\\n') of the lines joined in `text`, from one gpugrep_match_spans call, and the
+    index of the line of each entry.  A failed call, or a line over the step budget, takes re.finditer()."""
+    lib = _get_hyperscanner_lib()
+    spans = None
+    found = ctypes.c_size_t(0)
+    entry = getattr(lib, "gpugrep_match_spans", None)
+    if entry is not None:
+        entry.restype = ctypes.c_int
+        entry.argtypes = [ctypes.c_char_p, ctypes.c_size_t, ctypes.c_int, ctypes.c_char_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_size_t,
+                          ctypes.POINTER(ctypes.c_size_t), ctypes.c_void_p]
+        capacity = 2 * len(numbers) + 1024
+        for _ in range(2):
+            spans = (_MatchSpan * capacity)()
+            code = entry(text, len(text), 0, pattern.encode(), 262140, spans, capacity, ctypes.byref(found), None)
+            if code != 0:
+                spans = None
+                break
+            if found.value <= capacity:
+                break
+            capacity, spans = found.value, None
+    if spans is None:
+        entries, first_line = [], []
+        for line, raw in enumerate(raws):
+            parts = [(numbers[line] + 1, f"{part.group()}\n") for part in python_pattern.finditer(raw.decode(errors=errors))]
+            entries += parts
+            first_line += [line] * len(parts)
+        return entries, first_line
+    # the records as 32-bit words (line_number low / high, start, end), read in one step
+    total = found.value
+    words = (ctypes.c_uint * (4 * total)).from_buffer(spans)[:] if total else []
+    lines, starts, ends = words[0::4], words[2::4], words[3::4]
+    offsets = list(itertools.accumulate(map(len, raws), initial=0))
+    whole = text.decode("ascii")
+    if _SPAN_OVER_BUDGET not in starts:
+        return [(numbers[line] + 1, whole[offsets[line] + start:offsets[line] + end] + "\n")
+                for line, start, end in zip(lines, starts, ends)], lines
+    entries, first_line = [], []
+    for line, start, end in zip(lines, starts, ends):
+        if start == _SPAN_OVER_BUDGET:
+            parts = [(numbers[line] + 1, f"{part.group()}\n") for part in python_pattern.finditer(raws[line].decode(errors=errors))]
+            entries += parts
+            first_line += [line] * len(parts)
+        else:
+            entries.append((numbers[line] + 1, whole[offsets[line] + start:offsets[line] + end] + "\n"))
+            first_line.append(line)
+    return entries, first_line
+
+
 def _fill_spans(groups: list, deferred: list, patterns: Sequence[str], widths: list[int] | None, python_patterns: list,
-                errors: str) -> None:
-    """SURVEY.md section 8(f-4): the spans of the deferred records from ONE scan of their lines that reports every match
-    end (gpugrep_match_ends, patterns compiled without flags like the reference's re.compile(pattern)).  A pattern of
-    fixed width w matches [end - w, end); finditer()'s left-to-right, non-overlapping choice is a greedy pass over the
-    ends.  Any failure falls back to re.finditer() for those records."""
-    if not deferred:
-        return
+                errors: str, span_lines: _SpanLines | None = None) -> None:
+    """SURVEY.md section 8(f-4): the spans of the records that the engine's answers cover.  Patterns of one fixed width
+    (`deferred`) take ONE scan of their lines that reports every match end (gpugrep_match_ends, patterns compiled without
+    flags like the reference's re.compile(pattern)): a pattern of fixed width w matches [end - w, end), and finditer()'s
+    left-to-right, non-overlapping choice is a greedy pass over the ends.  The other patterns that pass the span screen
+    (`span_lines`) take one gpugrep_match_spans call per pattern id, which returns the finditer() spans themselves.  Any
+    failure falls back to re.finditer() for the records concerned."""
+    if span_lines is not None:
+        span_lines.fill(patterns, python_patterns, errors)
+    if deferred:
+        _fill_from_ends(groups, deferred, patterns, widths, python_patterns, errors)
+
+
+def _fill_from_ends(groups: list, deferred: list, patterns: Sequence[str], widths: list[int], python_patterns: list,
+                    errors: str) -> None:
+    """The spans of fixed-width records from their match ends (gpugrep_match_ends)."""
     lib = _get_hyperscanner_lib()
     entry = lib.gpugrep_match_ends
     entry.restype = ctypes.c_int

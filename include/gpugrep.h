@@ -174,6 +174,34 @@ GPUGREP_API int gpugrep_match_ends(const void* data, size_t size, int location, 
  * sorted ends.  Host only (no CUDA). */
 GPUGREP_API int gpugrep_span_width(const char* pattern);
 
+/* 1 if `pattern` (compiled WITHOUT flags) is accepted by gpugrep_match_spans(), else 0.  Accepted patterns use only syntax that
+ * Python's re and this compiler read the same way (literals, classes without POSIX names, . \d \D \w \W \b \B \A ^, groups
+ * and (?:...), alternation, * + ? {m} {m,} {m,n} and their lazy forms); they cannot match the empty string, no repeated item
+ * can match it either, and the span program has at most 128 instructions.  Rejected, among others: {,n}, $, \s, inline flags,
+ * POSIX classes, possessive quantifiers and non-ASCII bytes.  Host only (no CUDA). */
+GPUGREP_API int gpugrep_span_exact(const char* pattern);
+
+/* ---- leftmost-first match spans (`grep -o` of any pattern that passes gpugrep_span_exact) ----------------------------------
+ * One record per match, in line order and then start order.  For every pseudo-line (split as hyperscan() splits them), the
+ * records of its scanned block (leading NULs skipped, cut at the next NUL, the trailing '\n' included) are, on every byte
+ * value, exactly [m.span() for m in re.compile(pattern.encode()).finditer(block)]: the leftmost start, then the end a
+ * backtracking matcher picks (greedy and lazy quantifiers and alternation order count), each search resuming at the previous
+ * end.  Python's bytes patterns are ASCII, so on ASCII blocks the spans also equal those of the str finditer.  `pattern` is
+ * compiled without flags; one that fails gpugrep_span_exact returns 4.  A block whose searches need more than
+ * min(128 * (length + 1), 2^25) thread steps (searches that rescan the block, such as `a.*b|a` on a long run of `a`, or
+ * programs near the instruction cap on long lines) yields one record with start == end == GPUGREP_SPAN_OVER_BUDGET and no
+ * other record: the caller finds its spans another way.  Capacity, retry and return codes as gpugrep_match_ends().
+ * A build of the engine without the span stage returns 7. */
+#define GPUGREP_SPAN_OVER_BUDGET 0xFFFFFFFFu
+typedef struct gpugrep_match_span {
+    unsigned long long line_number; /* 0-based pseudo-line index inside `data` */
+    unsigned int start;             /* offset of the first byte of the match   */
+    unsigned int end;               /* offset just behind the match            */
+} gpugrep_match_span;
+
+GPUGREP_API int gpugrep_match_spans(const void* data, size_t size, int location, const char* pattern, int buffer_size,
+                        gpugrep_match_span* out, size_t capacity, size_t* count, gpugrep_stats* stats);
+
 /* An hs_event that discards its batch (benchmarks: full delivery path without a Python frame per batch). */
 GPUGREP_API void gpugrep_discard_results(hyperscanner_result_t* results, int result_count);
 
