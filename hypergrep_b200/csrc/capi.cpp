@@ -533,6 +533,7 @@ struct Params {
     const PikeProgram* span_program = nullptr;
     bool invert = false;        // gpugrep_invert_scan_*(): deliver the pseudo-lines in which no pattern reports
     bool context_scan = false;  // gpugrep_context_scan_*(): lines around the selected ones too
+    bool literal = false;       // gpugrep_literal_scan_*(): `patterns` are fixed strings (flags: CASELESS only, no ids)
     uint32_t before = 0, after = 0;
     // the context stage runs only when lines are delivered (count-only scans ignore context)
     bool context() const { return context_scan && cb != nullptr && (before || after); }
@@ -560,11 +561,15 @@ void set_context(ScanSlot* slot, const Params& pr) {
 void set_spans(ScanSlot* slot, const Params& pr) {
     if (slot_set_spans) slot_set_spans(slot, pr.span_program);
 }
+void set_literals(ScanSlot* slot, const Params& pr) {
+    if (slot_set_literals) slot_set_literals(slot, pr.literal);
+}
 
 int setup_job(const Params& pr, Job& job, Deliverer& out, unsigned long long weight = 0) {
     int rc = 0;
-    job.db = cached_database(pr.patterns, pr.flags, pr.ids, pr.elements, rc, job.error);
-    if (job.db && (pr.invert || pr.context_scan)) {
+    if (pr.literal) job.db = cached_literal_database(pr.patterns, pr.flags, pr.elements, rc, job.error);
+    else job.db = cached_database(pr.patterns, pr.flags, pr.ids, pr.elements, rc, job.error);
+    if (job.db && !pr.literal && (pr.invert || pr.context_scan)) {
         // Which lines match does not depend on ids or SINGLEMATCH: once the set compiles as given, it is scanned as "every
         // pattern SINGLEMATCH, one id 0" (simple mode, so multi-id sets take the fast path too), CASELESS/DOTALL/MULTILINE kept.
         std::vector<unsigned> flags(pr.elements), ids(pr.elements, 0u);
@@ -579,6 +584,7 @@ int setup_job(const Params& pr, Job& job, Deliverer& out, unsigned long long wei
     if (pr.invert && !slot_set_invert) { job.error = "this build of the engine has no inverted scan"; return GPUGREP_SCAN; }
     if (pr.context_scan && !slot_set_context) { job.error = "this build of the engine has no context lines"; return GPUGREP_SCAN; }
     if (pr.span_program && !slot_set_spans) { job.error = "this build of the engine has no span stage"; return GPUGREP_SCAN; }
+    if (pr.literal && !slot_set_literals) { job.error = "this build of the engine has no fixed-string stage"; return GPUGREP_SCAN; }
     job.device_weight = weight;
     job.device = pick_device(weight, &job.device_charged);
     if (engine_select_device(job.device, job.error) != 0) {
@@ -691,6 +697,7 @@ int scan_file(const char* path, const Params& pr, gpugrep_stats* stats_out, cons
         set_invert(sl, pr.invert);
         set_context(sl, pr);
         set_spans(sl, pr);
+        set_literals(sl, pr);
     }
     SegmentQueue q;
     for (int i = 0; i < kSlots; i++) q.free_slots.push_back(i);
@@ -861,6 +868,7 @@ int scan_memory(const uint8_t* data, size_t size, int location, const Params& pr
         set_invert(sl, pr.invert);
         set_context(sl, pr);
         set_spans(sl, pr);
+        set_literals(sl, pr);
     }
     const uint8_t* seg_host[2] = {nullptr, nullptr};
     const uint8_t* seg_dev[2] = {nullptr, nullptr};
@@ -1244,6 +1252,30 @@ int gpugrep_context_scan_buffer(const void* data, size_t size, int location, con
                                 unsigned long long max_match_count, unsigned int before, unsigned int after, int invert, void* stream,
                                 gpugrep_stats* stats) {
     gpugrep::Params pr{patterns, pattern_flags, pattern_ids, elements, on_event, buffer_size, buffer_count, max_match_count, stream};
+    pr.invert = invert != 0;
+    pr.context_scan = true;
+    pr.before = before;
+    pr.after = after;
+    return gpugrep::scan_buffer(data, size, location, pr, stats);
+}
+
+int gpugrep_literal_scan_file(const char* file_name, const char* const* literals, const unsigned int* literal_flags, unsigned int elements,
+                              hs_event on_event, int buffer_size, int buffer_count, unsigned long long max_match_count, unsigned int before,
+                              unsigned int after, int invert, gpugrep_stats* stats) {
+    gpugrep::Params pr{literals, literal_flags, nullptr, elements, on_event, buffer_size, buffer_count, max_match_count, nullptr};
+    pr.literal = true;
+    pr.invert = invert != 0;
+    pr.context_scan = true;
+    pr.before = before;
+    pr.after = after;
+    return gpugrep::scan_path(file_name, pr, stats);
+}
+
+int gpugrep_literal_scan_buffer(const void* data, size_t size, int location, const char* const* literals, const unsigned int* literal_flags,
+                                unsigned int elements, hs_event on_event, int buffer_size, int buffer_count, unsigned long long max_match_count,
+                                unsigned int before, unsigned int after, int invert, void* stream, gpugrep_stats* stats) {
+    gpugrep::Params pr{literals, literal_flags, nullptr, elements, on_event, buffer_size, buffer_count, max_match_count, stream};
+    pr.literal = true;
     pr.invert = invert != 0;
     pr.context_scan = true;
     pr.before = before;

@@ -236,6 +236,13 @@ int check_patterns(const char* const* patterns, const unsigned int* pattern_flag
     return 0;
 }
 
+int gpugrep_check_literals(const char* const* literals, const unsigned int* literal_flags, unsigned int elements) {
+    std::string err;
+    const int rc = gpugrep::check_literals(literals, literal_flags, elements, err);
+    gpugrep::set_last_error(err);
+    return rc;
+}
+
 int gpugrep_span_width(const char* pattern) {
     if (!pattern) return -1;
     const std::string text(pattern);

@@ -3,6 +3,9 @@
 
 #include <algorithm>
 #include <cstdlib>
+#include <cstring>
+#include <functional>
+#include <string_view>
 #include <list>
 #include <future>
 #include <map>
@@ -174,11 +177,36 @@ int compile_database(const char* const* patterns, const unsigned* flags, const u
     return 0;
 }
 
-std::shared_ptr<Database> cached_database(const char* const* patterns, const unsigned* flags, const unsigned* ids,
-                                          unsigned n, int& rc, std::string& error) {
+namespace {
+
+// Most recent first; a fixed-string set and a regex set never share an entry, whatever their keys.
+std::shared_ptr<Database> cached(bool literal, std::string key, const std::function<int(std::shared_ptr<Database>&)>& compile, int& rc) {
     static std::mutex mu;
-    static std::list<std::shared_ptr<Database>> cache;   // most recent first
-    // (built for every scan call: 10,000 patterns are 300 KB of key, so no per-pattern formatting or allocation here)
+    static std::list<std::shared_ptr<Database>> cache;
+    {
+        std::lock_guard<std::mutex> lk(mu);
+        for (auto it = cache.begin(); it != cache.end(); ++it) {
+            if ((*it)->literal == literal && (*it)->key == key) {
+                auto db = *it;
+                cache.erase(it);
+                cache.push_front(db);
+                rc = 0;
+                return db;
+            }
+        }
+    }
+    std::shared_ptr<Database> db;
+    rc = compile(db);
+    if (rc != 0) return nullptr;
+    db->key = std::move(key);
+    std::lock_guard<std::mutex> lk(mu);
+    cache.push_front(db);
+    while (cache.size() > 8) cache.pop_back();
+    return db;
+}
+
+// (built for every scan call: 10,000 patterns are 300 KB of key, so no per-pattern formatting or allocation here)
+std::string cache_key(const char* const* patterns, const unsigned* flags, const unsigned* ids, unsigned n) {
     std::string key;
     key.reserve((size_t)n * 48 + 64);
     for (unsigned i = 0; i < n; i++) {
@@ -189,27 +217,132 @@ std::shared_ptr<Database> cached_database(const char* const* patterns, const uns
         key.append(reinterpret_cast<const char*>(tail), sizeof(tail));
     }
     key.append(std::getenv("GPUGREP_NO_PREFILTER") ? "np" : "");
+    return key;
+}
+
+}  // namespace
+
+std::shared_ptr<Database> cached_database(const char* const* patterns, const unsigned* flags, const unsigned* ids,
+                                          unsigned n, int& rc, std::string& error) {
+    std::string key = cache_key(patterns, flags, ids, n);
     if (const char* b = std::getenv("GPUGREP_MAX_DFA_STATES")) key.append(b);
-    {
-        std::lock_guard<std::mutex> lk(mu);
-        for (auto it = cache.begin(); it != cache.end(); ++it) {
-            if ((*it)->key == key) {
-                auto db = *it;
-                cache.erase(it);
-                cache.push_front(db);
-                rc = 0;
-                return db;
-            }
+    return cached(false, std::move(key), [&](std::shared_ptr<Database>& db) { return compile_database(patterns, flags, ids, n, db, error); }, rc);
+}
+
+// ---- fixed strings ----------------------------------------------------------------------------------------------
+int check_literals(const char* const* literals, const unsigned* flags, unsigned n, std::string& error) {
+    const int kDbError = 4;
+    if (n == 0 || !literals) { error = "no literals"; return kDbError; }
+    for (unsigned i = 0; i < n; i++) {
+        if (!literals[i] || !literals[i][0]) { error = "literal " + std::to_string(i) + " is empty"; return kDbError; }
+        if (flags && (flags[i] & ~(FLAG_CASELESS | FLAG_DOTALL | FLAG_MULTILINE | FLAG_SINGLEMATCH))) {
+            error = "literal " + std::to_string(i) + ": unsupported flag bits";
+            return kDbError;
         }
     }
-    std::shared_ptr<Database> db;
-    rc = compile_database(patterns, flags, ids, n, db, error);
-    if (rc != 0) return nullptr;
-    db->key = key;
-    std::lock_guard<std::mutex> lk(mu);
-    cache.push_front(db);
-    while (cache.size() > 8) cache.pop_back();
-    return db;
+    return 0;
+}
+
+int compile_literal_database(const char* const* literals, const unsigned* flags, unsigned n, std::shared_ptr<Database>& out,
+                             std::string& error) {
+    int rc = check_literals(literals, flags, n, error);
+    if (rc) return rc;
+    auto db = std::make_shared<Database>();
+    db->simple = true;
+    db->simple_id = 0;
+    db->literal = true;
+    LiteralSet& L = db->literals;
+    L.given = n;
+    // folded candidates per class, sorted; a literal with '\n' before its last byte can never lie inside a line
+    struct Cand { std::string_view text; unsigned cls; };
+    std::vector<std::string> folded(n);
+    std::vector<Cand> cands;
+    cands.reserve(n);
+    for (unsigned i = 0; i < n; i++) {
+        const size_t len = std::strlen(literals[i]);
+        const char* nl = static_cast<const char*>(std::memchr(literals[i], '\n', len));
+        if (nl && nl != literals[i] + len - 1) continue;
+        const unsigned cls = flags && (flags[i] & FLAG_CASELESS) ? 1u : 0u;
+        folded[i].assign(literals[i], len);
+        if (cls) for (char& c : folded[i]) c = (char)fold_ascii((uint8_t)c);
+        cands.push_back(Cand{folded[i], cls});
+    }
+    std::sort(cands.begin(), cands.end(), [](const Cand& a, const Cand& b) { return a.cls != b.cls ? a.cls < b.cls : a.text < b.text; });
+    // prefix-free per class: in sorted order every string that has a kept prefix follows that prefix directly
+    std::vector<Cand> kept;
+    for (const Cand& c : cands) {
+        if (!kept.empty() && kept.back().cls == c.cls && c.text.substr(0, kept.back().text.size()) == kept.back().text) continue;
+        kept.push_back(c);
+    }
+    L.bucket.assign(2 * 65537, 0);
+    L.one.assign(2 * 8, 0);
+    size_t total = 0;
+    for (const Cand& c : kept) total += c.text.size();
+    L.bytes.reserve(total);
+    std::vector<uint32_t> count(2 * 65536, 0);
+    for (const Cand& c : kept) {
+        const uint32_t id = (uint32_t)L.off.size();
+        L.off.push_back((uint32_t)L.bytes.size());
+        L.len.push_back((uint32_t)c.text.size());
+        L.caseless.push_back((uint8_t)c.cls);
+        L.bytes.insert(L.bytes.end(), c.text.begin(), c.text.end());
+        const uint8_t b0 = (uint8_t)c.text[0];
+        if (c.text.size() == 1) {
+            L.one[c.cls * 8 + b0 / 32] |= 1u << (b0 % 32);
+            L.rank.push_back(0);
+        } else {
+            L.rank.push_back((uint32_t)L.order.size());
+            L.order.push_back(id);
+            count[c.cls * 65536 + ((uint32_t)b0 << 8 | (uint8_t)c.text[1])]++;
+        }
+    }
+    // (order is sorted by class, then bytes: the literals of one two-byte prefix are one range of it)
+    uint32_t at = 0;
+    for (unsigned cls = 0; cls < 2; cls++) {
+        for (uint32_t k = 0; k < 65536; k++) {
+            L.bucket[cls * 65537 + k] = at;
+            at += count[cls * 65536 + k];
+        }
+        L.bucket[cls * 65537 + 65536] = at;
+    }
+    // one class-string per literal: the prefilter picks a rare window in each (caseless letters: both cases)
+    const size_t m = L.off.size();
+    FactorSet& fs = db->factors;
+    fs.factors.resize(m);
+    fs.before.assign(m, 0);
+    fs.literal_rank = L.rank;
+    fs.literal_class = L.caseless;
+    size_t min_len = m ? SIZE_MAX : 0;
+    for (size_t i = 0; i < m; i++) {
+        ClassString s(L.len[i]);
+        for (uint32_t k = 0; k < L.len[i]; k++) {
+            const uint8_t b = L.bytes[L.off[i] + k];
+            s[k].set(b);
+            if (L.caseless[i] && (unsigned)b - 'a' < 26u) s[k].set(b & ~0x20u);
+        }
+        fs.factors[i].push_back(std::move(s));
+        min_len = std::min<size_t>(min_len, L.len[i]);
+    }
+    fs.min_len = min_len;
+    fs.usable = m > 0 && min_len >= 4;
+    if (!fs.usable) fs.note = m ? "a literal is shorter than 4 bytes" : "no literal can match";
+    if (fs.usable && env_size("GPUGREP_NO_PREFILTER", 0) != 0) {
+        fs.usable = false;
+        db->prefilter.note = fs.note = "disabled by GPUGREP_NO_PREFILTER";
+    }
+    if (fs.usable) build_prefilter(fs, nullptr, db->prefilter);
+    else if (db->prefilter.note.empty()) db->prefilter.note = fs.note;
+    PatternInfo info;
+    info.source = "(" + std::to_string(n) + " literals)";
+    db->patterns.push_back(std::move(info));
+    out = db;
+    return 0;
+}
+
+std::shared_ptr<Database> cached_literal_database(const char* const* literals, const unsigned* flags, unsigned n, int& rc,
+                                                  std::string& error) {
+    return cached(true, cache_key(literals, flags, nullptr, n),
+                  [&](std::shared_ptr<Database>& db) { return compile_literal_database(literals, flags, n, db, error); }, rc);
 }
 
 }  // namespace gpugrep

@@ -35,6 +35,22 @@ struct NfaPattern {
     uint32_t report_begin = 0;   // its single report: Database::reports[report_begin]
 };
 
+// Fixed-string set (grep -F): the literals that can select a line, without automata.  A literal with an inner '\n' never
+// matches and is dropped; so is one that has another literal of its class as a prefix (the shorter one matches wherever the
+// longer one does).  What is kept is prefix-free per class, so at any text position at most one literal of a class can
+// match: the largest one not above the text, found by binary search.
+struct LiteralSet {
+    std::vector<uint8_t> bytes;          // the kept literals, caseless ones folded to lower case (A-Z only)
+    std::vector<uint32_t> off, len;      // per kept literal: offset into bytes, length
+    std::vector<uint8_t> caseless;       // per kept literal: class 1 (compared folded) or 0 (exact)
+    std::vector<uint32_t> rank;          // per kept literal: position in `order` (sorted by folded bytes within the class)
+    std::vector<uint32_t> order;         // class 0 literals of >= 2 bytes in byte order, then those of class 1
+    std::vector<uint32_t> bucket;        // [class][65537]: the literals of `order` whose first two bytes are (b0 << 8 | b1) are
+                                         // order[bucket[k] .. bucket[k + 1])
+    std::vector<uint32_t> one;           // [class][8]: bitmap of the one-byte literals
+    unsigned given = 0;                  // literals passed in
+};
+
 struct Database {
     std::vector<PatternInfo> patterns;
     std::vector<NfaPattern> nfas;
@@ -48,6 +64,8 @@ struct Database {
     FactorSet factors;       // required factors per pattern (input of the prefilter builder)
     Prefilter prefilter;     // statically chosen windows (used when no input sample is available)
     std::string key;   // cache key: patterns + flags + ids
+    bool literal = false;   // fixed-string set: no groups, `literals` holds what a line is matched against
+    LiteralSet literals;
 };
 
 // Return codes follow the reference's enum (hyperscanner.c:25-33): 0 ok, 4 = HYPERSCANNER_DB for any rejection.
@@ -58,5 +76,16 @@ int compile_database(const char* const* patterns, const unsigned* flags, const u
 // Process-wide cache (the reference recompiles per call, hyperscanner.c:296; SURVEY.md §8f-3).
 std::shared_ptr<Database> cached_database(const char* const* patterns, const unsigned* flags, const unsigned* ids,
                                           unsigned n, int& rc, std::string& error);
+
+// Fixed strings (gpugrep_literal_scan_*): `n` >= 1 non-empty literals, flags CASELESS (honoured) and DOTALL / MULTILINE /
+// SINGLEMATCH (accepted, they change nothing).  Returns 0 or 4 like compile_database.
+int check_literals(const char* const* literals, const unsigned* flags, unsigned n, std::string& error);
+int compile_literal_database(const char* const* literals, const unsigned* flags, unsigned n, std::shared_ptr<Database>& out,
+                             std::string& error);
+// Cached like cached_database, apart from it: the literal "a.b" is not the regex "a.b".
+std::shared_ptr<Database> cached_literal_database(const char* const* literals, const unsigned* flags, unsigned n, int& rc,
+                                                  std::string& error);
+
+inline uint8_t fold_ascii(uint8_t b) { return (uint8_t)((unsigned)b - 'A' < 26u ? b | 0x20u : b); }
 
 }  // namespace gpugrep

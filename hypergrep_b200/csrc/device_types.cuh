@@ -37,6 +37,9 @@ constexpr uint32_t kHasNulBit = 0x80000000u;    // LineRec.len flag: the line co
 constexpr unsigned int kFallbackFlags = 7u;      // Totals::flags bits that send a fast-path segment to the general path
 constexpr unsigned int kSegmentNulFlag = 8u;     // Totals::flags bit: some byte of the segment is NUL
 
+constexpr int kEmitThreads = 256;
+constexpr int kEmitTile = 512;    // candidates per emit step (and per record-offset entry): small enough that sparse candidate lists still spread over all SMs
+
 struct Totals {
     unsigned long long meta_total;   // candidates << 32 | newlines
     unsigned long long rec_total;    // records to emit (fast path) / generic scan totals

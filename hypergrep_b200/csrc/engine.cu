@@ -13,6 +13,8 @@
 // (k_invert.cuh, run from slot_collect), the general path negates the per-line flags of k_match_pl_simple.
 // SPANS (grep -o, slot_set_spans): the general path up to the pseudo-line table, then k_spans (count) -> scan -> k_spans (write)
 // instead of the automata (k_spans.cuh).
+// FIXED STRINGS (grep -F, slot_set_literals): the same two paths without automata; k_verify_literals takes the place of the
+// DFA verification (k_confirm always runs before it) and k_match_pl_literals that of k_match_pl_simple (k_literal.cuh).
 // CONTEXT lines (grep -A/-B/-C, scans with records): a window test over the prefix count of the selected lines picks the
 // output lines of a segment (k_context.cuh, after the dedupe on the fast path, after k_match_pl_simple on the general path).
 // All byte offsets inside a segment are 32-bit (segments are < 4 GiB); line numbers are rebased on the host.
@@ -39,6 +41,7 @@
 #include "k_stream.cuh"
 #include "scan.cuh"
 #include "dfa_walk.cuh"
+#include "k_literal.cuh"
 #include "k_fast.cuh"
 #include "k_general.cuh"
 #include "k_invert.cuh"
@@ -137,6 +140,8 @@ struct DeviceDb {
     int nnfa = 0;
     bool simple = false;
     size_t smem_table_bytes = 0;   // single group with a class-compressed table (GroupDev::ctab): its size, else 0
+    bool literal = false;          // fixed-string set: `lits` instead of groups
+    LiteralView lits{};
     ~DeviceDb() { for (void* p : allocs) cudaFree(p); }
 };
 
@@ -160,7 +165,10 @@ struct DevicePrefilter {
     uint32_t confirm_mul = 0, confirm_mul2 = 0;
     double bloom_false_rate = 0;     // expected share of 16-byte chunks flagged by bloom collisions alone
     double expected_hits_per_mib = -1;   // gram hits per MiB of the tuning sample (-1: no sample)
+    LiteralIndex lit_index{};            // fixed-string sets: Prefilter::lit_begin / lit_entries (null otherwise)
     ~DevicePrefilter() {
+        if (lit_index.begin) cudaFree((void*)lit_index.begin);
+        if (lit_index.entries) cudaFree((void*)lit_index.entries);
         if (d_table) cudaFree(d_table);
         if (d_confirm) cudaFree(d_confirm);
         if (d_confirm_groups) cudaFree(d_confirm_groups);
@@ -192,6 +200,7 @@ public:
     bool invert = false;        // deliver the lines without a match (slot_set_invert)
     uint32_t ctx_before = 0, ctx_after = 0;   // context lines (slot_set_context)
     const PikeProgram* pike = nullptr;        // span stage (slot_set_spans)
+    bool literal = false;                     // fixed-string scan (slot_set_literals)
     SegmentStats stats;
     bool in_use = false;
 
@@ -249,6 +258,22 @@ std::shared_ptr<DeviceDb> engine_upload(const std::shared_ptr<Database>& db, std
         if (bytes && cudaMemcpy(p, src, bytes, cudaMemcpyHostToDevice) != cudaSuccess) return nullptr;
         return p;
     };
+    if (db->literal) {
+        const LiteralSet& L = db->literals;
+        std::vector<uint8_t> bytes(L.bytes);
+        bytes.resize(bytes.size() + 16, 0);   // (k_literal.cuh lit_compare: 8-byte loads)
+        LiteralView v{};
+        v.bytes = (const uint8_t*)upload(bytes.data(), bytes.size());
+        v.off = (const uint32_t*)upload(L.off.data(), L.off.size() * 4);
+        v.len = (const uint32_t*)upload(L.len.data(), L.len.size() * 4);
+        v.order = (const uint32_t*)upload(L.order.data(), L.order.size() * 4);
+        v.bucket = (const uint32_t*)upload(L.bucket.data(), L.bucket.size() * 4);
+        v.one = (const uint32_t*)upload(L.one.data(), L.one.size() * 4);
+        for (uint8_t c : L.caseless) v.classes |= 1u << c;
+        if (!v.bytes || !v.off || !v.len || !v.order || !v.bucket || !v.one) { error = "cudaMalloc/cudaMemcpy failed while uploading the literals"; return nullptr; }
+        out->literal = true;
+        out->lits = v;
+    }
     std::vector<GroupDev> groups;
     for (size_t g = 0; g < db->groups.size(); g++) {
         const Dfa& d = db->groups[g].dfa;
@@ -425,6 +450,16 @@ std::shared_ptr<DevicePrefilter> engine_upload_prefilter(const Prefilter& pf, st
             }
         }
     }
+    if (!pf.lit_begin.empty() && out->d_confirm) {
+        void* b = nullptr;
+        void* e = nullptr;
+        const bool ok = cudaMalloc(&b, pf.lit_begin.size() * 4) == cudaSuccess && (out->lit_index.begin = (const uint32_t*)b) &&
+                        cudaMemcpy(b, pf.lit_begin.data(), pf.lit_begin.size() * 4, cudaMemcpyHostToDevice) == cudaSuccess &&
+                        cudaMalloc(&e, std::max<size_t>(pf.lit_entries.size(), 1) * 8) == cudaSuccess &&
+                        (out->lit_index.entries = (const unsigned long long*)e) &&
+                        cudaMemcpy(e, pf.lit_entries.data(), pf.lit_entries.size() * 8, cudaMemcpyHostToDevice) == cudaSuccess;
+        if (!ok) { error = "cudaMalloc/cudaMemcpy failed for the literal index"; return nullptr; }
+    }
     out->bloom_false_rate = (double)pf.num_grams * (16.0 / pf.stride) / (double)((size_t)1 << pf.log2_bits);
     out->expected_hits_per_mib = pf.expected_hits_per_mib;
     out->table_words = (int)src->size();
@@ -489,6 +524,7 @@ void engine_release_slot(ScanSlot* slot) {
 void slot_set_want_records(ScanSlot* slot, bool want) { slot->want_records = want; }
 void slot_set_invert(ScanSlot* slot, bool invert) { slot->invert = invert; }
 void slot_set_spans(ScanSlot* slot, const PikeProgram* program) { slot->pike = program; }
+void slot_set_literals(ScanSlot* slot, bool literal) { slot->literal = literal; }
 void slot_set_context(ScanSlot* slot, uint32_t before, uint32_t after) {
     slot->ctx_before = before;
     slot->ctx_after = after;
@@ -560,6 +596,7 @@ static cudaError_t launch_stream_m(cudaStream_t st, int grid, int block, size_t 
 int slot_submit(ScanSlot* s, const DeviceDb& ddb, const DevicePrefilter* pf, const uint8_t* host_data, const uint8_t* dev_data, size_t n,
                 int buffer_size, void* user_stream, std::string& error) {
     if (n >= ((size_t)1 << 32) - 1024) { error = "segment too large"; return 7; }
+    if (s->literal != ddb.literal) { error = "fixed-string scan of a database that is not a fixed-string set, or the reverse"; return 7; }
     s->stream = user_stream ? (cudaStream_t)user_stream : s->own_stream;
     cudaStream_t st = s->stream;
     s->ddb = &ddb;
@@ -575,8 +612,10 @@ int slot_submit(ScanSlot* s, const DeviceDb& ddb, const DevicePrefilter* pf, con
         while (super_bytes * 4 <= (size_t)buffer_size && super_bytes < 65536) super_bytes *= 2;   // 2*super-1 <= buffer_size-1
     }
     // (NFA-fallback patterns ride the fast path when the exact gram table is there: it tells which candidates they own)
+    // (fixed strings need the literal index, and the confirm table it hangs off; mode 2 is the bloom table k_confirm reads)
     s->fast = s->pike == nullptr && ddb.simple && pf != nullptr && super_bytes >= 2048 && std::getenv("GPUGREP_FORCE_GENERAL") == nullptr &&
-              (ddb.nnfa == 0 || (pf->mode == 2 && pf->d_confirm != nullptr && std::getenv("GPUGREP_NFA_GENERAL") == nullptr));
+              (ddb.nnfa == 0 || (pf->mode == 2 && pf->d_confirm != nullptr && std::getenv("GPUGREP_NFA_GENERAL") == nullptr)) &&
+              (!ddb.literal || (pf->mode == 2 && pf->lit_index.begin != nullptr));
 
     if (host_data) {
         if (s->d_input.reserve(n + 1024) != cudaSuccess) { error = "cudaMalloc failed for the input segment"; return 3; }
@@ -609,7 +648,7 @@ int slot_submit(ScanSlot* s, const DeviceDb& ddb, const DevicePrefilter* pf, con
         }
         // (confirmation scratch too, although only multi-group / large sets use it: an allocation in the middle of the launch
         //  sequence would stall the stream)
-        if ((ddb.ngroups >= 2 || ddb.nnfa > 0 || pf->bloom_false_rate > 0.005) &&
+        if ((ddb.ngroups >= 2 || ddb.nnfa > 0 || pf->bloom_false_rate > 0.005 || ddb.literal) &&
             (s->d_hitinfo.reserve(s->cand_cap * 8) != cudaSuccess || s->d_survivors.reserve(s->cand_cap * 4) != cudaSuccess)) {
             error = "cudaMalloc failed for candidate scratch"; return 3;
         }
@@ -628,7 +667,8 @@ int slot_submit(ScanSlot* s, const DeviceDb& ddb, const DevicePrefilter* pf, con
         // noticeable share of chunks (large gram sets: those candidates are dropped without a walk) and when several DFA
         // groups would each walk the whole chunk (measured with 32 patterns / 1 group / 415 grams: no gain, so not there).
         const bool want_reprobe = ddb.ngroups >= 2 || pf->bloom_false_rate > 0.005 || ddb.nnfa > 0;
-        if (pf->mode >= 2 && pf->d_confirm && want_reprobe && (ddb.nnfa > 0 || std::getenv("GPUGREP_NO_REPROBE") == nullptr)) {
+        // (fixed strings: always, the literal index is found through the confirm slot of each hit)
+        if (pf->mode >= 2 && pf->d_confirm && ((want_reprobe && (ddb.nnfa > 0 || std::getenv("GPUGREP_NO_REPROBE") == nullptr)) || ddb.literal)) {
             rp.keys = pf->d_confirm;
             rp.groups = pf->d_confirm_groups;
             rp.mul = pf->confirm_mul; rp.mul2 = pf->confirm_mul2; rp.shift = 32 - pf->confirm_log2; rp.half = 1u << pf->confirm_log2;
@@ -714,7 +754,12 @@ int slot_submit(ScanSlot* s, const DeviceDb& ddb, const DevicePrefilter* pf, con
         }
         const char* vsel = std::getenv("GPUGREP_VERIFY");
         const bool v1 = vsel && std::strcmp(vsel, "v1") == 0;
-        if (!v1 && ddb.smem_table_bytes && hitinfo == nullptr && pf->lookback <= 64u) {
+        if (ddb.literal) {
+            const unsigned per_sm = blocks_per_sm(k_verify_literals, 128);
+            const unsigned vgrid = (unsigned)std::min<size_t>((s->cand_cap + 127) / 128, (size_t)per_sm * sms);
+            k_verify_literals<<<vgrid, 128, 0, st>>>(ddb.lits, pf->lit_index, rp, s->data, n, s->d_cand.as<uint32_t>(), hitinfo, survivors, dT,
+                                                     s->d_res.as<uint32_t>(), tile_records);
+        } else if (!v1 && ddb.smem_table_bytes && hitinfo == nullptr && pf->lookback <= 64u) {
             const size_t vsmem = 256 + ddb.smem_table_bytes;
             static SmemLimit verify_limit;
             CUDA_TRY(raise_smem_limit(verify_limit, k_verify_smem, vsmem));
@@ -736,13 +781,14 @@ int slot_submit(ScanSlot* s, const DeviceDb& ddb, const DevicePrefilter* pf, con
         // k_count_keys counts the distinct lines.  Either way a segment with more records than fit falls back to the general
         // path (flags bit 2), so that the count never depends on the capacity.
         const bool count_only = !s->want_records;
-        auto emit_kernel = ddb.nnfa > 0 ? (count_only ? k_emit_nlm<true, true> : k_emit_nlm<true, false>)
-                                        : (count_only ? k_emit_nlm<false, true> : k_emit_nlm<false, false>);
+        auto emit_kernel = ddb.literal ? (count_only ? k_emit_nlm<false, true, true> : k_emit_nlm<false, false, true>)
+                           : ddb.nnfa > 0 ? (count_only ? k_emit_nlm<true, true> : k_emit_nlm<true, false>)
+                                          : (count_only ? k_emit_nlm<false, true> : k_emit_nlm<false, false>);
         const size_t out_cap = count_only ? s->rec_cap * sizeof(LineRec) / sizeof(uint32_t) : s->rec_cap;
         const unsigned emit_per_sm = blocks_per_sm(emit_kernel, kEmitThreads);
         emit_kernel<<<(unsigned)std::min<size_t>((s->cand_cap + kEmitTile - 1) / kEmitTile, (size_t)emit_per_sm * sms), kEmitThreads, 0, st>>>(
             view, s->data, n, s->d_cand.as<uint32_t>(), s->d_res.as<uint32_t>(), tile_records, meta, prefix, nlmask, &dT->meta_total,
-            s->cand_cap, s->d_recs.as<LineRec>(), s->d_recs.as<uint32_t>(), out_cap, dT);
+            s->cand_cap, s->d_recs.as<LineRec>(), s->d_recs.as<uint32_t>(), out_cap, dT, ddb.lits);
         if (count_only)
             k_count_keys<<<(unsigned)std::min<size_t>((out_cap + 255) / 256, (size_t)sms * 4), 256, 0, st>>>(s->d_recs.as<uint32_t>(), out_cap, dT);
         else
@@ -809,7 +855,10 @@ int ScanSlot::run_general(SegmentResult& out, std::string& error, size_t split_a
     unsigned mgrid = (unsigned)((npl_total + 127) / 128);
     if (ddb->simple) {
         if (d_flags.reserve(npl_total) != cudaSuccess) { error = "cudaMalloc failed"; return 3; }
-        k_match_pl_simple<<<mgrid, 128, 0, st>>>(view, data, d_plstart.as<uint32_t>(), d_pllen.as<uint32_t>(), npl_total, d_flags.as<uint8_t>(), invert);
+        if (ddb->literal)
+            k_match_pl_literals<<<mgrid, 128, 0, st>>>(ddb->lits, data, d_plstart.as<uint32_t>(), d_pllen.as<uint32_t>(), npl_total, d_flags.as<uint8_t>(), invert);
+        else
+            k_match_pl_simple<<<mgrid, 128, 0, st>>>(view, data, d_plstart.as<uint32_t>(), d_pllen.as<uint32_t>(), npl_total, d_flags.as<uint8_t>(), invert);
         stats.launches++;
         launch_scan(st, LoadU8{d_flags.as<uint8_t>()}, npl_total, d_recoff.as<unsigned long long>(), d_sums.as<unsigned long long>(), &dT->rec_total, stats);
         // context lines: the output flags from the window test over the prefix of the selected flags, and their prefix

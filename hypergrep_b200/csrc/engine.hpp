@@ -111,6 +111,10 @@ __attribute__((weak)) void slot_set_context(ScanSlot* slot, uint32_t before, uin
 // `program` stays valid until slot_collect returns.  Call before slot_submit.  Weak like slot_set_invert (a build without it
 // fails span scans with 7).
 __attribute__((weak)) void slot_set_spans(ScanSlot* slot, const PikeProgram* program);
+// Fixed-string scan (grep -F, gpugrep_literal_scan_*): the database is a fixed-string set (Database::literal) and the segment
+// is matched against its literals instead of automata, on both paths.  Call before slot_submit, which fails with 7 when the
+// database is not of the kind the slot is set to.  Weak like slot_set_invert (a build without it fails such scans with 7).
+__attribute__((weak)) void slot_set_literals(ScanSlot* slot, bool literal);
 // Wait for the segment and expose its results (valid until the next slot_submit on this slot).
 // Returns kSplitSegment (and no results) when the fast path hit one of its capacity bounds - a line too long for it, a
 // candidate or record overflow - in a segment of more than `split_above` bytes: the caller then scans the same bytes again

@@ -202,9 +202,6 @@ __device__ uint32_t walk_local(const GroupDev& G, const uint8_t* __restrict__ da
     return mask;
 }
 
-constexpr int kEmitThreads = 256;
-constexpr int kEmitTile = 512;    // candidates per emit step (and per record-offset entry): small enough that sparse candidate lists still spread over all SMs
-
 // Confirmation of candidate chunks (databases with several DFA groups, large gram sets, NFA-fallback patterns): which
 // sampled grams of the chunk are REALLY in the set, and which DFA groups do they lead to?  k_stream only said "some gram
 // of this chunk may be".  One thread per candidate:
@@ -605,11 +602,12 @@ constexpr uint32_t kNulBound = 512;
 // COUNT_ONLY: instead of a LineRec, one 32-bit key per record goes to keys[at] (kInvalidLen: failed NUL re-check), from
 // which k_count_keys counts the distinct valid lines; no line numbers.  In a NUL-free segment the key is nlm_line_key
 // (no line extents at all), else the line start (the extents are needed for the re-check anyway).
-template <bool WITH_NFA, bool COUNT_ONLY>
+template <bool WITH_NFA, bool COUNT_ONLY, bool LITERAL>
 __device__ uint32_t emit_lane_nlm(const DbView& db, const uint8_t* __restrict__ data, size_t n, const uint32_t* __restrict__ cand,
                                   const uint32_t* __restrict__ marks, const unsigned long long* __restrict__ meta,
                                   const unsigned long long* __restrict__ prefix, const uint32_t* __restrict__ nlmask, uint32_t nblk, bool live, size_t i,
-                                  size_t at, LineRec* __restrict__ recs, uint32_t* __restrict__ keys, size_t rec_cap, bool nul_free, Totals* totals) {
+                                  size_t at, LineRec* __restrict__ recs, uint32_t* __restrict__ keys, size_t rec_cap, bool nul_free, Totals* totals,
+                                  const LiteralView& lits) {
     const uint32_t lane = threadIdx.x & 31;
     uint32_t valid = 0;
     uint32_t mask = live ? marks[i] : 0u;
@@ -667,7 +665,8 @@ __device__ uint32_t emit_lane_nlm(const DbView& db, const uint8_t* __restrict__ 
             if ((int)lane == src) has_nul = more;
         }
         if (work) {
-            if (ok && has_nul) ok = block_matches<false>(db, data, st, en) || (WITH_NFA && block_matches_nfa(db, data, st, en));
+            if (ok && has_nul)
+                ok = LITERAL ? block_matches_literal(lits, data, st, en) : block_matches<false>(db, data, st, en) || (WITH_NFA && block_matches_nfa(db, data, st, en));
             valid += ok ? 1u : 0u;
             if (COUNT_ONLY) {
                 if (at < rec_cap) keys[at] = ok ? st : kInvalidLen;
@@ -692,12 +691,14 @@ __device__ uint32_t emit_lane_nlm(const DbView& db, const uint8_t* __restrict__ 
 
 // COUNT_ONLY (the caller wants no records: grep -c, count-only scans): keys for k_count_keys instead of records (see
 // emit_lane_nlm); `recs` is unused and `rec_cap` is the capacity of `keys`.
-template <bool WITH_NFA, bool COUNT_ONLY>   // WITH_NFA: the database holds NFA-fallback patterns: lines with NUL bytes are re-checked with them too (1 KiB of local memory)
+// LITERAL: a fixed-string set (k_literal.cuh): lines with NUL bytes are re-checked against `lits`, which only it reads.
+template <bool WITH_NFA, bool COUNT_ONLY, bool LITERAL = false>   // WITH_NFA: the database holds NFA-fallback patterns: lines with NUL bytes are re-checked with them too (1 KiB of local memory)
 __global__ void __launch_bounds__(kEmitThreads, 6) k_emit_nlm(DbView db, const uint8_t* __restrict__ data, size_t n, const uint32_t* __restrict__ cand,
                                                            const uint32_t* __restrict__ marks, const uint32_t* __restrict__ tile_offsets,
                                                            const unsigned long long* __restrict__ meta, const unsigned long long* __restrict__ prefix,
                                                            const uint32_t* __restrict__ nlmask, const unsigned long long* meta_total, size_t cap,
-                                                           LineRec* __restrict__ recs, uint32_t* __restrict__ keys, size_t rec_cap, Totals* totals) {
+                                                           LineRec* __restrict__ recs, uint32_t* __restrict__ keys, size_t rec_cap, Totals* totals,
+                                                           LiteralView lits = {}) {
     __shared__ uint32_t q_cand[kEmitQueue], q_at[kEmitQueue];
     __shared__ unsigned long long s_warp[kEmitThreads / 32], s_total;
     const uint32_t nblk = (uint32_t)((n + 511) >> 9);
@@ -740,8 +741,8 @@ __global__ void __launch_bounds__(kEmitThreads, 6) k_emit_nlm(DbView db, const u
         __syncthreads();
         while (queued >= (uint32_t)kEmitThreads) {
             const uint32_t k = (head + threadIdx.x) & (kEmitQueue - 1);
-            valid += emit_lane_nlm<WITH_NFA, COUNT_ONLY>(db, data, n, cand, marks, meta, prefix, nlmask, nblk, true, q_cand[k], q_at[k], recs, keys, rec_cap,
-                                                                 nul_free, totals);
+            valid += emit_lane_nlm<WITH_NFA, COUNT_ONLY, LITERAL>(db, data, n, cand, marks, meta, prefix, nlmask, nblk, true, q_cand[k], q_at[k], recs, keys,
+                                                                  rec_cap, nul_free, totals, lits);
             head += kEmitThreads;
             queued -= kEmitThreads;
         }
@@ -754,8 +755,8 @@ __global__ void __launch_bounds__(kEmitThreads, 6) k_emit_nlm(DbView db, const u
         const uint32_t j = (threadIdx.x >> 5) + kWarps * (threadIdx.x & 31);
         const uint32_t k = (head + j) & (kEmitQueue - 1);
         const bool live = j < queued;
-        valid += emit_lane_nlm<WITH_NFA, COUNT_ONLY>(db, data, n, cand, marks, meta, prefix, nlmask, nblk, live, live ? q_cand[k] : 0, live ? q_at[k] : 0,
-                                                             recs, keys, rec_cap, nul_free, totals);
+        valid += emit_lane_nlm<WITH_NFA, COUNT_ONLY, LITERAL>(db, data, n, cand, marks, meta, prefix, nlmask, nblk, live, live ? q_cand[k] : 0,
+                                                              live ? q_at[k] : 0, recs, keys, rec_cap, nul_free, totals, lits);
     }
     (void)valid;   // the unique valid records are counted by k_dedupe_records / k_count_keys
 }

@@ -209,9 +209,8 @@ double grams_in_window(const ClassString& s, size_t t, int stride, bool fold) {
         double p = 1;
         for (int i = 0; i < 4; i++) {
             const ByteSet& b = s[t + j + i];
-            int c = 0;
-            if (fold) { ByteSet f; for (unsigned v = 0; v < 256; v++) if (b.test(v)) f.set(v | 0x20); c = f.count(); }
-            else c = b.count();
+            int c = b.count();
+            if (fold && c > 1) { ByteSet f; for (unsigned v = 0; v < 256; v++) if (b.test(v)) f.set(v | 0x20); c = f.count(); }
             p *= c;
         }
         total += p;
@@ -315,7 +314,24 @@ ByteSet effective(const ByteSet& b, bool fold) {
     return f;
 }
 
+// The one gram of s[at, at+4) when every position holds one byte (literals, most regex factors); false otherwise.
+bool single_gram(const ClassString& s, size_t at, bool fold, uint32_t& gram) {
+    gram = 0;
+    for (int i = 0; i < 4; i++) {
+        const ByteSet& b = s[at + i];
+        if (b.count() != 1) return false;
+        unsigned v = 0;
+        while (!b.w[v >> 6]) v += 64;
+        v += (unsigned)__builtin_ctzll(b.w[v >> 6]);
+        if (fold) v |= 0x20;
+        gram |= v << (8 * i);
+    }
+    return true;
+}
+
 void expand_gram(const ClassString& s, size_t at, bool fold, std::vector<uint32_t>& out) {
+    uint32_t one = 0;
+    if (single_gram(s, at, fold, one)) { out.push_back(one); return; }
     std::vector<uint32_t> cur = {0};
     for (int i = 0; i < 4; i++) {
         ByteSet eff = effective(s[at + i], fold);
@@ -333,6 +349,8 @@ double window_hits(const ClassString& s, size_t t, int stride, bool fold, const 
     std::vector<uint32_t> grams;
     double hits = 0;
     for (int j = 0; j < stride; j++) {
+        uint32_t one = 0;
+        if (single_gram(s, t + j, fold, one)) { hits += h.count(one, fold); continue; }
         grams.clear();
         expand_gram(s, t + j, fold, grams);
         for (uint32_t g : grams) hits += h.count(g, fold);
@@ -691,6 +709,44 @@ bool build_mixed(const FactorSet& fs, const GramHistogram* sample, bool fold, Pr
     return true;
 }
 
+// Literal index of a fixed-string set (Prefilter::lit_begin): every gram of each literal's window, under the confirm slot
+// of the gram.  Without an exact confirm table there is no index, and the set goes without a prefilter.
+void build_literal_index(const FactorSet& fs, const std::vector<Window>& wins, int stride, bool fold, Prefilter& out) {
+    if (out.confirm_keys.empty()) {
+        out = Prefilter();
+        out.note = "no exact gram table for the literal index";
+        return;
+    }
+    const size_t half = (size_t)1 << out.confirm_log2;
+    struct E { uint32_t slot, key, rank, lit; };
+    std::vector<E> es;
+    es.reserve(wins.size() * (size_t)stride);
+    std::vector<uint32_t> grams;
+    for (const Window& wn : wins) {
+        const uint32_t cls = fs.literal_class[wn.pattern];
+        for (int j = 0; j < stride; j++) {
+            grams.clear();
+            expand_gram(*wn.s, wn.start + j, fold, grams);
+            for (uint32_t g : grams) {
+                const size_t h1 = prefilter_hash(g, out.confirm_mul, out.confirm_log2), h2 = half + prefilter_hash(g, out.confirm_mul2, out.confirm_log2);
+                const uint32_t slot = (uint32_t)(out.confirm_keys[h1] == g ? h1 : h2);
+                es.push_back(E{slot, cls << 31 | (uint32_t)(wn.start + (size_t)j), fs.literal_rank[wn.pattern], (uint32_t)wn.pattern});
+            }
+        }
+    }
+    std::sort(es.begin(), es.end(), [](const E& a, const E& b) {
+        return a.slot != b.slot ? a.slot < b.slot : (a.key != b.key ? a.key < b.key : a.rank < b.rank);
+    });
+    es.erase(std::unique(es.begin(), es.end(), [](const E& a, const E& b) { return a.slot == b.slot && a.key == b.key && a.lit == b.lit; }), es.end());
+    out.lit_begin.assign(out.confirm_keys.size() + 1, 0);
+    out.lit_entries.resize(es.size());
+    for (size_t k = 0; k < es.size(); k++) {
+        out.lit_begin[es[k].slot + 1]++;
+        out.lit_entries[k] = (uint64_t)es[k].key << 32 | es[k].lit;
+    }
+    for (size_t h = 0; h < out.confirm_keys.size(); h++) out.lit_begin[h + 1] += out.lit_begin[h];
+}
+
 }  // namespace
 
 static void build_uniform(const FactorSet& fs, const GramHistogram* sample, Prefilter& out) {
@@ -726,7 +782,8 @@ static void build_uniform(const FactorSet& fs, const GramHistogram* sample, Pref
                 }
                 if (!ok) break;
             }
-            if (!ok || total > (double)kMaxGramsTotal) continue;
+            // (the gram tables of a fixed-string set are global-memory tables: only the shared-memory bloom has a fixed size)
+            if (!ok || (total > (double)kMaxGramsTotal && !fs.literal())) continue;
             if (!fold) {
                 // prefer exact-case grams unless folding shrinks the table a lot (caseless sets)
                 double folded_total = 0;
@@ -741,6 +798,7 @@ static void build_uniform(const FactorSet& fs, const GramHistogram* sample, Pref
             if (sample && sample->positions()) out.expected_hits_per_mib = hits * 1048576.0 / (double)sample->positions();
             finish_tables(all, fold, sample, out);
             out.note = describe(out, sample != nullptr);
+            if (fs.literal()) build_literal_index(fs, wins, stride, fold, out);
             return;
         }
     }
@@ -753,7 +811,8 @@ void build_prefilter(const FactorSet& fs, const GramHistogram* sample, Prefilter
     // compares (half the shared-memory lookups of the streaming kernel; measured 0.54 -> 0.45 ms per 2 GiB), unless that
     // flags more text or makes the verification walks longer.  (Four compares were measured too: the streaming kernel
     // gains 8 %, verification loses more through the longer look-back of the 7-byte windows.)
-    if (out.enabled && out.stride == 2 && std::getenv("GPUGREP_NO_MIXED_STRIDE") == nullptr) {
+    // (not for fixed-string sets: their literal index holds the grams of whole windows, which the register compares are not)
+    if (out.enabled && out.stride == 2 && !fs.literal() && std::getenv("GPUGREP_NO_MIXED_STRIDE") == nullptr) {
         Prefilter mixed;
         if (build_mixed(fs, sample, out.fold_case, mixed) && mixed.enabled && mixed.lookback <= out.lookback + 4 &&
             (!sample || mixed.expected_hits_per_mib <= 1.1 * out.expected_hits_per_mib + 16.0))

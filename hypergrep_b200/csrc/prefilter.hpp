@@ -26,6 +26,12 @@ struct FactorSet {
     std::vector<uint32_t> group_mask;                  // per pattern: bit (g mod 32) of the DFA group(s) the pattern is compiled into (empty: unknown)
     size_t min_len = 0;
     std::string note;
+    // Fixed-string sets only (empty for regex sets): per pattern, i.e. per literal, its rank in the byte order of its class
+    // and that class (1: caseless).  Their gram tables are not capped by size (they live in global memory) and carry a
+    // literal index (Prefilter::lit_begin).
+    std::vector<uint32_t> literal_rank;
+    std::vector<uint8_t> literal_class;
+    bool literal() const { return !literal_rank.empty(); }
 };
 
 // 4-gram histogram of a text sample (raw and case-folded), used to pick selective windows.
@@ -95,6 +101,12 @@ struct Prefilter {
     uint32_t lookback = 0xffffffffu;
     double expected_hits_per_mib = -1;   // from the sample histogram, -1 without a sample
     std::string note;           // why it is disabled, or a one-line summary
+    // Literal index (fixed-string sets): the grams of the window chosen in each literal, each with the literal and the
+    // offset of the gram in it.  Entries of confirm slot h are lit_entries[lit_begin[h] .. lit_begin[h + 1]), each
+    // (class << 31 | offset) << 32 | literal, sorted by that key and then by the literal's rank: one (class, offset) run
+    // is in byte order and is searched, not walked.
+    std::vector<uint32_t> lit_begin;
+    std::vector<uint64_t> lit_entries;
 };
 
 // Required-factor analysis of one pattern.  Returns false if no usable factor exists.

@@ -66,10 +66,14 @@ def get_argparse_patterns(args: argparse.Namespace) -> list[str]:
     for name in args.pattern_files or []:
         with open(name, "rt", encoding="utf-8") as handle:
             patterns += [line.rstrip("\n") for line in handle.readlines()]
-    for pattern in patterns:
-        _validate_python_regex(pattern)
+    fixed = getattr(args, "regexp", None) == "fixed"
+    if not fixed:   # (-F: literals, whatever Python's re thinks of them)
+        for pattern in patterns:
+            _validate_python_regex(pattern)
     # The compile check runs in the parent, before any pool exists, and never touches CUDA (fork-safe).
-    if hypergrep.check_compatibility(patterns):
+    if fixed and hypergrep.check_compatibility(patterns, fixed_strings=True):
+        raise ValueError("hyperscanner: invalid fixed string")
+    if not fixed and hypergrep.check_compatibility(patterns):
         raise ValueError(f"hyperscanner: incompatible regex: for more information visit {_UNSUPPORTED_URL}")
     return patterns
 
@@ -156,6 +160,7 @@ def parallel_grep(  # pylint: disable=too-many-arguments,too-many-locals
     before_context: int | None = None,
     after_context: int | None = None,
     group_separator: str | None = "--",
+    fixed_strings: bool = False,
 ) -> int:
     """Scan files and print grep-formatted results (reference multiscanner.py:86-223).
 
@@ -166,6 +171,7 @@ def parallel_grep(  # pylint: disable=too-many-arguments,too-many-locals
     width of 0 still separates the groups, and None (the default) prints no context output at all.  -c, -t, -l, -L and
     -q ignore them; with -o only the matched parts are printed, and a separator goes between two selected lines whose gap
     exceeds ``before_context + after_context`` lines.
+    ``fixed_strings`` (``-F``): the patterns are literals.
     """
     if invert_match and only_matching:
         # GNU grep -v -o: a selected line has no matching part, so nothing is printed; the exit code still says whether
@@ -206,6 +212,7 @@ def parallel_grep(  # pylint: disable=too-many-arguments,too-many-locals
         # (-o prints matched parts only: the grouping of the selected lines is all the printer needs)
         "before_context": 0 if only_matching else before_context,
         "after_context": 0 if only_matching else after_context,
+        "fixed_strings": fixed_strings,
     }
     workers = min(max(multiprocessing.cpu_count() - 1, 1), len(files))
     pool_type = ThreadPool if use_multithreading else multiprocessing.Pool
@@ -325,6 +332,8 @@ def parse_args(args: list | None = None) -> argparse.Namespace:
     syntax.set_defaults(regexp="bre")
     for short, long_name, value, text in (
         ("-E", "--extended-regexp", "ere", "Interpret PATTERNS as extended regular expressions (EREs)."),
+        ("-F", "--fixed-strings", "fixed", "Interpret PATTERNS as fixed strings, not regular expressions. Unlike GNU grep,\n"
+                                           "an empty pattern is an error here (GNU grep matches every line)."),
         ("-G", "--basic-regexp", "bre", "Interpret PATTERNS as basic regular expressions. This is the default."),
         ("-P", "--perl-regexp", "pcre", "Interpret PATTERNS as Perl-compatible regular expressions (PCREs)."),
     ):
@@ -412,7 +421,7 @@ def main() -> None:
     except ValueError as error:
         print(error)
         raise SystemExit(2) from error
-    if args.gnu_regexp and args.regexp != "pcre":
+    if args.gnu_regexp and args.regexp not in ("pcre", "fixed"):
         patterns = to_gnu_regular_expressions(patterns)
     after_context = args.after_context if args.after_context is not None else args.context
     before_context = args.before_context if args.before_context is not None else args.context
@@ -457,6 +466,7 @@ def main() -> None:
             before_context=before_context,
             after_context=after_context,
             group_separator=args.group_separator,
+            fixed_strings=args.regexp == "fixed",
         )
     )
 

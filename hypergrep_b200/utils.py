@@ -131,10 +131,13 @@ def prepare_patterns(
     return pattern_array, flags_array, ids_array
 
 
-def check_compatibility(patterns: list, flags: Sequence[int] = ()) -> int:
-    """Compile-check patterns without scanning (reference utils.py:97-122): 0, or 4 when any pattern is rejected."""
+def check_compatibility(patterns: list, flags: Sequence[int] = (), fixed_strings: bool = False) -> int:
+    """Compile-check patterns without scanning (reference utils.py:97-122): 0, or 4 when any pattern is rejected.
+    ``fixed_strings``: the patterns are literals (``grep -F``), checked by gpugrep_check_literals."""
     pattern_array, flags_array, ids_array = prepare_patterns(patterns, flags=flags)
     lib = _get_hyperscanner_lib()
+    if fixed_strings:
+        return _literal_check_entry(lib)(pattern_array, flags_array, len(pattern_array))
     return lib.check_patterns(pattern_array, flags_array, ids_array, len(pattern_array))
 
 
@@ -153,6 +156,7 @@ def scan(  # pylint: disable=too-many-arguments
     invert_match: bool = False,
     before_context: int = 0,
     after_context: int = 0,
+    fixed_strings: bool = False,
 ) -> int:
     """Scan one plain/gzip/zstd file on the GPU, delivering matched lines in batches (reference utils.py:292-358).
 
@@ -163,16 +167,27 @@ def scan(  # pylint: disable=too-many-arguments
     ``before_context`` / ``after_context`` (``grep -B`` / ``-A``) also deliver the lines that lie up to that many lines
     before / after a selected line, with id ``CONTEXT_ID``; selected lines then carry id 0.  ``max_match_count`` counts
     selected lines, and the ``after_context`` lines behind the one that reaches it are still delivered, as context.
+    ``fixed_strings`` (``grep -F``): the patterns are literals, not regular expressions (gpugrep_literal_scan_file); only
+    ``HS_FLAG_CASELESS`` of the flags changes anything, and every record has id 0, so ``ids`` raise ValueError.
     """
     _check_context(before_context, after_context)
+    if fixed_strings and ids:
+        raise ValueError("fixed_strings scans take no ids: every selected line is reported with id 0")
     pattern_array, flags_array, ids_array = prepare_patterns(patterns, flags=flags, ids=ids)
     c_callback = CALLBACK_TYPE(callback)
     lib = _get_hyperscanner_lib()
     context = before_context > 0 or after_context > 0
-    entry = _context_entry(lib) if context else (_invert_entry(lib) if invert_match else None)
+    if fixed_strings:
+        entry = _literal_entry(lib)
+    else:
+        entry = _context_entry(lib) if context else (_invert_entry(lib) if invert_match else None)
     outcome = {"rc": 0}
 
     def _run() -> None:
+        if fixed_strings:
+            outcome["rc"] = entry(path.encode(), pattern_array, flags_array, len(pattern_array), c_callback, buffer_size, buffer_count,
+                                  max_match_count, before_context, after_context, int(invert_match), None)
+            return
         if context:
             outcome["rc"] = entry(path.encode(), pattern_array, flags_array, ids_array, len(pattern_array), c_callback, buffer_size,
                                   buffer_count, max_match_count, before_context, after_context, int(invert_match), None)
@@ -256,14 +271,46 @@ def _context_entry(lib: ctypes.CDLL):
     return entry
 
 
+def _literal_entry(lib: ctypes.CDLL):
+    """gpugrep_literal_scan_file of the loaded library.  Fixed strings have no CPU fallback: a library without the entry
+    point (a plain libhyperscanner.so through GPUGREP_LIBRARY) is an error."""
+    try:
+        entry = lib.gpugrep_literal_scan_file
+    except AttributeError as error:
+        raise NotImplementedError(
+            "fixed_strings needs gpugrep_literal_scan_file, which the loaded native library does not export "
+            f"({_library_path()}); there is no CPU fallback"
+        ) from error
+    entry.restype = ctypes.c_int
+    entry.argtypes = [ctypes.c_char_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint, ctypes.c_void_p, ctypes.c_int, ctypes.c_int,
+                      ctypes.c_ulonglong, ctypes.c_uint, ctypes.c_uint, ctypes.c_int, ctypes.c_void_p]
+    return entry
+
+
+def _literal_check_entry(lib: ctypes.CDLL):
+    """gpugrep_check_literals of the loaded library (see _literal_entry)."""
+    try:
+        entry = lib.gpugrep_check_literals
+    except AttributeError as error:
+        raise NotImplementedError(
+            f"fixed_strings needs gpugrep_check_literals, which the loaded native library does not export ({_library_path()})"
+        ) from error
+    entry.restype = ctypes.c_int
+    entry.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint]
+    return entry
+
+
 def _count_matches(path: str, patterns: Sequence[str], flags: Sequence[int], max_match_count: int,
-                   invert_match: bool = False) -> tuple[int, int] | None:
+                   invert_match: bool = False, fixed_strings: bool = False) -> tuple[int, int] | None:
     """Count-only scan without a callback: the library counts on the device and copies no line back
     (gpugrep_scan_file with on_event = NULL).  Returns None if the loaded library has no such entry point (a plain
     libhyperscanner.so), in which case the caller counts through the callback like the reference does.
-    ``invert_match`` counts the lines without a match (gpugrep_invert_scan_file); it has no such fallback."""
+    ``invert_match`` counts the lines without a match (gpugrep_invert_scan_file); it has no such fallback, nor has
+    ``fixed_strings`` (gpugrep_literal_scan_file)."""
     lib = _get_hyperscanner_lib()
-    if invert_match:
+    if fixed_strings:
+        entry = _literal_entry(lib)
+    elif invert_match:
         entry = _invert_entry(lib)
     else:
         try:
@@ -277,6 +324,10 @@ def _count_matches(path: str, patterns: Sequence[str], flags: Sequence[int], max
     outcome = {"rc": 0}
 
     def _run() -> None:
+        if fixed_strings:
+            outcome["rc"] = entry(path.encode(), pattern_array, flags_array, len(pattern_array), None, 262140, 16, max_match_count, 0, 0,
+                                  int(invert_match), ctypes.byref(stats))
+            return
         outcome["rc"] = entry(path.encode(), pattern_array, flags_array, ids_array, len(pattern_array), None, 262140, 16,
                               max_match_count, ctypes.byref(stats))
 
@@ -301,6 +352,7 @@ def grep(  # pylint: disable=too-many-arguments
     invert_match: bool = False,
     before_context: int = 0,
     after_context: int = 0,
+    fixed_strings: bool = False,
 ) -> tuple[int | list[tuple[int, str]] | list[tuple[int, str, bool]], int]:
     """grep-like collector on top of :func:`scan` (reference utils.py:147-231).
 
@@ -312,10 +364,15 @@ def grep(  # pylint: disable=too-many-arguments
     ``before_context`` / ``after_context`` (``grep -B`` / ``-A``) add the lines up to that many lines before / after each
     selected line; results are then ``(line number, line text, is_context)``.  ``count_only`` and ``only_matching`` ignore
     context.  Negative counts raise ValueError.
+    ``fixed_strings`` (``grep -F``): the patterns are literals (:func:`scan`).  With ``only_matching`` the result is that of
+    the ``re.escape``-d patterns as regular expressions.
     """
     _check_context(before_context, after_context)
+    if fixed_strings and only_matching:
+        patterns = [re.escape(pattern) for pattern in patterns]
+        fixed_strings = False
     context = (before_context > 0 or after_context > 0) and not (count_only or only_matching)
-    python_patterns = [re.compile(pattern) for pattern in patterns]
+    python_patterns = [] if fixed_strings else [re.compile(pattern) for pattern in patterns]
     collected: list[tuple[int, str]] = []
     counter = [0]
 
@@ -370,7 +427,7 @@ def grep(  # pylint: disable=too-many-arguments
     pattern_flags = _DEFAULT_FLAGS | (HS_FLAG_CASELESS if ignore_case else 0)
     if count_only:
         # SURVEY.md section 8(f)-2: counting needs no line copies and no Python frame per batch of 16 results
-        counted = _count_matches(file, patterns, [pattern_flags] * len(patterns), max_match_count, invert_match)
+        counted = _count_matches(file, patterns, [pattern_flags] * len(patterns), max_match_count, invert_match, fixed_strings)
         if counted is not None:
             return counted
     code = scan(
@@ -383,6 +440,7 @@ def grep(  # pylint: disable=too-many-arguments
         invert_match=invert_match,
         before_context=before_context if context else 0,
         after_context=after_context if context else 0,
+        fixed_strings=fixed_strings,
     )
     if only_matching:
         _fill_spans(groups, deferred, patterns, widths, python_patterns, errors, span_lines)

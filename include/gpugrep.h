@@ -149,6 +149,28 @@ GPUGREP_API int gpugrep_context_scan_buffer(const void* data, size_t size, int l
                                 hs_event on_event, int buffer_size, int buffer_count, unsigned long long max_match_count,
                                 unsigned int before, unsigned int after, int invert, void* stream, gpugrep_stats* stats);
 
+/* ---- fixed strings (`grep -F`) ------------------------------------------------------------------------------------
+ * `elements` >= 1 NUL-terminated, non-empty literals (byte strings, not patterns) with per-literal flags (NULL: all 0):
+ * HS_FLAG_CASELESS (1) is honoured, 2, 4 and 8 are accepted and change nothing, any other bit, an empty literal or
+ * elements == 0 return 4.  A pseudo-line is split as hyperscan() splits it and is SELECTED when its scanned block (leading
+ * NULs skipped, cut at the next NUL, the trailing '\n' included) contains some literal as a contiguous substring.  Caseless
+ * literals compare with ASCII folding of A-Z / a-z only: other bytes, >= 0x80 included, compare exactly ('@' is not '`').
+ * So a literal ending in '\n' matches only at a line end, and one with a '\n' before its last byte never matches.
+ * Records, batches, max_match_count, trailing context after the limit, GPUGREP_CONTEXT_ID, on_event == NULL counting and
+ * every input form are those of gpugrep_context_scan_* for the same set with every byte written as \xHH, the flags as
+ * given plus SINGLEMATCH and ids 0.  No automaton is built: the sample-tuned gram prefilter flags candidates, and a literal
+ * index over its grams leads each gram hit to the few literals it can belong to, compared byte for byte.
+ * gpugrep_check_literals checks a set on the host (0 or 4).  A build of the engine without the fixed-string stage returns 7. */
+GPUGREP_API int gpugrep_literal_scan_file(const char* file_name, const char* const* literals, const unsigned int* literal_flags,
+                              unsigned int elements, hs_event on_event, int buffer_size, int buffer_count,
+                              unsigned long long max_match_count, unsigned int before, unsigned int after, int invert,
+                              gpugrep_stats* stats);
+GPUGREP_API int gpugrep_literal_scan_buffer(const void* data, size_t size, int location, const char* const* literals,
+                                const unsigned int* literal_flags, unsigned int elements, hs_event on_event, int buffer_size,
+                                int buffer_count, unsigned long long max_match_count, unsigned int before, unsigned int after,
+                                int invert, void* stream, gpugrep_stats* stats);
+GPUGREP_API int gpugrep_check_literals(const char* const* literals, const unsigned int* literal_flags, unsigned int elements);
+
 /* ---- match END offsets (SURVEY.md section 8f-4: spans for `grep -o`) --------------------------------------------
  * The reference gets the spans of `-o` by re-running Python's re.finditer() over every matched line (utils.py:205-212);
  * Hyperscan itself reports (id, end offset) per match and the reference drops the offset (hyperscanner.c:83-102).
