@@ -17,6 +17,7 @@ from hypergrep_b200.utils import configure_libraries
 from hypergrep_b200.utils import grep
 from hypergrep_b200.utils import prepare_patterns
 from hypergrep_b200.utils import scan
+from hypergrep_b200.utils import scan_literals
 
 __version__ = "0.1.0"
 __all__ = [
@@ -33,4 +34,5 @@ __all__ = [
     "grep",
     "prepare_patterns",
     "scan",
+    "scan_literals",
 ]

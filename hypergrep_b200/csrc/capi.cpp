@@ -369,7 +369,16 @@ struct Job {
         retunes++;
     }
 
+    // events, not line records: general-mode sets and fixed-string sets compiled for reports
+    bool wants_events() const { return !db->simple || db->literal_reports; }
+
     void prepare() {
+        if (db->literal_reports) {   // device events carry the node of the report table
+            const auto& rb = db->lit_reports.report_begin;
+            report_begin_flat.assign(rb.begin(), rb.end() - 1);
+            report_end_flat.assign(rb.begin() + 1, rb.end());
+            return;
+        }
         if (db->simple) return;   // the flat report ranges are only read when events are expanded to ids
         for (auto& rb : db->report_begin) {
             // every group's list ends with a sentinel; keep [begin, next begin) pairs addressable by flat index
@@ -397,7 +406,7 @@ struct Job {
         stats.segments++;
         stats.nul_segments += r.stats.nul ? 1u : 0u;
         if (stop) return 0;
-        int rc = out->wants_spans() ? deliver_spans(r) : (db->simple ? deliver_simple(r, host, slot) : deliver_events(r, host, slot));
+        int rc = out->wants_spans() ? deliver_spans(r) : (wants_events() ? deliver_events(r, host, slot) : deliver_simple(r, host, slot));
         line_base += r.num_lines;
         return rc;
     }
@@ -534,6 +543,7 @@ struct Params {
     bool invert = false;        // gpugrep_invert_scan_*(): deliver the pseudo-lines in which no pattern reports
     bool context_scan = false;  // gpugrep_context_scan_*(): lines around the selected ones too
     bool literal = false;       // gpugrep_literal_scan_*(): `patterns` are fixed strings (flags: CASELESS only, no ids)
+    bool literal_reports = false;   // gpugrep_literal_report_scan_*(): fixed strings with ids, one record per (id, end)
     uint32_t before = 0, after = 0;
     // the context stage runs only when lines are delivered (count-only scans ignore context)
     bool context() const { return context_scan && cb != nullptr && (before || after); }
@@ -563,11 +573,13 @@ void set_spans(ScanSlot* slot, const Params& pr) {
 }
 void set_literals(ScanSlot* slot, const Params& pr) {
     if (slot_set_literals) slot_set_literals(slot, pr.literal);
+    if (slot_set_literal_reports) slot_set_literal_reports(slot, pr.literal_reports);
 }
 
 int setup_job(const Params& pr, Job& job, Deliverer& out, unsigned long long weight = 0) {
     int rc = 0;
-    if (pr.literal) job.db = cached_literal_database(pr.patterns, pr.flags, pr.elements, rc, job.error);
+    if (pr.literal_reports) job.db = cached_literal_report_database(pr.patterns, pr.flags, pr.ids, pr.elements, rc, job.error);
+    else if (pr.literal) job.db = cached_literal_database(pr.patterns, pr.flags, pr.elements, rc, job.error);
     else job.db = cached_database(pr.patterns, pr.flags, pr.ids, pr.elements, rc, job.error);
     if (job.db && !pr.literal && (pr.invert || pr.context_scan)) {
         // Which lines match does not depend on ids or SINGLEMATCH: once the set compiles as given, it is scanned as "every
@@ -585,6 +597,7 @@ int setup_job(const Params& pr, Job& job, Deliverer& out, unsigned long long wei
     if (pr.context_scan && !slot_set_context) { job.error = "this build of the engine has no context lines"; return GPUGREP_SCAN; }
     if (pr.span_program && !slot_set_spans) { job.error = "this build of the engine has no span stage"; return GPUGREP_SCAN; }
     if (pr.literal && !slot_set_literals) { job.error = "this build of the engine has no fixed-string stage"; return GPUGREP_SCAN; }
+    if (pr.literal_reports && !slot_set_literal_reports) { job.error = "this build of the engine has no fixed-string report stage"; return GPUGREP_SCAN; }
     job.device_weight = weight;
     job.device = pick_device(weight, &job.device_charged);
     if (engine_select_device(job.device, job.error) != 0) {
@@ -691,7 +704,7 @@ int scan_file(const char* path, const Params& pr, gpugrep_stats* stats_out, cons
         return GPUGREP_SCRATCH;
     }
 
-    const bool count_only = !out.wants_lines() && pr.max_match == 0 && job.db->simple;
+    const bool count_only = !out.wants_lines() && pr.max_match == 0 && !job.wants_events();
     for (ScanSlot* sl : slots) {
         slot_set_want_records(sl, !count_only);
         set_invert(sl, pr.invert);
@@ -862,7 +875,7 @@ int scan_memory(const uint8_t* data, size_t size, int location, const Params& pr
     }
     ScanSlot* slots[2] = {engine_acquire_slot(err, location != GPUGREP_LOC_DEVICE), engine_acquire_slot(err, location != GPUGREP_LOC_DEVICE)};
     if (!slots[0] || !slots[1]) { engine_release_slot(slots[0]); engine_release_slot(slots[1]); set_last_error(err); return GPUGREP_SCRATCH; }
-    const bool count_only = !out.wants_lines() && pr.max_match == 0 && job.db->simple;
+    const bool count_only = !out.wants_lines() && pr.max_match == 0 && !job.wants_events();
     for (ScanSlot* sl : slots) {
         slot_set_want_records(sl, !count_only);
         set_invert(sl, pr.invert);
@@ -1280,6 +1293,24 @@ int gpugrep_literal_scan_buffer(const void* data, size_t size, int location, con
     pr.context_scan = true;
     pr.before = before;
     pr.after = after;
+    return gpugrep::scan_buffer(data, size, location, pr, stats);
+}
+
+int gpugrep_literal_report_scan_file(const char* file_name, const char* const* literals, const unsigned int* literal_flags,
+                                     const unsigned int* literal_ids, unsigned int elements, hs_event on_event, int buffer_size, int buffer_count,
+                                     unsigned long long max_match_count, gpugrep_stats* stats) {
+    gpugrep::Params pr{literals, literal_flags, literal_ids, elements, on_event, buffer_size, buffer_count, max_match_count, nullptr};
+    pr.literal = true;
+    pr.literal_reports = true;
+    return gpugrep::scan_path(file_name, pr, stats);
+}
+
+int gpugrep_literal_report_scan_buffer(const void* data, size_t size, int location, const char* const* literals, const unsigned int* literal_flags,
+                                       const unsigned int* literal_ids, unsigned int elements, hs_event on_event, int buffer_size, int buffer_count,
+                                       unsigned long long max_match_count, void* stream, gpugrep_stats* stats) {
+    gpugrep::Params pr{literals, literal_flags, literal_ids, elements, on_event, buffer_size, buffer_count, max_match_count, stream};
+    pr.literal = true;
+    pr.literal_reports = true;
     return gpugrep::scan_buffer(data, size, location, pr, stats);
 }
 

@@ -345,4 +345,93 @@ std::shared_ptr<Database> cached_literal_database(const char* const* literals, c
                   [&](std::shared_ptr<Database>& db) { return compile_literal_database(literals, flags, n, db, error); }, rc);
 }
 
+int compile_literal_report_database(const char* const* literals, const unsigned* flags, const unsigned* ids, unsigned n,
+                                    std::shared_ptr<Database>& out, std::string& error) {
+    const int kDbError = 4;
+    int rc = check_literals(literals, flags, n, error);
+    if (rc) return rc;
+    {   // hs_compile.h: expressions sharing a match id must agree on SINGLEMATCH
+        std::map<unsigned, unsigned> sm;
+        for (unsigned i = 0; i < n; i++) {
+            const unsigned id = ids ? ids[i] : 0u, v = flags ? flags[i] & FLAG_SINGLEMATCH : 0u;
+            auto it = sm.emplace(id, v).first;
+            if (it->second != v) { error = "literals sharing id " + std::to_string(id) + " disagree on SINGLEMATCH"; return kDbError; }
+        }
+    }
+    rc = compile_literal_database(literals, flags, n, out, error);
+    if (rc) return rc;
+    Database& db = *out;
+    db.literal_reports = true;
+    LiteralReports& R = db.lit_reports;
+    struct Given { std::string text; unsigned cls, id, sm; };
+    std::vector<Given> given;
+    given.reserve(n);
+    for (unsigned i = 0; i < n; i++) {
+        const size_t len = std::strlen(literals[i]);
+        const char* nl = static_cast<const char*>(std::memchr(literals[i], '\n', len));
+        if (nl && nl != literals[i] + len - 1) continue;   // can never lie inside a line
+        Given g{std::string(literals[i], len), flags && (flags[i] & FLAG_CASELESS) ? 1u : 0u, ids ? ids[i] : 0u,
+                flags && (flags[i] & FLAG_SINGLEMATCH) ? 1u : 0u};
+        if (g.cls) for (char& c : g.text) c = (char)fold_ascii((uint8_t)c);
+        given.push_back(std::move(g));
+    }
+    std::sort(given.begin(), given.end(), [](const Given& a, const Given& b) {
+        if (a.cls != b.cls) return a.cls < b.cls;
+        if (a.text != b.text) return a.text < b.text;
+        return a.id != b.id ? a.id < b.id : a.sm < b.sm;
+    });
+    R.bucket.assign(2 * 65537, 0);
+    R.one.assign(2 * 256, kNoLiteral);
+    std::vector<uint32_t> count(2 * 65536, 0);
+    std::vector<uint32_t> chain;   // the nodes that are prefixes of the last node, shortest first
+    for (size_t i = 0; i < given.size(); i++) {
+        const Given& g = given[i];
+        const bool fresh = i == 0 || given[i - 1].cls != g.cls || given[i - 1].text != g.text;
+        if (fresh) {
+            const uint32_t node = (uint32_t)R.off.size();
+            // (in byte order every node that is a prefix of this one comes before it, and is on the chain of its predecessor)
+            while (!chain.empty()) {
+                const uint32_t top = chain.back();
+                const std::string_view t(reinterpret_cast<const char*>(R.bytes.data()) + R.off[top], R.len[top]);
+                if (R.caseless[top] == g.cls && t.size() < g.text.size() && std::string_view(g.text).substr(0, t.size()) == t) break;
+                chain.pop_back();
+            }
+            R.parent.push_back(chain.empty() ? kNoLiteral : chain.back());
+            chain.push_back(node);
+            R.off.push_back((uint32_t)R.bytes.size());
+            R.len.push_back((uint32_t)g.text.size());
+            R.caseless.push_back((uint8_t)g.cls);
+            R.bytes.insert(R.bytes.end(), g.text.begin(), g.text.end());
+            R.report_begin.push_back((uint32_t)db.reports.size());
+            const uint8_t b0 = (uint8_t)g.text[0];
+            if (g.text.size() == 1) {
+                R.one[g.cls * 256 + b0] = node;
+            } else {
+                R.order.push_back(node);
+                count[g.cls * 65536 + ((uint32_t)b0 << 8 | (uint8_t)g.text[1])]++;
+            }
+        }
+        if (fresh || given[i - 1].id != g.id || given[i - 1].sm != g.sm) db.reports.push_back(ReportDesc{g.id, g.sm});
+    }
+    R.report_begin.push_back((uint32_t)db.reports.size());
+    uint32_t at = 0;
+    for (unsigned cls = 0; cls < 2; cls++) {
+        for (uint32_t k = 0; k < 65536; k++) {
+            R.bucket[cls * 65537 + k] = at;
+            at += count[cls * 65536 + k];
+        }
+        R.bucket[cls * 65537 + 65536] = at;
+    }
+    return 0;
+}
+
+std::shared_ptr<Database> cached_literal_report_database(const char* const* literals, const unsigned* flags, const unsigned* ids,
+                                                         unsigned n, int& rc, std::string& error) {
+    // (the ids and every flag bit are part of the key; the tag keeps it apart from a selection set with ids 0)
+    std::string key = cache_key(literals, flags, ids, n);
+    key.append("\x01reports");
+    return cached(true, std::move(key),
+                  [&](std::shared_ptr<Database>& db) { return compile_literal_report_database(literals, flags, ids, n, db, error); }, rc);
+}
+
 }  // namespace gpugrep

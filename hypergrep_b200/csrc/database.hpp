@@ -51,6 +51,25 @@ struct LiteralSet {
     unsigned given = 0;                  // literals passed in
 };
 
+// Report table of a fixed-string set compiled for reports (gpugrep_literal_report_scan_*): every distinct (class, folded
+// bytes) literal that can lie inside a line is one node, numbered in (class, byte) order.  Unlike LiteralSet nothing is
+// pruned: every literal that matches at a position reports.  At a text position the matching nodes of a class are the
+// parent chain of the greatest node of the two-byte bucket that is not above the text, cut where a node is longer than
+// the common prefix of that node and the text (DESIGN.md section 9).
+constexpr uint32_t kNoLiteral = 0xffffffffu;
+struct LiteralReports {
+    std::vector<uint8_t> bytes;          // the nodes, caseless ones folded to lower case (A-Z only)
+    std::vector<uint32_t> off, len;      // per node: offset into bytes, length
+    std::vector<uint8_t> caseless;       // per node: class
+    std::vector<uint32_t> parent;        // per node: its longest proper prefix that is a node of its class, or kNoLiteral
+    std::vector<uint32_t> order;         // nodes of >= 2 bytes, in node order
+    std::vector<uint32_t> bucket;        // [class][65537]: the nodes of `order` whose first two bytes are (b0 << 8 | b1) are
+                                         // order[bucket[k] .. bucket[k + 1])
+    std::vector<uint32_t> one;           // [class][256]: the node of the one-byte literal b, or kNoLiteral
+    std::vector<uint32_t> report_begin;  // per node, + 1: its (id, singlematch) descriptors are
+                                         // Database::reports[report_begin[k] .. report_begin[k + 1])
+};
+
 struct Database {
     std::vector<PatternInfo> patterns;
     std::vector<NfaPattern> nfas;
@@ -66,6 +85,10 @@ struct Database {
     std::string key;   // cache key: patterns + flags + ids
     bool literal = false;   // fixed-string set: no groups, `literals` holds what a line is matched against
     LiteralSet literals;
+    // fixed-string set compiled for reports: `literals` selects the lines (simple stays true), then `literal_reports` finds
+    // every (node, end) in them and `reports` expands a node to its ids
+    bool literal_reports = false;
+    LiteralReports lit_reports;
 };
 
 // Return codes follow the reference's enum (hyperscanner.c:25-33): 0 ok, 4 = HYPERSCANNER_DB for any rejection.
@@ -85,6 +108,13 @@ int compile_literal_database(const char* const* literals, const unsigned* flags,
 // Cached like cached_database, apart from it: the literal "a.b" is not the regex "a.b".
 std::shared_ptr<Database> cached_literal_database(const char* const* literals, const unsigned* flags, unsigned n, int& rc,
                                                   std::string& error);
+// Fixed strings with reports (gpugrep_literal_report_scan_*): the set of compile_literal_database plus the report table.
+// SINGLEMATCH is honoured, and literals that share an id must agree on it (4 otherwise, as compile_database).  `ids` null:
+// all 0.  Cached apart from both kinds above.
+int compile_literal_report_database(const char* const* literals, const unsigned* flags, const unsigned* ids, unsigned n,
+                                    std::shared_ptr<Database>& out, std::string& error);
+std::shared_ptr<Database> cached_literal_report_database(const char* const* literals, const unsigned* flags, const unsigned* ids,
+                                                         unsigned n, int& rc, std::string& error);
 
 inline uint8_t fold_ascii(uint8_t b) { return (uint8_t)((unsigned)b - 'A' < 26u ? b | 0x20u : b); }
 

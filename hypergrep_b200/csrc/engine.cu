@@ -15,6 +15,9 @@
 // instead of the automata (k_spans.cuh).
 // FIXED STRINGS (grep -F, slot_set_literals): the same two paths without automata; k_verify_literals takes the place of the
 // DFA verification (k_confirm always runs before it) and k_match_pl_literals that of k_match_pl_simple (k_literal.cuh).
+// FIXED-STRING REPORTS (gpugrep_literal_report_scan_*, slot_set_literal_reports): the lines are selected as above, then
+// k_literal_reports (count) -> scan -> k_literal_reports (write) finds every (literal, end) in the selected lines only
+// (k_literal_reports.cuh).
 // CONTEXT lines (grep -A/-B/-C, scans with records): a window test over the prefix count of the selected lines picks the
 // output lines of a segment (k_context.cuh, after the dedupe on the fast path, after k_match_pl_simple on the general path).
 // All byte offsets inside a segment are 32-bit (segments are < 4 GiB); line numbers are rebased on the host.
@@ -42,6 +45,7 @@
 #include "scan.cuh"
 #include "dfa_walk.cuh"
 #include "k_literal.cuh"
+#include "k_literal_reports.cuh"
 #include "k_fast.cuh"
 #include "k_general.cuh"
 #include "k_invert.cuh"
@@ -142,6 +146,8 @@ struct DeviceDb {
     size_t smem_table_bytes = 0;   // single group with a class-compressed table (GroupDev::ctab): its size, else 0
     bool literal = false;          // fixed-string set: `lits` instead of groups
     LiteralView lits{};
+    bool literal_reports = false;  // fixed-string set with a report table: `reps`
+    LiteralReportView reps{};
     ~DeviceDb() { for (void* p : allocs) cudaFree(p); }
 };
 
@@ -201,11 +207,13 @@ public:
     uint32_t ctx_before = 0, ctx_after = 0;   // context lines (slot_set_context)
     const PikeProgram* pike = nullptr;        // span stage (slot_set_spans)
     bool literal = false;                     // fixed-string scan (slot_set_literals)
+    bool reports = false;                     // fixed-string report stage (slot_set_literal_reports)
     SegmentStats stats;
     bool in_use = false;
 
     int run_general(SegmentResult& out, std::string& error, size_t split_above);
     int run_spans(SegmentResult& out, size_t npl_total, std::string& error, size_t split_above);
+    int run_reports(SegmentResult& out, size_t nrec, std::string& error, size_t split_above);
     int run_complement(size_t nrec, size_t nlines, size_t selected, std::string& error);
     int run_context(size_t nrec, size_t nlines, size_t selected, size_t& count, std::string& error);
     bool context() const { return want_records && (ctx_before || ctx_after); }
@@ -273,6 +281,26 @@ std::shared_ptr<DeviceDb> engine_upload(const std::shared_ptr<Database>& db, std
         if (!v.bytes || !v.off || !v.len || !v.order || !v.bucket || !v.one) { error = "cudaMalloc/cudaMemcpy failed while uploading the literals"; return nullptr; }
         out->literal = true;
         out->lits = v;
+    }
+    if (db->literal_reports) {
+        const LiteralReports& R = db->lit_reports;
+        std::vector<uint8_t> bytes(R.bytes);
+        bytes.resize(bytes.size() + 16, 0);   // (k_literal.cuh lit_compare: 8-byte loads)
+        LiteralReportView v{};
+        v.lits.bytes = (const uint8_t*)upload(bytes.data(), bytes.size());
+        v.lits.off = (const uint32_t*)upload(R.off.data(), R.off.size() * 4);
+        v.lits.len = (const uint32_t*)upload(R.len.data(), R.len.size() * 4);
+        v.lits.order = (const uint32_t*)upload(R.order.data(), R.order.size() * 4);
+        v.lits.bucket = (const uint32_t*)upload(R.bucket.data(), R.bucket.size() * 4);
+        v.parent = (const uint32_t*)upload(R.parent.data(), R.parent.size() * 4);
+        v.one = (const uint32_t*)upload(R.one.data(), R.one.size() * 4);
+        for (uint8_t c : R.caseless) v.lits.classes |= 1u << c;
+        if (!v.lits.bytes || !v.lits.off || !v.lits.len || !v.lits.order || !v.lits.bucket || !v.parent || !v.one) {
+            error = "cudaMalloc/cudaMemcpy failed while uploading the literal report table";
+            return nullptr;
+        }
+        out->literal_reports = true;
+        out->reps = v;
     }
     std::vector<GroupDev> groups;
     for (size_t g = 0; g < db->groups.size(); g++) {
@@ -525,6 +553,7 @@ void slot_set_want_records(ScanSlot* slot, bool want) { slot->want_records = wan
 void slot_set_invert(ScanSlot* slot, bool invert) { slot->invert = invert; }
 void slot_set_spans(ScanSlot* slot, const PikeProgram* program) { slot->pike = program; }
 void slot_set_literals(ScanSlot* slot, bool literal) { slot->literal = literal; }
+void slot_set_literal_reports(ScanSlot* slot, bool reports) { slot->reports = reports; }
 void slot_set_context(ScanSlot* slot, uint32_t before, uint32_t after) {
     slot->ctx_before = before;
     slot->ctx_after = after;
@@ -597,6 +626,7 @@ int slot_submit(ScanSlot* s, const DeviceDb& ddb, const DevicePrefilter* pf, con
                 int buffer_size, void* user_stream, std::string& error) {
     if (n >= ((size_t)1 << 32) - 1024) { error = "segment too large"; return 7; }
     if (s->literal != ddb.literal) { error = "fixed-string scan of a database that is not a fixed-string set, or the reverse"; return 7; }
+    if (s->reports && (!ddb.literal_reports || !s->want_records)) { error = "fixed-string report scan of a database without a report table, or without records"; return 7; }
     s->stream = user_stream ? (cudaStream_t)user_stream : s->own_stream;
     cudaStream_t st = s->stream;
     s->ddb = &ddb;
@@ -873,6 +903,13 @@ int ScanSlot::run_general(SegmentResult& out, std::string& error, size_t split_a
         CUDA_TRY(cudaMemcpyAsync(hT, dT, sizeof(Totals), cudaMemcpyDeviceToHost, st));
         CUDA_TRY(cudaStreamSynchronize(st));
         size_t nrec = (size_t)(ctx ? hT->aux_total : hT->rec_total);
+        if (reports && nrec) {
+            if (d_recs.reserve(nrec * sizeof(LineRec)) != cudaSuccess) { error = "cudaMalloc failed"; return 3; }
+            k_emit_pl_simple<<<(unsigned)((npl_total + 255) / 256), 256, 0, st>>>(d_plstart.as<uint32_t>(), d_pllen.as<uint32_t>(), npl_total,
+                                                                                    d_flags.as<uint8_t>(), d_recoff.as<unsigned long long>(), d_recs.as<LineRec>());
+            stats.launches++;
+        }
+        if (reports) return run_reports(out, nrec, error, split_above);
         if (nrec) {
             if (d_recs.reserve(nrec * sizeof(LineRec)) != cudaSuccess) { error = "cudaMalloc failed"; return 3; }
             if (h_recs.reserve(nrec * sizeof(LineRec)) != cudaSuccess) { error = "cudaHostAlloc failed"; return 3; }
@@ -969,6 +1006,56 @@ int ScanSlot::run_spans(SegmentResult& out, size_t npl_total, std::string& error
     CUDA_TRY(cudaGetLastError());
     out.spans = h_recs.as<SpanRec>();
     out.num_spans = nspan;
+    return 0;
+}
+
+// Report stage of a fixed-string report scan: the events of the first `nrec` records of d_recs (the selected lines, in line
+// order; kLineInvalid ones skipped), in line order, copied to h_recs.
+int ScanSlot::run_reports(SegmentResult& out, size_t nrec, std::string& error, size_t split_above) {
+    cudaStream_t st = stream;
+    Totals* dT = d_totals.as<Totals>();
+    Totals* hT = h_totals.as<Totals>();
+    out.lines = nullptr;
+    out.num_line_recs = out.num_valid_recs = 0;
+    out.events = nullptr;
+    out.num_events = 0;
+    size_t nev = 0;
+    if (nrec) {
+        const size_t nb_scan = (nrec + kScanTile - 1) / kScanTile + 1;
+        if (d_counts.reserve(nrec * 4) != cudaSuccess || d_recoff.reserve(nrec * 8) != cudaSuccess || d_sums.reserve(nb_scan * 8) != cudaSuccess) {
+            error = "cudaMalloc failed for the report stage"; return 3;
+        }
+        static const unsigned per_sm = blocks_per_sm(k_literal_reports, 128);
+        const unsigned grid = (unsigned)std::min<size_t>((nrec + 3) / 4, (size_t)per_sm * device_sms());   // a warp per record
+        const LineRec* recs = d_recs.as<LineRec>();
+        k_literal_reports<<<grid, 128, 0, st>>>(ddb->reps, data, recs, nrec, d_counts.as<uint32_t>(), nullptr, nullptr);
+        stats.launches++;
+        launch_scan(st, LoadU32{d_counts.as<uint32_t>()}, nrec, d_recoff.as<unsigned long long>(), d_sums.as<unsigned long long>(), &dT->rec_total, stats);
+        CUDA_TRY(cudaMemcpyAsync(hT, dT, sizeof(Totals), cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+        nev = (size_t)hT->rec_total;
+        if (nev > ((size_t)1 << 27)) {
+            if (split_above && n > split_above) return kSplitSegment;
+            error = "too many match events in one segment (non-SINGLEMATCH pattern matching nearly every byte?)";
+            return 7;
+        }
+        if (nev) {
+            if (d_events.reserve(nev * sizeof(EventRec)) != cudaSuccess) { error = "cudaMalloc failed"; return 3; }
+            if (h_recs.reserve(nev * sizeof(EventRec)) != cudaSuccess) { error = "cudaHostAlloc failed"; return 3; }
+            k_literal_reports<<<grid, 128, 0, st>>>(ddb->reps, data, recs, nrec, d_counts.as<uint32_t>(), d_recoff.as<unsigned long long>(),
+                                                    d_events.as<EventRec>());
+            stats.launches++;
+        }
+    }
+    CUDA_TRY(cudaEventRecord(ev[1], st));
+    if (nev) {
+        CUDA_TRY(cudaMemcpyAsync(h_recs.p, d_events.p, nev * sizeof(EventRec), cudaMemcpyDeviceToHost, st));
+        stats.d2h_bytes += nev * sizeof(EventRec);
+    }
+    CUDA_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaGetLastError());
+    out.events = h_recs.as<EventRec>();
+    out.num_events = nev;
     return 0;
 }
 
@@ -1073,7 +1160,12 @@ int slot_collect(ScanSlot* s, SegmentResult& out, std::string& error, size_t spl
             out.num_valid_recs = (size_t)hT->aux_total;
             const size_t nl_total = (size_t)(uint32_t)hT->meta_total;
             out.num_lines = nl_total + ((hT->last_byte & 0xff) != '\n' ? 1 : 0);
-            if (s->context()) {
+            if (s->reports) {
+                int rc = s->run_reports(out, nrec, error, split_above);
+                if (rc == kSplitSegment) out.stats = s->stats;
+                if (rc) return rc;
+                nrec = 0;
+            } else if (s->context()) {
                 const size_t selected = s->invert ? (size_t)out.num_lines - out.num_valid_recs : out.num_valid_recs;
                 size_t count = 0;
                 int rc = s->run_context(nrec, (size_t)out.num_lines, selected, count, error);
@@ -1095,8 +1187,10 @@ int slot_collect(ScanSlot* s, SegmentResult& out, std::string& error, size_t spl
                 CUDA_TRY(cudaStreamSynchronize(s->copy_stream));
                 s->stats.d2h_bytes += nrec * sizeof(LineRec);
             }
-            out.lines = s->want_records ? s->h_recs.as<LineRec>() : nullptr;
-            out.num_line_recs = nrec;
+            if (!s->reports) {
+                out.lines = s->want_records ? s->h_recs.as<LineRec>() : nullptr;
+                out.num_line_recs = nrec;
+            }
             done = true;
         }
     }

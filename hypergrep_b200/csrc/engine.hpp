@@ -115,6 +115,11 @@ __attribute__((weak)) void slot_set_spans(ScanSlot* slot, const PikeProgram* pro
 // is matched against its literals instead of automata, on both paths.  Call before slot_submit, which fails with 7 when the
 // database is not of the kind the slot is set to.  Weak like slot_set_invert (a build without it fails such scans with 7).
 __attribute__((weak)) void slot_set_literals(ScanSlot* slot, bool literal);
+// Fixed-string reports (gpugrep_literal_report_scan_*): on a fixed-string slot whose database has a report table
+// (Database::literal_reports), the lines are selected as without it, then a report stage finds every (node of the report
+// table, end) in the selected lines: the segment's results are EventRecs whose `report` is that node (no line records;
+// count-only is off).  Weak like slot_set_invert (a build without it fails such scans with 7).
+__attribute__((weak)) void slot_set_literal_reports(ScanSlot* slot, bool reports);
 // Wait for the segment and expose its results (valid until the next slot_submit on this slot).
 // Returns kSplitSegment (and no results) when the fast path hit one of its capacity bounds - a line too long for it, a
 // candidate or record overflow - in a segment of more than `split_above` bytes: the caller then scans the same bytes again

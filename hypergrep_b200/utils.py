@@ -287,6 +287,56 @@ def _literal_entry(lib: ctypes.CDLL):
     return entry
 
 
+def _literal_report_entry(lib: ctypes.CDLL):
+    """gpugrep_literal_report_scan_file of the loaded library (see _literal_entry)."""
+    try:
+        entry = lib.gpugrep_literal_report_scan_file
+    except AttributeError as error:
+        raise NotImplementedError(
+            "scan_literals needs gpugrep_literal_report_scan_file, which the loaded native library does not export "
+            f"({_library_path()}); there is no CPU fallback"
+        ) from error
+    entry.restype = ctypes.c_int
+    entry.argtypes = _FILE_ENTRY_ARGTYPES
+    return entry
+
+
+def scan_literals(  # pylint: disable=too-many-arguments
+    path: str,
+    literals: Sequence[str],
+    callback: Callable,
+    flags: Sequence[int] = (),
+    ids: Sequence[int] = (),
+    buffer_size: int = 262140,
+    buffer_count: int = 16,
+    max_match_count: int = 0,
+) -> int:
+    """Scan one plain/gzip/zstd file for fixed strings and report which literal matched (gpugrep_literal_report_scan_file).
+
+    The records are those of :func:`scan` on the same set with the UTF-8 bytes of every literal written as ``\\xHH``, the same
+    flags and the same ids: one record per distinct (id, match end) in a line, a SINGLEMATCH id once per line, in the order
+    of the match ends.  Only ``HS_FLAG_CASELESS`` (A-Z / a-z folded) and ``HS_FLAG_SINGLEMATCH`` change anything.  Defaults
+    follow :func:`prepare_patterns`: DOTALL|MULTILINE|SINGLEMATCH and ids all 0, which gives the records of
+    ``scan(..., fixed_strings=True)``.  No automaton is built, so lists of 10^6 literals work.
+    """
+    pattern_array, flags_array, ids_array = prepare_patterns(literals, flags=flags, ids=ids)
+    c_callback = CALLBACK_TYPE(callback)
+    entry = _literal_report_entry(_get_hyperscanner_lib())
+    outcome = {"rc": 0}
+
+    def _run() -> None:
+        outcome["rc"] = entry(path.encode(), pattern_array, flags_array, ids_array, len(pattern_array), c_callback, buffer_size,
+                              buffer_count, max_match_count, None)
+
+    worker = threading.Thread(target=_run, daemon=True)   # same interruptible wait as scan()
+    worker.start()
+    try:
+        worker.join(timeout=3600)
+    except KeyboardInterrupt:
+        outcome["rc"] = _RC_INTERRUPTED
+    return outcome["rc"]
+
+
 def _literal_check_entry(lib: ctypes.CDLL):
     """gpugrep_check_literals of the loaded library (see _literal_entry)."""
     try:
@@ -365,9 +415,12 @@ def grep(  # pylint: disable=too-many-arguments
     selected line; results are then ``(line number, line text, is_context)``.  ``count_only`` and ``only_matching`` ignore
     context.  Negative counts raise ValueError.
     ``fixed_strings`` (``grep -F``): the patterns are literals (:func:`scan`).  With ``only_matching`` the result is that of
-    the ``re.escape``-d patterns as regular expressions.
+    the ``re.escape``-d patterns as regular expressions: every record has id 0, and the reference takes the parts of the
+    pattern that the id indexes, so they are the occurrences of the first literal alone (case-sensitive, as ``re.compile``).
     """
     _check_context(before_context, after_context)
+    if fixed_strings and only_matching and not invert_match:
+        return _grep_fixed_only_matching(file, patterns, ignore_case, count_only, no_messages, errors, max_match_count)
     if fixed_strings and only_matching:
         patterns = [re.escape(pattern) for pattern in patterns]
         fixed_strings = False
@@ -446,6 +499,42 @@ def grep(  # pylint: disable=too-many-arguments
         _fill_spans(groups, deferred, patterns, widths, python_patterns, errors, span_lines)
         collected = [entry for group in groups for entry in group]
     return (counter[0] if count_only else collected), code
+
+
+def _grep_fixed_only_matching(file: str, literals: list[str], ignore_case: bool, count_only: bool, no_messages: bool, errors: str,
+                              max_match_count: int) -> tuple[int | list[tuple[int, str]], int]:
+    """``grep(fixed_strings=True, only_matching=True)`` without automata: the literal scan selects the lines (the records of
+    the escaped set, ids 0), and the parts are those of ``re.escape(literals[0])``: a left-to-right, non-overlapping
+    ``bytes.find`` on ASCII lines, ``re.finditer`` of that one pattern on the others."""
+    if count_only:
+        return grep(file, literals, ignore_case=ignore_case, count_only=True, no_messages=no_messages, errors=errors,
+                    max_match_count=max_match_count, fixed_strings=True)
+    if not os.path.exists(file) or os.path.isdir(file):   # the errors of grep() itself
+        return grep(file, literals, no_messages=no_messages, fixed_strings=True)
+    first = literals[0] if literals else ""
+    needle = first.encode()
+    first_pattern = None
+    collected: list[tuple[int, str]] = []
+
+    def _on_batch(matches: ctypes.Array, count: int) -> None:
+        nonlocal first_pattern
+        for position in range(count):
+            record = matches[position]
+            raw, number = record.line, record.line_number + 1
+            if raw.isascii():
+                at = raw.find(needle)
+                while at >= 0:
+                    collected.append((number, needle.decode() + "\n"))
+                    at = raw.find(needle, at + len(needle))
+                continue
+            if first_pattern is None:
+                first_pattern = re.compile(re.escape(first))
+            collected.extend((number, f"{part.group()}\n") for part in first_pattern.finditer(raw.decode(errors=errors)))
+
+    pattern_flags = _DEFAULT_FLAGS | (HS_FLAG_CASELESS if ignore_case else 0)
+    code = scan(file, literals, _on_batch, flags=[pattern_flags] * len(literals), max_match_count=max_match_count,
+                buffer_count=_GREP_BATCH, fixed_strings=True)
+    return collected, code
 
 
 class _MatchEnd(ctypes.Structure):

@@ -171,6 +171,30 @@ GPUGREP_API int gpugrep_literal_scan_buffer(const void* data, size_t size, int l
                                 int invert, void* stream, gpugrep_stats* stats);
 GPUGREP_API int gpugrep_check_literals(const char* const* literals, const unsigned int* literal_flags, unsigned int elements);
 
+/* ---- fixed strings with reports: which literal matched, and where --------------------------------------------------
+ * The records are exactly those of hyperscan() / gpugrep_scan_buffer for the same set with every byte written as \xHH,
+ * the same flags and the same ids (`literal_ids` NULL: all 0; `literal_flags` NULL: all 0).  That is:
+ *  - flags: CASELESS folds A-Z / a-z only, as above; SINGLEMATCH is honoured; DOTALL and MULTILINE change nothing; any
+ *    other bit, an empty literal or elements == 0 return 4, as do literals that share an id but disagree on SINGLEMATCH.
+ *  - a report is (id, end) for every occurrence of a literal in the scanned block of a pseudo-line (formed as above);
+ *    `end` is the offset just past the occurrence, counted from the block start after leading NULs are skipped.  A record
+ *    carries the id and the line; its end is not delivered (gpugrep_match_ends has ends).
+ *  - within a line, reports go out by end offset, then id, one per distinct (id, end); a SINGLEMATCH id reports once per
+ *    block, at its first end.  Duplicate literals, and literals that are prefixes or suffixes of one another, all report.
+ *  - max_match_count counts records and is checked after all reports of a line; batches, on_event == NULL counting
+ *    (stats->matches), every input form and $GPUGREP_DEVICES sharding follow hyperscan().
+ * With ids all 0 and SINGLEMATCH on every literal, the records equal those of gpugrep_literal_scan_* without context.
+ * There are no context lines or inverted form.  Lines are selected as gpugrep_literal_scan_* selects them, then a report
+ * stage on the GPU finds every (literal, end) in the selected lines only.  A build of the engine without the report stage
+ * returns 7. */
+GPUGREP_API int gpugrep_literal_report_scan_file(const char* file_name, const char* const* literals, const unsigned int* literal_flags,
+                                     const unsigned int* literal_ids, unsigned int elements, hs_event on_event, int buffer_size,
+                                     int buffer_count, unsigned long long max_match_count, gpugrep_stats* stats);
+GPUGREP_API int gpugrep_literal_report_scan_buffer(const void* data, size_t size, int location, const char* const* literals,
+                                       const unsigned int* literal_flags, const unsigned int* literal_ids, unsigned int elements,
+                                       hs_event on_event, int buffer_size, int buffer_count, unsigned long long max_match_count,
+                                       void* stream, gpugrep_stats* stats);
+
 /* ---- match END offsets (SURVEY.md section 8f-4: spans for `grep -o`) --------------------------------------------
  * The reference gets the spans of `-o` by re-running Python's re.finditer() over every matched line (utils.py:205-212);
  * Hyperscan itself reports (id, end offset) per match and the reference drops the offset (hyperscanner.c:83-102).
