@@ -544,6 +544,7 @@ struct Params {
     bool context_scan = false;  // gpugrep_context_scan_*(): lines around the selected ones too
     bool literal = false;       // gpugrep_literal_scan_*(): `patterns` are fixed strings (flags: CASELESS only, no ids)
     bool literal_reports = false;   // gpugrep_literal_report_scan_*(): fixed strings with ids, one record per (id, end)
+    unsigned whole = 0;         // gpugrep_literal_whole_scan_*(): GPUGREP_WHOLE_WORD or GPUGREP_WHOLE_LINE
     uint32_t before = 0, after = 0;
     // the context stage runs only when lines are delivered (count-only scans ignore context)
     bool context() const { return context_scan && cb != nullptr && (before || after); }
@@ -574,11 +575,13 @@ void set_spans(ScanSlot* slot, const Params& pr) {
 void set_literals(ScanSlot* slot, const Params& pr) {
     if (slot_set_literals) slot_set_literals(slot, pr.literal);
     if (slot_set_literal_reports) slot_set_literal_reports(slot, pr.literal_reports);
+    if (slot_set_literal_whole) slot_set_literal_whole(slot, pr.whole);
 }
 
 int setup_job(const Params& pr, Job& job, Deliverer& out, unsigned long long weight = 0) {
     int rc = 0;
     if (pr.literal_reports) job.db = cached_literal_report_database(pr.patterns, pr.flags, pr.ids, pr.elements, rc, job.error);
+    else if (pr.whole) job.db = cached_literal_whole_database(pr.patterns, pr.flags, pr.elements, rc, job.error);
     else if (pr.literal) job.db = cached_literal_database(pr.patterns, pr.flags, pr.elements, rc, job.error);
     else job.db = cached_database(pr.patterns, pr.flags, pr.ids, pr.elements, rc, job.error);
     if (job.db && !pr.literal && (pr.invert || pr.context_scan)) {
@@ -598,6 +601,7 @@ int setup_job(const Params& pr, Job& job, Deliverer& out, unsigned long long wei
     if (pr.span_program && !slot_set_spans) { job.error = "this build of the engine has no span stage"; return GPUGREP_SCAN; }
     if (pr.literal && !slot_set_literals) { job.error = "this build of the engine has no fixed-string stage"; return GPUGREP_SCAN; }
     if (pr.literal_reports && !slot_set_literal_reports) { job.error = "this build of the engine has no fixed-string report stage"; return GPUGREP_SCAN; }
+    if (pr.whole && !slot_set_literal_whole) { job.error = "this build of the engine has no whole-word / whole-line stage"; return GPUGREP_SCAN; }
     job.device_weight = weight;
     job.device = pick_device(weight, &job.device_charged);
     if (engine_select_device(job.device, job.error) != 0) {
@@ -1289,6 +1293,35 @@ int gpugrep_literal_scan_buffer(const void* data, size_t size, int location, con
                                 unsigned int before, unsigned int after, int invert, void* stream, gpugrep_stats* stats) {
     gpugrep::Params pr{literals, literal_flags, nullptr, elements, on_event, buffer_size, buffer_count, max_match_count, stream};
     pr.literal = true;
+    pr.invert = invert != 0;
+    pr.context_scan = true;
+    pr.before = before;
+    pr.after = after;
+    return gpugrep::scan_buffer(data, size, location, pr, stats);
+}
+
+int gpugrep_literal_whole_scan_file(const char* file_name, const char* const* literals, const unsigned int* literal_flags, unsigned int elements,
+                                    unsigned int whole, hs_event on_event, int buffer_size, int buffer_count, unsigned long long max_match_count,
+                                    unsigned int before, unsigned int after, int invert, gpugrep_stats* stats) {
+    if (whole != GPUGREP_WHOLE_WORD && whole != GPUGREP_WHOLE_LINE) { gpugrep::set_last_error("whole must be GPUGREP_WHOLE_WORD or GPUGREP_WHOLE_LINE"); return GPUGREP_DB; }
+    gpugrep::Params pr{literals, literal_flags, nullptr, elements, on_event, buffer_size, buffer_count, max_match_count, nullptr};
+    pr.literal = true;
+    pr.whole = whole;
+    pr.invert = invert != 0;
+    pr.context_scan = true;
+    pr.before = before;
+    pr.after = after;
+    return gpugrep::scan_path(file_name, pr, stats);
+}
+
+int gpugrep_literal_whole_scan_buffer(const void* data, size_t size, int location, const char* const* literals, const unsigned int* literal_flags,
+                                      unsigned int elements, unsigned int whole, hs_event on_event, int buffer_size, int buffer_count,
+                                      unsigned long long max_match_count, unsigned int before, unsigned int after, int invert, void* stream,
+                                      gpugrep_stats* stats) {
+    if (whole != GPUGREP_WHOLE_WORD && whole != GPUGREP_WHOLE_LINE) { gpugrep::set_last_error("whole must be GPUGREP_WHOLE_WORD or GPUGREP_WHOLE_LINE"); return GPUGREP_DB; }
+    gpugrep::Params pr{literals, literal_flags, nullptr, elements, on_event, buffer_size, buffer_count, max_match_count, stream};
+    pr.literal = true;
+    pr.whole = whole;
     pr.invert = invert != 0;
     pr.context_scan = true;
     pr.before = before;

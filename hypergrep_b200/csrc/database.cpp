@@ -345,23 +345,9 @@ std::shared_ptr<Database> cached_literal_database(const char* const* literals, c
                   [&](std::shared_ptr<Database>& db) { return compile_literal_database(literals, flags, n, db, error); }, rc);
 }
 
-int compile_literal_report_database(const char* const* literals, const unsigned* flags, const unsigned* ids, unsigned n,
-                                    std::shared_ptr<Database>& out, std::string& error) {
-    const int kDbError = 4;
-    int rc = check_literals(literals, flags, n, error);
-    if (rc) return rc;
-    {   // hs_compile.h: expressions sharing a match id must agree on SINGLEMATCH
-        std::map<unsigned, unsigned> sm;
-        for (unsigned i = 0; i < n; i++) {
-            const unsigned id = ids ? ids[i] : 0u, v = flags ? flags[i] & FLAG_SINGLEMATCH : 0u;
-            auto it = sm.emplace(id, v).first;
-            if (it->second != v) { error = "literals sharing id " + std::to_string(id) + " disagree on SINGLEMATCH"; return kDbError; }
-        }
-    }
-    rc = compile_literal_database(literals, flags, n, out, error);
-    if (rc) return rc;
-    Database& db = *out;
-    db.literal_reports = true;
+// The report table (database.hpp LiteralReports) of the literals that can lie inside a line, and the (id, singlematch)
+// descriptors of its nodes in db.reports.  The literals have passed check_literals.
+static void build_literal_reports(const char* const* literals, const unsigned* flags, const unsigned* ids, unsigned n, Database& db) {
     LiteralReports& R = db.lit_reports;
     struct Given { std::string text; unsigned cls, id, sm; };
     std::vector<Given> given;
@@ -422,6 +408,25 @@ int compile_literal_report_database(const char* const* literals, const unsigned*
         }
         R.bucket[cls * 65537 + 65536] = at;
     }
+}
+
+int compile_literal_report_database(const char* const* literals, const unsigned* flags, const unsigned* ids, unsigned n,
+                                    std::shared_ptr<Database>& out, std::string& error) {
+    const int kDbError = 4;
+    int rc = check_literals(literals, flags, n, error);
+    if (rc) return rc;
+    {   // hs_compile.h: expressions sharing a match id must agree on SINGLEMATCH
+        std::map<unsigned, unsigned> sm;
+        for (unsigned i = 0; i < n; i++) {
+            const unsigned id = ids ? ids[i] : 0u, v = flags ? flags[i] & FLAG_SINGLEMATCH : 0u;
+            auto it = sm.emplace(id, v).first;
+            if (it->second != v) { error = "literals sharing id " + std::to_string(id) + " disagree on SINGLEMATCH"; return kDbError; }
+        }
+    }
+    rc = compile_literal_database(literals, flags, n, out, error);
+    if (rc) return rc;
+    build_literal_reports(literals, flags, ids, n, *out);
+    out->literal_reports = true;
     return 0;
 }
 
@@ -432,6 +437,25 @@ std::shared_ptr<Database> cached_literal_report_database(const char* const* lite
     key.append("\x01reports");
     return cached(true, std::move(key),
                   [&](std::shared_ptr<Database>& db) { return compile_literal_report_database(literals, flags, ids, n, db, error); }, rc);
+}
+
+int compile_literal_whole_database(const char* const* literals, const unsigned* flags, unsigned n, std::shared_ptr<Database>& out,
+                                   std::string& error) {
+    int rc = compile_literal_database(literals, flags, n, out, error);
+    if (rc) return rc;
+    // (ids and SINGLEMATCH do not matter here: the table only tells which literals occur where)
+    build_literal_reports(literals, flags, nullptr, n, *out);
+    out->literal_whole = true;
+    return 0;
+}
+
+std::shared_ptr<Database> cached_literal_whole_database(const char* const* literals, const unsigned* flags, unsigned n, int& rc,
+                                                        std::string& error) {
+    // (one entry serves word and line scans: the mode is a slot setting; the tag keeps it apart from the other two kinds)
+    std::string key = cache_key(literals, flags, nullptr, n);
+    key.append("\x01whole");
+    return cached(true, std::move(key),
+                  [&](std::shared_ptr<Database>& db) { return compile_literal_whole_database(literals, flags, n, db, error); }, rc);
 }
 
 }  // namespace gpugrep

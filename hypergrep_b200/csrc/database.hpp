@@ -89,6 +89,9 @@ struct Database {
     // every (node, end) in them and `reports` expands a node to its ids
     bool literal_reports = false;
     LiteralReports lit_reports;
+    // fixed-string set compiled for whole-word / whole-line scans (gpugrep_literal_whole_scan_*): `literals` selects the
+    // lines, then `lit_reports` (ids 0) decides which of them hold a literal as a word or as the whole line
+    bool literal_whole = false;
 };
 
 // Return codes follow the reference's enum (hyperscanner.c:25-33): 0 ok, 4 = HYPERSCANNER_DB for any rejection.
@@ -115,6 +118,13 @@ int compile_literal_report_database(const char* const* literals, const unsigned*
                                     std::shared_ptr<Database>& out, std::string& error);
 std::shared_ptr<Database> cached_literal_report_database(const char* const* literals, const unsigned* flags, const unsigned* ids,
                                                          unsigned n, int& rc, std::string& error);
+// Fixed strings for whole-word and whole-line scans (gpugrep_literal_whole_scan_*): the set of compile_literal_database
+// plus the report table of every literal, not only the prefix-free kept ones (`foo` must not hide `foobar`).  One database
+// serves both modes.  Cached apart from the three kinds above.
+int compile_literal_whole_database(const char* const* literals, const unsigned* flags, unsigned n, std::shared_ptr<Database>& out,
+                                   std::string& error);
+std::shared_ptr<Database> cached_literal_whole_database(const char* const* literals, const unsigned* flags, unsigned n, int& rc,
+                                                        std::string& error);
 
 inline uint8_t fold_ascii(uint8_t b) { return (uint8_t)((unsigned)b - 'A' < 26u ? b | 0x20u : b); }
 

@@ -18,6 +18,10 @@
 // FIXED-STRING REPORTS (gpugrep_literal_report_scan_*, slot_set_literal_reports): the lines are selected as above, then
 // k_literal_reports (count) -> scan -> k_literal_reports (write) finds every (literal, end) in the selected lines only
 // (k_literal_reports.cuh).
+// WHOLE-WORD / WHOLE-LINE FIXED STRINGS (gpugrep_literal_whole_scan_*, slot_set_literal_whole): the fast path runs the
+// fixed-string chain up to k_emit_nlm<*, LITERAL> (records even in count-only scans), then k_literal_whole_filter drops the
+// records of lines without a word / whole-line occurrence before k_dedupe_records counts them; the general path takes
+// k_match_pl_literal_whole in place of k_match_pl_literals (k_literal_whole.cuh).
 // CONTEXT lines (grep -A/-B/-C, scans with records): a window test over the prefix count of the selected lines picks the
 // output lines of a segment (k_context.cuh, after the dedupe on the fast path, after k_match_pl_simple on the general path).
 // All byte offsets inside a segment are 32-bit (segments are < 4 GiB); line numbers are rebased on the host.
@@ -46,6 +50,7 @@
 #include "dfa_walk.cuh"
 #include "k_literal.cuh"
 #include "k_literal_reports.cuh"
+#include "k_literal_whole.cuh"
 #include "k_fast.cuh"
 #include "k_general.cuh"
 #include "k_invert.cuh"
@@ -147,6 +152,7 @@ struct DeviceDb {
     bool literal = false;          // fixed-string set: `lits` instead of groups
     LiteralView lits{};
     bool literal_reports = false;  // fixed-string set with a report table: `reps`
+    bool literal_whole = false;    // fixed-string set for whole-word / whole-line scans: the report table is in `reps` too
     LiteralReportView reps{};
     ~DeviceDb() { for (void* p : allocs) cudaFree(p); }
 };
@@ -208,6 +214,7 @@ public:
     const PikeProgram* pike = nullptr;        // span stage (slot_set_spans)
     bool literal = false;                     // fixed-string scan (slot_set_literals)
     bool reports = false;                     // fixed-string report stage (slot_set_literal_reports)
+    unsigned whole = 0;                       // whole-word (1) / whole-line (2) fixed strings (slot_set_literal_whole)
     SegmentStats stats;
     bool in_use = false;
 
@@ -282,7 +289,7 @@ std::shared_ptr<DeviceDb> engine_upload(const std::shared_ptr<Database>& db, std
         out->literal = true;
         out->lits = v;
     }
-    if (db->literal_reports) {
+    if (db->literal_reports || db->literal_whole) {
         const LiteralReports& R = db->lit_reports;
         std::vector<uint8_t> bytes(R.bytes);
         bytes.resize(bytes.size() + 16, 0);   // (k_literal.cuh lit_compare: 8-byte loads)
@@ -299,7 +306,8 @@ std::shared_ptr<DeviceDb> engine_upload(const std::shared_ptr<Database>& db, std
             error = "cudaMalloc/cudaMemcpy failed while uploading the literal report table";
             return nullptr;
         }
-        out->literal_reports = true;
+        out->literal_reports = db->literal_reports;
+        out->literal_whole = db->literal_whole;
         out->reps = v;
     }
     std::vector<GroupDev> groups;
@@ -554,6 +562,7 @@ void slot_set_invert(ScanSlot* slot, bool invert) { slot->invert = invert; }
 void slot_set_spans(ScanSlot* slot, const PikeProgram* program) { slot->pike = program; }
 void slot_set_literals(ScanSlot* slot, bool literal) { slot->literal = literal; }
 void slot_set_literal_reports(ScanSlot* slot, bool reports) { slot->reports = reports; }
+void slot_set_literal_whole(ScanSlot* slot, unsigned whole) { slot->whole = whole; }
 void slot_set_context(ScanSlot* slot, uint32_t before, uint32_t after) {
     slot->ctx_before = before;
     slot->ctx_after = after;
@@ -627,6 +636,7 @@ int slot_submit(ScanSlot* s, const DeviceDb& ddb, const DevicePrefilter* pf, con
     if (n >= ((size_t)1 << 32) - 1024) { error = "segment too large"; return 7; }
     if (s->literal != ddb.literal) { error = "fixed-string scan of a database that is not a fixed-string set, or the reverse"; return 7; }
     if (s->reports && (!ddb.literal_reports || !s->want_records)) { error = "fixed-string report scan of a database without a report table, or without records"; return 7; }
+    if (s->whole && (!ddb.literal_whole || s->whole > kWholeLine)) { error = "whole-word / whole-line scan of a database not compiled for it"; return 7; }
     s->stream = user_stream ? (cudaStream_t)user_stream : s->own_stream;
     cudaStream_t st = s->stream;
     s->ddb = &ddb;
@@ -810,7 +820,8 @@ int slot_submit(ScanSlot* s, const DeviceDb& ddb, const DevicePrefilter* pf, con
         // Without records (count-only scans) the emit kernel writes one 4-byte key per record into the record buffer, and
         // k_count_keys counts the distinct lines.  Either way a segment with more records than fit falls back to the general
         // path (flags bit 2), so that the count never depends on the capacity.
-        const bool count_only = !s->want_records;
+        // (whole-word / whole-line scans filter line extents: records, also when only the count is wanted)
+        const bool count_only = !s->want_records && !s->whole;
         auto emit_kernel = ddb.literal ? (count_only ? k_emit_nlm<false, true, true> : k_emit_nlm<false, false, true>)
                            : ddb.nnfa > 0 ? (count_only ? k_emit_nlm<true, true> : k_emit_nlm<true, false>)
                                           : (count_only ? k_emit_nlm<false, true> : k_emit_nlm<false, false>);
@@ -819,6 +830,12 @@ int slot_submit(ScanSlot* s, const DeviceDb& ddb, const DevicePrefilter* pf, con
         emit_kernel<<<(unsigned)std::min<size_t>((s->cand_cap + kEmitTile - 1) / kEmitTile, (size_t)emit_per_sm * sms), kEmitThreads, 0, st>>>(
             view, s->data, n, s->d_cand.as<uint32_t>(), s->d_res.as<uint32_t>(), tile_records, meta, prefix, nlmask, &dT->meta_total,
             s->cand_cap, s->d_recs.as<LineRec>(), s->d_recs.as<uint32_t>(), out_cap, dT, ddb.lits);
+        if (s->whole) {
+            static const unsigned whole_per_sm = blocks_per_sm(k_literal_whole_filter, 128);
+            k_literal_whole_filter<<<(unsigned)std::min<size_t>((s->rec_cap + 3) / 4, (size_t)whole_per_sm * sms), 128, 0, st>>>(
+                ddb.reps, s->data, s->d_recs.as<LineRec>(), s->rec_cap, dT, s->whole);
+            s->stats.launches++;
+        }
         if (count_only)
             k_count_keys<<<(unsigned)std::min<size_t>((out_cap + 255) / 256, (size_t)sms * 4), 256, 0, st>>>(s->d_recs.as<uint32_t>(), out_cap, dT);
         else
@@ -885,7 +902,12 @@ int ScanSlot::run_general(SegmentResult& out, std::string& error, size_t split_a
     unsigned mgrid = (unsigned)((npl_total + 127) / 128);
     if (ddb->simple) {
         if (d_flags.reserve(npl_total) != cudaSuccess) { error = "cudaMalloc failed"; return 3; }
-        if (ddb->literal)
+        if (whole) {
+            static const unsigned whole_per_sm = blocks_per_sm(k_match_pl_literal_whole, 128);
+            const unsigned wgrid = (unsigned)std::min<size_t>((npl_total + 3) / 4, (size_t)whole_per_sm * device_sms());   // a warp per pseudo-line
+            k_match_pl_literal_whole<<<wgrid, 128, 0, st>>>(ddb->reps, data, d_plstart.as<uint32_t>(), d_pllen.as<uint32_t>(), npl_total,
+                                                            d_flags.as<uint8_t>(), invert, whole);
+        } else if (ddb->literal)
             k_match_pl_literals<<<mgrid, 128, 0, st>>>(ddb->lits, data, d_plstart.as<uint32_t>(), d_pllen.as<uint32_t>(), npl_total, d_flags.as<uint8_t>(), invert);
         else
             k_match_pl_simple<<<mgrid, 128, 0, st>>>(view, data, d_plstart.as<uint32_t>(), d_pllen.as<uint32_t>(), npl_total, d_flags.as<uint8_t>(), invert);

@@ -120,6 +120,12 @@ __attribute__((weak)) void slot_set_literals(ScanSlot* slot, bool literal);
 // table, end) in the selected lines: the segment's results are EventRecs whose `report` is that node (no line records;
 // count-only is off).  Weak like slot_set_invert (a build without it fails such scans with 7).
 __attribute__((weak)) void slot_set_literal_reports(ScanSlot* slot, bool reports);
+// Whole-word / whole-line fixed strings (gpugrep_literal_whole_scan_*): on a fixed-string slot whose database was compiled
+// for it (Database::literal_whole), `whole` 1 keeps a selected line only when a literal occurs in it as a word, 2 only when
+// the line (its scanned block without the final '\n') is a literal; 0 switches it off.  Everything downstream of the line
+// selection (inversion, context lines, counts, records) follows from the lines kept.  Call before slot_submit.  Weak like
+// slot_set_invert (a build without it fails such scans with 7).
+__attribute__((weak)) void slot_set_literal_whole(ScanSlot* slot, unsigned whole);
 // Wait for the segment and expose its results (valid until the next slot_submit on this slot).
 // Returns kSplitSegment (and no results) when the fast path hit one of its capacity bounds - a line too long for it, a
 // candidate or record overflow - in a segment of more than `split_above` bytes: the caller then scans the same bytes again

@@ -65,6 +65,23 @@ __device__ __forceinline__ uint32_t lit_reports_at(const LiteralReportView& R, c
     return found;
 }
 
+// Whole warp: the scanned block [a, e) of the pseudo-line [st, lim): leading NULs skipped, cut at the next NUL.
+__device__ __forceinline__ void warp_scanned_block(const uint8_t* __restrict__ data, size_t st, size_t lim, size_t& a, size_t& e) {
+    const uint32_t lane = threadIdx.x & 31u;
+    a = st;
+    for (;; a += 32) {
+        const uint32_t nonzero = __ballot_sync(0xffffffffu, a + lane < lim && data[a + lane] != 0);
+        if (nonzero) { a += __ffs(nonzero) - 1; break; }
+        if (a + 32 >= lim) { a = lim; break; }
+    }
+    e = a;
+    for (; e < lim; e += 32) {
+        const uint32_t nul = __ballot_sync(0xffffffffu, e + lane < lim && data[e + lane] == 0);
+        if (nul) { e += __ffs(nul) - 1; break; }
+    }
+    if (e > lim) e = lim;
+}
+
 // Count pass (out == nullptr): counts[r] = events of record r.  Write pass: the events of record r at out + off[r].
 // Records marked kLineInvalid (fast-path repeats, failed NUL re-checks) have none.
 __global__ void __launch_bounds__(128) k_literal_reports(LiteralReportView R, const uint8_t* __restrict__ data, const LineRec* __restrict__ recs,
@@ -79,19 +96,9 @@ __global__ void __launch_bounds__(128) k_literal_reports(LiteralReportView R, co
             continue;
         }
         const size_t st = rec.start, lim = st + (rec.len & kLineLenMask);
-        // the scanned block [a, e): leading NULs skipped, cut at the next NUL (a literal holds no NUL: none spans the cut)
-        size_t a = st;
-        for (;; a += 32) {
-            const uint32_t nonzero = __ballot_sync(0xffffffffu, a + lane < lim && data[a + lane] != 0);
-            if (nonzero) { a += __ffs(nonzero) - 1; break; }
-            if (a + 32 >= lim) { a = lim; break; }
-        }
-        size_t e = a;
-        for (; e < lim; e += 32) {
-            const uint32_t nul = __ballot_sync(0xffffffffu, e + lane < lim && data[e + lane] == 0);
-            if (nul) { e += __ffs(nul) - 1; break; }
-        }
-        if (e > lim) e = lim;
+        // the scanned block [a, e) (a literal holds no NUL: none spans the cut)
+        size_t a, e;
+        warp_scanned_block(data, st, lim, a, e);
         uint32_t total = 0;   // events of the lanes' earlier rounds (write pass: events already written)
         EventRec* dst = out ? out + off[r] : nullptr;
         const uint32_t line_len = rec.len & kLineLenMask;

@@ -161,6 +161,8 @@ def parallel_grep(  # pylint: disable=too-many-arguments,too-many-locals
     after_context: int | None = None,
     group_separator: str | None = "--",
     fixed_strings: bool = False,
+    word_regexp: bool = False,
+    line_regexp: bool = False,
 ) -> int:
     """Scan files and print grep-formatted results (reference multiscanner.py:86-223).
 
@@ -172,7 +174,11 @@ def parallel_grep(  # pylint: disable=too-many-arguments,too-many-locals
     -q ignore them; with -o only the matched parts are printed, and a separator goes between two selected lines whose gap
     exceeds ``before_context + after_context`` lines.
     ``fixed_strings`` (``-F``): the patterns are literals.
+    ``word_regexp`` / ``line_regexp`` (``-F -w`` / ``-F -x``): a literal must occur as a whole word, or be the whole line;
+    they need ``fixed_strings`` and do not combine with ``only_matching`` (ValueError).
     """
+    if (word_regexp or line_regexp) and (only_matching or not fixed_strings):
+        raise ValueError("word_regexp / line_regexp need fixed_strings and do not combine with only_matching")
     if invert_match and only_matching:
         # GNU grep -v -o: a selected line has no matching part, so nothing is printed; the exit code still says whether
         # some line was selected.  -c / -t / -l / -L keep their output.
@@ -213,6 +219,8 @@ def parallel_grep(  # pylint: disable=too-many-arguments,too-many-locals
         "before_context": 0 if only_matching else before_context,
         "after_context": 0 if only_matching else after_context,
         "fixed_strings": fixed_strings,
+        "word_regexp": word_regexp,
+        "line_regexp": line_regexp,
     }
     workers = min(max(multiprocessing.cpu_count() - 1, 1), len(files))
     pool_type = ThreadPool if use_multithreading else multiprocessing.Pool
@@ -347,6 +355,12 @@ def parse_args(args: list | None = None) -> argparse.Namespace:
     matching.add_argument("-i", "--ignore-case", action="store_true", help="Perform case insensitive matching.")
     matching.add_argument("-v", "--invert-match", action="store_true",
                           help="Invert the sense of matching, to select non-matching lines.")
+    matching.add_argument("-w", "--word-regexp", action="store_true",
+                          help="Select only lines in which a pattern occurs as a whole word: no [0-9A-Za-z_] byte\n"
+                               "right before or after it. Needs -F here; does not combine with -o.")
+    matching.add_argument("-x", "--line-regexp", action="store_true",
+                          help="Select only lines that a pattern matches exactly (the whole line). Needs -F here;\n"
+                               "does not combine with -o.")
 
     output = parser.add_argument_group("General Output Control")
     output.add_argument("-c", "--count", action="store_true",
@@ -421,6 +435,9 @@ def main() -> None:
     except ValueError as error:
         print(error)
         raise SystemExit(2) from error
+    if (args.word_regexp or args.line_regexp) and (args.regexp != "fixed" or args.only_matching):
+        print("hyperscanner: -w / -x need -F and do not combine with -o")
+        raise SystemExit(2)
     if args.gnu_regexp and args.regexp not in ("pcre", "fixed"):
         patterns = to_gnu_regular_expressions(patterns)
     after_context = args.after_context if args.after_context is not None else args.context
@@ -467,6 +484,8 @@ def main() -> None:
             after_context=after_context,
             group_separator=args.group_separator,
             fixed_strings=args.regexp == "fixed",
+            word_regexp=args.word_regexp,
+            line_regexp=args.line_regexp,
         )
     )
 

@@ -179,3 +179,24 @@ def jsonish_bytes(size: int, seed: int = 4321, patterns_to_plant: list[str] | No
             length += len(field) + 1
         out += (",".join(fields) + "}\n").encode()
     return bytes(out[:size].rsplit(b"\n", 1)[0] + b"\n")
+
+
+_FILLER = [b"session", b"opened", b"upstream", b"handler", b"timeout", b"pending", b"device", b"req=3ec9805d", b"dur=424ms", b"pod"]
+_ERROR_WORDS = [b"errors", b"xerror", b"error_1", b"terrorize", b"errorless", b"Aerror"]
+
+
+def dense_reject_bytes(lines: int, seed: int = 1) -> tuple[bytes, list[int]]:
+    """A text for whole-word scans of `error` in which nearly every selected line is rejected: every line (about 230 bytes)
+    holds `error` inside two longer words, and one line in 97 also holds it as a word.  Returns the text and the numbers
+    (0-based) of those lines.  The lines are long enough that the fast path keeps its candidate and record capacity."""
+    rng = random.Random(seed)
+    out, words = [], []
+    for k in range(lines):
+        parts = [rng.choice(_FILLER) for _ in range(rng.randint(22, 30))]
+        for _ in range(2):
+            parts.insert(rng.randint(0, len(parts)), rng.choice(_ERROR_WORDS))
+        if k % 97 == 5:
+            parts.insert(rng.randint(0, len(parts)), rng.choice([b"error", b"(error)", b"error:", b"-error-"]))
+            words.append(k)
+        out.append(b" ".join(parts))
+    return b"\n".join(out) + b"\n", words

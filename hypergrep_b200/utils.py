@@ -157,6 +157,8 @@ def scan(  # pylint: disable=too-many-arguments
     before_context: int = 0,
     after_context: int = 0,
     fixed_strings: bool = False,
+    word_regexp: bool = False,
+    line_regexp: bool = False,
 ) -> int:
     """Scan one plain/gzip/zstd file on the GPU, delivering matched lines in batches (reference utils.py:292-358).
 
@@ -169,21 +171,31 @@ def scan(  # pylint: disable=too-many-arguments
     selected lines, and the ``after_context`` lines behind the one that reaches it are still delivered, as context.
     ``fixed_strings`` (``grep -F``): the patterns are literals, not regular expressions (gpugrep_literal_scan_file); only
     ``HS_FLAG_CASELESS`` of the flags changes anything, and every record has id 0, so ``ids`` raise ValueError.
+    ``word_regexp`` / ``line_regexp`` (``grep -F -w`` / ``-F -x``, fixed strings only): a line is selected when a literal
+    occurs in it as a whole word (no ``[0-9A-Za-z_]`` byte on either side), or when the line without its ``\n`` is a
+    literal (gpugrep_literal_whole_scan_file); with both, the line test wins, as in GNU grep.
     """
     _check_context(before_context, after_context)
+    whole = _whole_mode(fixed_strings, word_regexp, line_regexp)
     if fixed_strings and ids:
         raise ValueError("fixed_strings scans take no ids: every selected line is reported with id 0")
     pattern_array, flags_array, ids_array = prepare_patterns(patterns, flags=flags, ids=ids)
     c_callback = CALLBACK_TYPE(callback)
     lib = _get_hyperscanner_lib()
     context = before_context > 0 or after_context > 0
-    if fixed_strings:
+    if whole:
+        entry = _literal_whole_entry(lib)
+    elif fixed_strings:
         entry = _literal_entry(lib)
     else:
         entry = _context_entry(lib) if context else (_invert_entry(lib) if invert_match else None)
     outcome = {"rc": 0}
 
     def _run() -> None:
+        if whole:
+            outcome["rc"] = entry(path.encode(), pattern_array, flags_array, len(pattern_array), whole, c_callback, buffer_size,
+                                  buffer_count, max_match_count, before_context, after_context, int(invert_match), None)
+            return
         if fixed_strings:
             outcome["rc"] = entry(path.encode(), pattern_array, flags_array, len(pattern_array), c_callback, buffer_size, buffer_count,
                                   max_match_count, before_context, after_context, int(invert_match), None)
@@ -287,6 +299,33 @@ def _literal_entry(lib: ctypes.CDLL):
     return entry
 
 
+WHOLE_WORD = 1   # GPUGREP_WHOLE_WORD (include/gpugrep.h)
+WHOLE_LINE = 2   # GPUGREP_WHOLE_LINE
+
+
+def _whole_mode(fixed_strings: bool, word_regexp: bool, line_regexp: bool) -> int:
+    """The `whole` argument of gpugrep_literal_whole_scan_file, or 0 for a plain scan.  Whole words and lines exist for fixed
+    strings only; the line test wins over the word test, as in GNU grep."""
+    if (word_regexp or line_regexp) and not fixed_strings:
+        raise ValueError("word_regexp / line_regexp need fixed_strings: whole words and lines of regular expressions are not supported")
+    return WHOLE_LINE if line_regexp else (WHOLE_WORD if word_regexp else 0)
+
+
+def _literal_whole_entry(lib: ctypes.CDLL):
+    """gpugrep_literal_whole_scan_file of the loaded library (see _literal_entry)."""
+    try:
+        entry = lib.gpugrep_literal_whole_scan_file
+    except AttributeError as error:
+        raise NotImplementedError(
+            "word_regexp / line_regexp need gpugrep_literal_whole_scan_file, which the loaded native library does not export "
+            f"({_library_path()}); there is no CPU fallback"
+        ) from error
+    entry.restype = ctypes.c_int
+    entry.argtypes = [ctypes.c_char_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint, ctypes.c_uint, ctypes.c_void_p, ctypes.c_int,
+                      ctypes.c_int, ctypes.c_ulonglong, ctypes.c_uint, ctypes.c_uint, ctypes.c_int, ctypes.c_void_p]
+    return entry
+
+
 def _literal_report_entry(lib: ctypes.CDLL):
     """gpugrep_literal_report_scan_file of the loaded library (see _literal_entry)."""
     try:
@@ -351,14 +390,16 @@ def _literal_check_entry(lib: ctypes.CDLL):
 
 
 def _count_matches(path: str, patterns: Sequence[str], flags: Sequence[int], max_match_count: int,
-                   invert_match: bool = False, fixed_strings: bool = False) -> tuple[int, int] | None:
+                   invert_match: bool = False, fixed_strings: bool = False, whole: int = 0) -> tuple[int, int] | None:
     """Count-only scan without a callback: the library counts on the device and copies no line back
     (gpugrep_scan_file with on_event = NULL).  Returns None if the loaded library has no such entry point (a plain
     libhyperscanner.so), in which case the caller counts through the callback like the reference does.
     ``invert_match`` counts the lines without a match (gpugrep_invert_scan_file); it has no such fallback, nor has
-    ``fixed_strings`` (gpugrep_literal_scan_file)."""
+    ``fixed_strings`` (gpugrep_literal_scan_file) or ``whole`` (gpugrep_literal_whole_scan_file)."""
     lib = _get_hyperscanner_lib()
-    if fixed_strings:
+    if whole:
+        entry = _literal_whole_entry(lib)
+    elif fixed_strings:
         entry = _literal_entry(lib)
     elif invert_match:
         entry = _invert_entry(lib)
@@ -374,6 +415,10 @@ def _count_matches(path: str, patterns: Sequence[str], flags: Sequence[int], max
     outcome = {"rc": 0}
 
     def _run() -> None:
+        if whole:
+            outcome["rc"] = entry(path.encode(), pattern_array, flags_array, len(pattern_array), whole, None, 262140, 16, max_match_count,
+                                  0, 0, int(invert_match), ctypes.byref(stats))
+            return
         if fixed_strings:
             outcome["rc"] = entry(path.encode(), pattern_array, flags_array, len(pattern_array), None, 262140, 16, max_match_count, 0, 0,
                                   int(invert_match), ctypes.byref(stats))
@@ -403,6 +448,8 @@ def grep(  # pylint: disable=too-many-arguments
     before_context: int = 0,
     after_context: int = 0,
     fixed_strings: bool = False,
+    word_regexp: bool = False,
+    line_regexp: bool = False,
 ) -> tuple[int | list[tuple[int, str]] | list[tuple[int, str, bool]], int]:
     """grep-like collector on top of :func:`scan` (reference utils.py:147-231).
 
@@ -417,8 +464,13 @@ def grep(  # pylint: disable=too-many-arguments
     ``fixed_strings`` (``grep -F``): the patterns are literals (:func:`scan`).  With ``only_matching`` the result is that of
     the ``re.escape``-d patterns as regular expressions: every record has id 0, and the reference takes the parts of the
     pattern that the id indexes, so they are the occurrences of the first literal alone (case-sensitive, as ``re.compile``).
+    ``word_regexp`` / ``line_regexp`` (``grep -F -w`` / ``-F -x``): see :func:`scan`; they need ``fixed_strings`` and do not
+    combine with ``only_matching`` (ValueError).
     """
     _check_context(before_context, after_context)
+    whole = _whole_mode(fixed_strings, word_regexp, line_regexp)
+    if whole and only_matching:
+        raise ValueError("only_matching does not combine with word_regexp / line_regexp")
     if fixed_strings and only_matching and not invert_match:
         return _grep_fixed_only_matching(file, patterns, ignore_case, count_only, no_messages, errors, max_match_count)
     if fixed_strings and only_matching:
@@ -480,7 +532,7 @@ def grep(  # pylint: disable=too-many-arguments
     pattern_flags = _DEFAULT_FLAGS | (HS_FLAG_CASELESS if ignore_case else 0)
     if count_only:
         # SURVEY.md section 8(f)-2: counting needs no line copies and no Python frame per batch of 16 results
-        counted = _count_matches(file, patterns, [pattern_flags] * len(patterns), max_match_count, invert_match, fixed_strings)
+        counted = _count_matches(file, patterns, [pattern_flags] * len(patterns), max_match_count, invert_match, fixed_strings, whole)
         if counted is not None:
             return counted
     code = scan(
@@ -494,6 +546,8 @@ def grep(  # pylint: disable=too-many-arguments
         before_context=before_context if context else 0,
         after_context=after_context if context else 0,
         fixed_strings=fixed_strings,
+        word_regexp=whole == WHOLE_WORD,
+        line_regexp=whole == WHOLE_LINE,
     )
     if only_matching:
         _fill_spans(groups, deferred, patterns, widths, python_patterns, errors, span_lines)

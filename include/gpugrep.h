@@ -171,6 +171,31 @@ GPUGREP_API int gpugrep_literal_scan_buffer(const void* data, size_t size, int l
                                 int invert, void* stream, gpugrep_stats* stats);
 GPUGREP_API int gpugrep_check_literals(const char* const* literals, const unsigned int* literal_flags, unsigned int elements);
 
+/* ---- whole-word and whole-line fixed strings (`grep -F -w`, `grep -F -x`) ----------------------------------------
+ * Everything is as in gpugrep_literal_scan_* (pseudo-lines, the scanned block, flags, records, batches, max_match_count,
+ * context lines, inversion, on_event == NULL counting, every input form, $GPUGREP_DEVICES sharding) except what selects
+ * a line.  Its scanned block (leading NULs skipped, cut at the next NUL, the trailing '\n' included) is [b, B):
+ *  - GPUGREP_WHOLE_WORD: the line is selected when the block holds an occurrence [s, e) of some literal such that s == b
+ *    or the byte at s-1 is not a word byte, and e == B or the byte at e is not a word byte.  Word bytes are [0-9A-Za-z_]
+ *    only (bytes >= 0x80 are not): GNU grep -w in the C locale.  Every occurrence of every literal counts, overlapping ones
+ *    and literals that are prefixes of others included ("xfoo foobar" with foo and foobar is selected).
+ *  - GPUGREP_WHOLE_LINE: the line is selected when the block, without its final '\n' if it has one, equals a literal.  So
+ *    a literal that holds a '\n' never matches.
+ * CASELESS folds A-Z / a-z only in the comparison; the word test reads the raw bytes.  A pseudo-line cut by buffer_size
+ * is a line of its own.  Flag bits and return codes are those of gpugrep_literal_scan_*; a `whole` other than 1 or 2
+ * returns 4.  On the GPU the lines that the literal scan selects (a superset: such an occurrence is an occurrence) go
+ * through one more stage that keeps the lines that pass.  A build of the engine without that stage returns 7. */
+#define GPUGREP_WHOLE_WORD 1u
+#define GPUGREP_WHOLE_LINE 2u
+GPUGREP_API int gpugrep_literal_whole_scan_file(const char* file_name, const char* const* literals, const unsigned int* literal_flags,
+                                    unsigned int elements, unsigned int whole, hs_event on_event, int buffer_size,
+                                    int buffer_count, unsigned long long max_match_count, unsigned int before,
+                                    unsigned int after, int invert, gpugrep_stats* stats);
+GPUGREP_API int gpugrep_literal_whole_scan_buffer(const void* data, size_t size, int location, const char* const* literals,
+                                      const unsigned int* literal_flags, unsigned int elements, unsigned int whole,
+                                      hs_event on_event, int buffer_size, int buffer_count, unsigned long long max_match_count,
+                                      unsigned int before, unsigned int after, int invert, void* stream, gpugrep_stats* stats);
+
 /* ---- fixed strings with reports: which literal matched, and where --------------------------------------------------
  * The records are exactly those of hyperscan() / gpugrep_scan_buffer for the same set with every byte written as \xHH,
  * the same flags and the same ids (`literal_ids` NULL: all 0; `literal_flags` NULL: all 0).  That is:
