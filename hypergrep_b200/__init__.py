@@ -14,6 +14,7 @@ from hypergrep_b200.utils import RC_INVALID_FILE
 from hypergrep_b200.utils import Result
 from hypergrep_b200.utils import check_compatibility
 from hypergrep_b200.utils import configure_libraries
+from hypergrep_b200.utils import count_patterns
 from hypergrep_b200.utils import grep
 from hypergrep_b200.utils import prepare_patterns
 from hypergrep_b200.utils import scan
@@ -31,6 +32,7 @@ __all__ = [
     "Result",
     "check_compatibility",
     "configure_libraries",
+    "count_patterns",
     "grep",
     "prepare_patterns",
     "scan",

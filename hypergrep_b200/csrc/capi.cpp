@@ -334,6 +334,11 @@ struct Job {
     std::shared_ptr<Database> db;
     std::shared_ptr<DeviceDb> ddb;
     std::shared_ptr<DevicePrefilter> dpf;   // null: general path
+    // pattern-count scans: the database that attributes reports to ids (regex sets: the patterns with ids = index, event
+    // mode; fixed strings: `db` itself), on the device unless a single regex is counted (then its count is the matched lines)
+    std::shared_ptr<Database> count_db;
+    std::shared_ptr<DeviceDb> count_ddb;
+    std::vector<unsigned long long> pcounts;   // summed over the segments
     int buffer_size = 0;
     unsigned long long max_match = 0;
     Deliverer* out = nullptr;
@@ -406,6 +411,11 @@ struct Job {
         stats.segments++;
         stats.nul_segments += r.stats.nul ? 1u : 0u;
         if (stop) return 0;
+        if (r.pattern_counts) {
+            out->emit_count_only(r.num_valid_recs);
+            line_base += r.num_lines;
+            return 0;
+        }
         int rc = out->wants_spans() ? deliver_spans(r) : (wants_events() ? deliver_events(r, host, slot) : deliver_simple(r, host, slot));
         line_base += r.num_lines;
         return rc;
@@ -545,6 +555,7 @@ struct Params {
     bool literal = false;       // gpugrep_literal_scan_*(): `patterns` are fixed strings (flags: CASELESS only, no ids)
     bool literal_reports = false;   // gpugrep_literal_report_scan_*(): fixed strings with ids, one record per (id, end)
     unsigned whole = 0;         // gpugrep_literal_whole_scan_*(): GPUGREP_WHOLE_WORD or GPUGREP_WHOLE_LINE
+    unsigned long long* pattern_counts = nullptr;   // gpugrep_pattern_counts_*(): lines per pattern are added here (ids = index)
     uint32_t before = 0, after = 0;
     // the context stage runs only when lines are delivered (count-only scans ignore context)
     bool context() const { return context_scan && cb != nullptr && (before || after); }
@@ -577,6 +588,23 @@ void set_literals(ScanSlot* slot, const Params& pr) {
     if (slot_set_literal_reports) slot_set_literal_reports(slot, pr.literal_reports);
     if (slot_set_literal_whole) slot_set_literal_whole(slot, pr.whole);
 }
+// (every scan sets it: slots are pooled)
+void set_pattern_counts(ScanSlot* slot, const Job& job) {
+    if (slot_set_pattern_counts) slot_set_pattern_counts(slot, job.count_ddb.get());
+}
+// A pattern-count scan that succeeded adds its counts to pr.pattern_counts: each slot's sum over its segments, read from
+// the device once (a single regex: the matched lines).  The shards of a scan over several GPUs add theirs concurrently.
+int add_pattern_counts(const Params& pr, Job& job, ScanSlot* const* slots, int nslots, unsigned long long matches) {
+    static std::mutex mu;
+    if (!pr.pattern_counts) return 0;
+    if (job.count_ddb)
+        for (int k = 0; k < nslots; k++)
+            if (int rc = slot_read_pattern_counts(slots[k], job.pcounts, job.error)) return rc;
+    std::lock_guard<std::mutex> lk(mu);
+    if (!job.count_ddb) pr.pattern_counts[0] += matches;
+    else for (size_t i = 0; i < job.pcounts.size(); i++) pr.pattern_counts[i] += job.pcounts[i];
+    return 0;
+}
 
 int setup_job(const Params& pr, Job& job, Deliverer& out, unsigned long long weight = 0) {
     int rc = 0;
@@ -584,7 +612,8 @@ int setup_job(const Params& pr, Job& job, Deliverer& out, unsigned long long wei
     else if (pr.whole) job.db = cached_literal_whole_database(pr.patterns, pr.flags, pr.elements, rc, job.error);
     else if (pr.literal) job.db = cached_literal_database(pr.patterns, pr.flags, pr.elements, rc, job.error);
     else job.db = cached_database(pr.patterns, pr.flags, pr.ids, pr.elements, rc, job.error);
-    if (job.db && !pr.literal && (pr.invert || pr.context_scan)) {
+    if (pr.pattern_counts) job.count_db = job.db;   // (compiled with ids = index; regex sets select with the set below)
+    if (job.db && !pr.literal && (pr.invert || pr.context_scan || pr.pattern_counts)) {
         // Which lines match does not depend on ids or SINGLEMATCH: once the set compiles as given, it is scanned as "every
         // pattern SINGLEMATCH, one id 0" (simple mode, so multi-id sets take the fast path too), CASELESS/DOTALL/MULTILINE kept.
         std::vector<unsigned> flags(pr.elements), ids(pr.elements, 0u);
@@ -602,6 +631,7 @@ int setup_job(const Params& pr, Job& job, Deliverer& out, unsigned long long wei
     if (pr.literal && !slot_set_literals) { job.error = "this build of the engine has no fixed-string stage"; return GPUGREP_SCAN; }
     if (pr.literal_reports && !slot_set_literal_reports) { job.error = "this build of the engine has no fixed-string report stage"; return GPUGREP_SCAN; }
     if (pr.whole && !slot_set_literal_whole) { job.error = "this build of the engine has no whole-word / whole-line stage"; return GPUGREP_SCAN; }
+    if (pr.pattern_counts && (!slot_set_pattern_counts || !slot_read_pattern_counts)) { job.error = "this build of the engine has no pattern-count stage"; return GPUGREP_SCAN; }
     job.device_weight = weight;
     job.device = pick_device(weight, &job.device_charged);
     if (engine_select_device(job.device, job.error) != 0) {
@@ -610,6 +640,13 @@ int setup_job(const Params& pr, Job& job, Deliverer& out, unsigned long long wei
     }
     job.ddb = engine_upload(job.db, job.error);
     if (!job.ddb) return GPUGREP_SCRATCH;
+    if (pr.literal && job.count_db) {
+        job.count_ddb = job.ddb;
+    } else if (job.count_db && !job.count_db->simple) {   // (a single pattern with id 0 is simple: its count is the matched lines)
+        job.count_ddb = engine_upload(job.count_db, job.error);
+        if (!job.count_ddb) return GPUGREP_SCRATCH;
+    }
+    job.pcounts.assign(pr.pattern_counts ? pr.elements : 0u, 0ull);
     job.buffer_size = pr.buffer_size;
     job.max_match = pr.max_match;
     job.out = &out;
@@ -708,13 +745,14 @@ int scan_file(const char* path, const Params& pr, gpugrep_stats* stats_out, cons
         return GPUGREP_SCRATCH;
     }
 
-    const bool count_only = !out.wants_lines() && pr.max_match == 0 && !job.wants_events();
+    const bool count_only = !out.wants_lines() && pr.max_match == 0 && !job.wants_events() && !job.count_ddb;
     for (ScanSlot* sl : slots) {
         slot_set_want_records(sl, !count_only);
         set_invert(sl, pr.invert);
         set_context(sl, pr);
         set_spans(sl, pr);
         set_literals(sl, pr);
+        set_pattern_counts(sl, job);
     }
     SegmentQueue q;
     for (int i = 0; i < kSlots; i++) q.free_slots.push_back(i);
@@ -809,6 +847,7 @@ int scan_file(const char* path, const Params& pr, gpugrep_stats* stats_out, cons
     }
     reader.join();
     out.flush();   // hyperscanner.c:311-313
+    if (rc == 0) rc = add_pattern_counts(pr, job, slots, kSlots, out.count());
     for (ScanSlot* sl : slots) engine_release_slot(sl);
     job.stats.matches = out.count();
     job.stats.wall_ms = now_ms() - t0;
@@ -879,13 +918,14 @@ int scan_memory(const uint8_t* data, size_t size, int location, const Params& pr
     }
     ScanSlot* slots[2] = {engine_acquire_slot(err, location != GPUGREP_LOC_DEVICE), engine_acquire_slot(err, location != GPUGREP_LOC_DEVICE)};
     if (!slots[0] || !slots[1]) { engine_release_slot(slots[0]); engine_release_slot(slots[1]); set_last_error(err); return GPUGREP_SCRATCH; }
-    const bool count_only = !out.wants_lines() && pr.max_match == 0 && !job.wants_events();
+    const bool count_only = !out.wants_lines() && pr.max_match == 0 && !job.wants_events() && !job.count_ddb;
     for (ScanSlot* sl : slots) {
         slot_set_want_records(sl, !count_only);
         set_invert(sl, pr.invert);
         set_context(sl, pr);
         set_spans(sl, pr);
         set_literals(sl, pr);
+        set_pattern_counts(sl, job);
     }
     const uint8_t* seg_host[2] = {nullptr, nullptr};
     const uint8_t* seg_dev[2] = {nullptr, nullptr};
@@ -1026,6 +1066,7 @@ int scan_memory(const uint8_t* data, size_t size, int location, const Params& pr
         if (rc == 0) rc = rc2;
     }
     out.flush();
+    if (rc == 0) rc = add_pattern_counts(pr, job, slots, 2, out.count());
     engine_release_slot(slots[0]);
     engine_release_slot(slots[1]);
     job.stats.matches = out.count();
@@ -1327,6 +1368,46 @@ int gpugrep_literal_whole_scan_buffer(const void* data, size_t size, int locatio
     pr.before = before;
     pr.after = after;
     return gpugrep::scan_buffer(data, size, location, pr, stats);
+}
+
+}  // extern "C"
+
+namespace gpugrep {
+// gpugrep_pattern_counts_*: the set as hyperscan() compiles it with SINGLEMATCH and ids = index (fixed strings: the report
+// database with those ids), no callback; `run` scans with the Params.
+static int pattern_counts(const char* const* patterns, const unsigned* pattern_flags, unsigned elements, int fixed, int buffer_size,
+                          void* stream, unsigned long long* counts, const std::function<int(const Params&)>& run) {
+    if (elements == 0 || !counts) { set_last_error("pattern counts need at least one pattern and a counts array"); return GPUGREP_DB; }
+    std::fill(counts, counts + elements, 0ull);
+    // (summed here, copied out only when every shard succeeded: a failed scan leaves all counts 0)
+    std::vector<unsigned long long> sum(elements, 0ull);
+    std::vector<unsigned> flags(elements), ids(elements);
+    for (unsigned i = 0; i < elements; i++) {
+        flags[i] = (pattern_flags ? pattern_flags[i] : 0u) | 8u;
+        ids[i] = i;
+    }
+    Params pr{patterns, flags.data(), ids.data(), elements, nullptr, buffer_size, 1, 0, stream};
+    pr.pattern_counts = sum.data();
+    pr.literal = pr.literal_reports = fixed != 0;
+    const int rc = run(pr);
+    if (rc == 0) std::copy(sum.begin(), sum.end(), counts);
+    return rc;
+}
+}  // namespace gpugrep
+
+extern "C" {
+
+int gpugrep_pattern_counts_file(const char* file_name, const char* const* patterns, const unsigned int* pattern_flags, unsigned int elements,
+                                int fixed, int buffer_size, unsigned long long* counts, gpugrep_stats* stats) {
+    return gpugrep::pattern_counts(patterns, pattern_flags, elements, fixed, buffer_size, nullptr, counts,
+                                   [&](const gpugrep::Params& pr) { return gpugrep::scan_path(file_name, pr, stats); });
+}
+
+int gpugrep_pattern_counts_buffer(const void* data, size_t size, int location, const char* const* patterns, const unsigned int* pattern_flags,
+                                  unsigned int elements, int fixed, int buffer_size, void* stream, unsigned long long* counts,
+                                  gpugrep_stats* stats) {
+    return gpugrep::pattern_counts(patterns, pattern_flags, elements, fixed, buffer_size, stream, counts,
+                                   [&](const gpugrep::Params& pr) { return gpugrep::scan_buffer(data, size, location, pr, stats); });
 }
 
 int gpugrep_literal_report_scan_file(const char* file_name, const char* const* literals, const unsigned int* literal_flags,

@@ -22,6 +22,11 @@
 // fixed-string chain up to k_emit_nlm<*, LITERAL> (records even in count-only scans), then k_literal_whole_filter drops the
 // records of lines without a word / whole-line occurrence before k_dedupe_records counts them; the general path takes
 // k_match_pl_literal_whole in place of k_match_pl_literals (k_literal_whole.cuh).
+// PATTERN COUNTS (gpugrep_pattern_counts_*, slot_set_pattern_counts): the lines in which each pattern reports.  Regex
+// sets: the fast path selects the lines as a scan with records does, then k_line_events (count) -> scan -> k_line_events
+// (write) walks them with the attribution database (ids = index); the general path runs k_match_pl_events with it over every
+// pseudo-line.  Fixed strings: the report stage above.  Then k_count_patterns [-> k_count_patterns_big] adds 1 per distinct
+// (line, id) on the device, and only the counts are copied back (k_pattern_counts.cuh).
 // CONTEXT lines (grep -A/-B/-C, scans with records): a window test over the prefix count of the selected lines picks the
 // output lines of a segment (k_context.cuh, after the dedupe on the fast path, after k_match_pl_simple on the general path).
 // All byte offsets inside a segment are 32-bit (segments are < 4 GiB); line numbers are rebased on the host.
@@ -51,6 +56,7 @@
 #include "k_literal.cuh"
 #include "k_literal_reports.cuh"
 #include "k_literal_whole.cuh"
+#include "k_pattern_counts.cuh"
 #include "k_fast.cuh"
 #include "k_general.cuh"
 #include "k_invert.cuh"
@@ -154,6 +160,8 @@ struct DeviceDb {
     bool literal_reports = false;  // fixed-string set with a report table: `reps`
     bool literal_whole = false;    // fixed-string set for whole-word / whole-line scans: the report table is in `reps` too
     LiteralReportView reps{};
+    ReportIdView rids{};           // event-mode and report sets: the ids of each flat report (pattern-count scans)
+    uint32_t nids = 0;             // largest id + 1
     ~DeviceDb() { for (void* p : allocs) cudaFree(p); }
 };
 
@@ -215,12 +223,20 @@ public:
     bool literal = false;                     // fixed-string scan (slot_set_literals)
     bool reports = false;                     // fixed-string report stage (slot_set_literal_reports)
     unsigned whole = 0;                       // whole-word (1) / whole-line (2) fixed strings (slot_set_literal_whole)
+    const DeviceDb* count_db = nullptr;       // pattern-count scan (slot_set_pattern_counts): the database that attributes reports
+    // pattern counts: the counts of every segment since slot_set_pattern_counts (count_ids of them; none yet while
+    // pcounts_fresh), the segment's two totals, the lines passed on, the per-block bitmaps (zero between lines)
+    DevBuf d_pcounts, d_pmeta, d_pbig, d_pbitmaps;
+    PinBuf h_pcounts, h_pmeta;
+    bool pcounts_fresh = true;
+    size_t count_ids = 0;
     SegmentStats stats;
     bool in_use = false;
 
     int run_general(SegmentResult& out, std::string& error, size_t split_above);
     int run_spans(SegmentResult& out, size_t npl_total, std::string& error, size_t split_above);
     int run_reports(SegmentResult& out, size_t nrec, std::string& error, size_t split_above);
+    int run_pattern_counts(SegmentResult& out, size_t nlines, size_t nev, std::string& error);
     int run_complement(size_t nrec, size_t nlines, size_t selected, std::string& error);
     int run_context(size_t nrec, size_t nlines, size_t selected, size_t& count, std::string& error);
     bool context() const { return want_records && (ctx_before || ctx_after); }
@@ -309,6 +325,27 @@ std::shared_ptr<DeviceDb> engine_upload(const std::shared_ptr<Database>& db, std
         out->literal_reports = db->literal_reports;
         out->literal_whole = db->literal_whole;
         out->reps = v;
+    }
+    if (!db->simple || db->literal_reports) {
+        // flat report r -> its ids, numbered as EventRec::report: the accept sets of every group, then the NFA-fallback
+        // patterns (event mode), or the nodes of the report table
+        std::vector<uint32_t> begin{0}, ids;
+        auto add = [&](uint32_t a, uint32_t b) {
+            for (uint32_t k = a; k < b; k++) ids.push_back(db->reports[k].id);
+            begin.push_back((uint32_t)ids.size());
+        };
+        if (db->literal_reports) {
+            const auto& rb = db->lit_reports.report_begin;
+            for (size_t k = 0; k + 1 < rb.size(); k++) add(rb[k], rb[k + 1]);
+        } else {
+            for (const auto& rb : db->report_begin)
+                for (size_t k = 0; k + 1 < rb.size(); k++) add(rb[k], rb[k + 1]);
+            for (const auto& np : db->nfas) add(np.report_begin, np.report_begin + 1);
+        }
+        for (const ReportDesc& d : db->reports) out->nids = std::max(out->nids, d.id + 1);
+        out->rids.begin = (const uint32_t*)upload(begin.data(), begin.size() * 4);
+        out->rids.ids = (const uint32_t*)upload(ids.data(), ids.size() * 4);
+        if (!out->rids.begin || !out->rids.ids) { error = "cudaMalloc/cudaMemcpy failed while uploading the report ids"; return nullptr; }
     }
     std::vector<GroupDev> groups;
     for (size_t g = 0; g < db->groups.size(); g++) {
@@ -563,6 +600,10 @@ void slot_set_spans(ScanSlot* slot, const PikeProgram* program) { slot->pike = p
 void slot_set_literals(ScanSlot* slot, bool literal) { slot->literal = literal; }
 void slot_set_literal_reports(ScanSlot* slot, bool reports) { slot->reports = reports; }
 void slot_set_literal_whole(ScanSlot* slot, unsigned whole) { slot->whole = whole; }
+void slot_set_pattern_counts(ScanSlot* slot, const DeviceDb* attribution) {
+    slot->count_db = attribution;
+    slot->pcounts_fresh = true;
+}
 void slot_set_context(ScanSlot* slot, uint32_t before, uint32_t after) {
     slot->ctx_before = before;
     slot->ctx_after = after;
@@ -637,6 +678,10 @@ int slot_submit(ScanSlot* s, const DeviceDb& ddb, const DevicePrefilter* pf, con
     if (s->literal != ddb.literal) { error = "fixed-string scan of a database that is not a fixed-string set, or the reverse"; return 7; }
     if (s->reports && (!ddb.literal_reports || !s->want_records)) { error = "fixed-string report scan of a database without a report table, or without records"; return 7; }
     if (s->whole && (!ddb.literal_whole || s->whole > kWholeLine)) { error = "whole-word / whole-line scan of a database not compiled for it"; return 7; }
+    if (s->count_db && (!s->want_records || !ddb.simple || !s->count_db->rids.begin || s->count_db->device != ddb.device ||
+                        (ddb.literal ? s->count_db != &ddb || !s->reports : s->count_db->simple))) {
+        error = "pattern-count scan without records, or with databases not compiled for it"; return 7;
+    }
     s->stream = user_stream ? (cudaStream_t)user_stream : s->own_stream;
     cudaStream_t st = s->stream;
     s->ddb = &ddb;
@@ -895,12 +940,14 @@ int ScanSlot::run_general(SegmentResult& out, std::string& error, size_t split_a
         CUDA_TRY(cudaStreamSynchronize(st));
         return 0;
     }
-    DbView view{ddb->d_groups, ddb->ngroups, ddb->d_nfas, ddb->nnfa};
+    // regex pattern counts: every pseudo-line under the attribution database (fixed strings select, then report)
+    const DeviceDb* mdb = count_db && !ddb->literal ? count_db : ddb;
+    DbView view{mdb->d_groups, mdb->ngroups, mdb->d_nfas, mdb->nnfa};
     size_t nb_scan = (npl_total + kScanTile - 1) / kScanTile + 1;
     if (d_sums.reserve(nb_scan * 8) != cudaSuccess || d_recoff.reserve(npl_total * 8) != cudaSuccess) { error = "cudaMalloc failed"; return 3; }
     if (pike) return run_spans(out, npl_total, error, split_above);
     unsigned mgrid = (unsigned)((npl_total + 127) / 128);
-    if (ddb->simple) {
+    if (mdb->simple) {
         if (d_flags.reserve(npl_total) != cudaSuccess) { error = "cudaMalloc failed"; return 3; }
         if (whole) {
             static const unsigned whole_per_sm = blocks_per_sm(k_match_pl_literal_whole, 128);
@@ -968,10 +1015,13 @@ int ScanSlot::run_general(SegmentResult& out, std::string& error, size_t split_a
         }
         if (nev) {
             if (d_events.reserve(nev * sizeof(EventRec)) != cudaSuccess) { error = "cudaMalloc failed"; return 3; }
-            if (h_recs.reserve(nev * sizeof(EventRec)) != cudaSuccess) { error = "cudaHostAlloc failed"; return 3; }
+            if (!count_db && h_recs.reserve(nev * sizeof(EventRec)) != cudaSuccess) { error = "cudaHostAlloc failed"; return 3; }
             k_match_pl_events<<<mgrid, 128, 0, st>>>(view, data, d_plstart.as<uint32_t>(), d_pllen.as<uint32_t>(), npl_total, d_counts.as<uint32_t>(),
                                                      d_recoff.as<unsigned long long>(), d_events.as<EventRec>());
             stats.launches++;
+        }
+        if (count_db) return run_pattern_counts(out, npl_total, nev, error);
+        if (nev) {
             CUDA_TRY(cudaEventRecord(ev[1], st));
             CUDA_TRY(cudaMemcpyAsync(h_recs.p, d_events.p, nev * sizeof(EventRec), cudaMemcpyDeviceToHost, st));
             stats.d2h_bytes += nev * sizeof(EventRec);
@@ -1032,7 +1082,8 @@ int ScanSlot::run_spans(SegmentResult& out, size_t npl_total, std::string& error
 }
 
 // Report stage of a fixed-string report scan: the events of the first `nrec` records of d_recs (the selected lines, in line
-// order; kLineInvalid ones skipped), in line order, copied to h_recs.
+// order; kLineInvalid ones skipped), in line order, copied to h_recs.  Pattern-count scans: the events of the attribution
+// database (regex sets: k_line_events), counted on the device instead (run_pattern_counts).
 int ScanSlot::run_reports(SegmentResult& out, size_t nrec, std::string& error, size_t split_above) {
     cudaStream_t st = stream;
     Totals* dT = d_totals.as<Totals>();
@@ -1050,7 +1101,13 @@ int ScanSlot::run_reports(SegmentResult& out, size_t nrec, std::string& error, s
         static const unsigned per_sm = blocks_per_sm(k_literal_reports, 128);
         const unsigned grid = (unsigned)std::min<size_t>((nrec + 3) / 4, (size_t)per_sm * device_sms());   // a warp per record
         const LineRec* recs = d_recs.as<LineRec>();
-        k_literal_reports<<<grid, 128, 0, st>>>(ddb->reps, data, recs, nrec, d_counts.as<uint32_t>(), nullptr, nullptr);
+        const bool line_events = !ddb->literal;   // regex pattern counts: a thread per record walks the attribution database
+        const DbView cview = line_events ? DbView{count_db->d_groups, count_db->ngroups, count_db->d_nfas, count_db->nnfa} : DbView{};
+        const unsigned egrid = (unsigned)((nrec + 127) / 128);
+        if (line_events)
+            k_line_events<<<egrid, 128, 0, st>>>(cview, data, recs, nrec, d_counts.as<uint32_t>(), nullptr, nullptr);
+        else
+            k_literal_reports<<<grid, 128, 0, st>>>(ddb->reps, data, recs, nrec, d_counts.as<uint32_t>(), nullptr, nullptr);
         stats.launches++;
         launch_scan(st, LoadU32{d_counts.as<uint32_t>()}, nrec, d_recoff.as<unsigned long long>(), d_sums.as<unsigned long long>(), &dT->rec_total, stats);
         CUDA_TRY(cudaMemcpyAsync(hT, dT, sizeof(Totals), cudaMemcpyDeviceToHost, st));
@@ -1063,12 +1120,17 @@ int ScanSlot::run_reports(SegmentResult& out, size_t nrec, std::string& error, s
         }
         if (nev) {
             if (d_events.reserve(nev * sizeof(EventRec)) != cudaSuccess) { error = "cudaMalloc failed"; return 3; }
-            if (h_recs.reserve(nev * sizeof(EventRec)) != cudaSuccess) { error = "cudaHostAlloc failed"; return 3; }
-            k_literal_reports<<<grid, 128, 0, st>>>(ddb->reps, data, recs, nrec, d_counts.as<uint32_t>(), d_recoff.as<unsigned long long>(),
-                                                    d_events.as<EventRec>());
+            if (!count_db && h_recs.reserve(nev * sizeof(EventRec)) != cudaSuccess) { error = "cudaHostAlloc failed"; return 3; }
+            if (line_events)
+                k_line_events<<<egrid, 128, 0, st>>>(cview, data, recs, nrec, d_counts.as<uint32_t>(), d_recoff.as<unsigned long long>(),
+                                                     d_events.as<EventRec>());
+            else
+                k_literal_reports<<<grid, 128, 0, st>>>(ddb->reps, data, recs, nrec, d_counts.as<uint32_t>(), d_recoff.as<unsigned long long>(),
+                                                        d_events.as<EventRec>());
             stats.launches++;
         }
     }
+    if (count_db) return run_pattern_counts(out, nrec, nev, error);
     CUDA_TRY(cudaEventRecord(ev[1], st));
     if (nev) {
         CUDA_TRY(cudaMemcpyAsync(h_recs.p, d_events.p, nev * sizeof(EventRec), cudaMemcpyDeviceToHost, st));
@@ -1078,6 +1140,65 @@ int ScanSlot::run_reports(SegmentResult& out, size_t nrec, std::string& error, s
     CUDA_TRY(cudaGetLastError());
     out.events = h_recs.as<EventRec>();
     out.num_events = nev;
+    return 0;
+}
+
+// Pattern counts of a segment: the `nev` events of d_events, those of line r at d_recoff[r] (d_counts[r] of them, r <
+// nlines), counted per distinct (line, id) and added to the slot's counts in d_pcounts, which stay on the device until
+// slot_read_pattern_counts.  The segment's matched lines (those with an event) are its num_valid_recs.
+int ScanSlot::run_pattern_counts(SegmentResult& out, size_t nlines, size_t nev, std::string& error) {
+    cudaStream_t st = stream;
+    const size_t nids = count_db->nids;
+    if (pcounts_fresh) {
+        if (d_pcounts.reserve(nids * 8) != cudaSuccess) { error = "cudaMalloc failed for the pattern counts"; return 3; }
+        CUDA_TRY(cudaMemsetAsync(d_pcounts.p, 0, nids * 8, st));
+        count_ids = nids;
+        pcounts_fresh = false;
+    }
+    if (d_pmeta.reserve(16) != cudaSuccess || h_pmeta.reserve(16) != cudaSuccess) { error = "allocation failed for the pattern counts"; return 3; }
+    unsigned long long* pc = d_pcounts.as<unsigned long long>();
+    unsigned long long* meta = d_pmeta.as<unsigned long long>();
+    CUDA_TRY(cudaMemsetAsync(meta, 0, 16, st));
+    if (nev) {
+        const unsigned sms = (unsigned)device_sms();
+        const size_t words = (nids + 31) / 32;
+        const unsigned bgrid = std::min(sms, 32u);
+        if (d_pbig.reserve(nlines * 4) != cudaSuccess || d_pbitmaps.reserve((size_t)bgrid * words * 4) != cudaSuccess) {
+            error = "cudaMalloc failed for the pattern counts"; return 3;
+        }
+        // (at most 32 bitmaps of nids bits: 4 MiB for 10^6 ids, cleared in a few microseconds)
+        CUDA_TRY(cudaMemsetAsync(d_pbitmaps.p, 0, (size_t)bgrid * words * 4, st));
+        static const unsigned per_sm = blocks_per_sm(k_count_patterns, 128);
+        const unsigned grid = (unsigned)std::min<size_t>((nlines + kCountWarps - 1) / kCountWarps, (size_t)per_sm * sms);   // a warp per line
+        k_count_patterns<<<grid, 128, 0, st>>>(count_db->rids, d_events.as<EventRec>(), d_counts.as<uint32_t>(), d_recoff.as<unsigned long long>(),
+                                               nlines, pc, meta, d_pbig.as<uint32_t>());
+        k_count_patterns_big<<<bgrid, 256, 0, st>>>(count_db->rids, d_events.as<EventRec>(), d_counts.as<uint32_t>(), d_recoff.as<unsigned long long>(),
+                                                    meta, d_pbig.as<uint32_t>(), pc, d_pbitmaps.as<uint32_t>(), words);
+        stats.launches += 2;
+    }
+    CUDA_TRY(cudaEventRecord(ev[1], st));
+    CUDA_TRY(cudaMemcpyAsync(h_pmeta.p, meta, 16, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaGetLastError());
+    stats.d2h_bytes += 16;
+    out.lines = nullptr;
+    out.num_line_recs = 0;
+    out.events = nullptr;
+    out.num_events = 0;
+    out.pattern_counts = true;
+    out.num_valid_recs = (size_t)h_pmeta.as<unsigned long long>()[0];
+    return 0;
+}
+
+int slot_read_pattern_counts(ScanSlot* s, std::vector<unsigned long long>& sum, std::string& error) {
+    if (s->pcounts_fresh) return 0;   // no segment was counted
+    const size_t nids = s->count_ids;
+    if (s->h_pcounts.reserve(nids * 8) != cudaSuccess) { error = "cudaHostAlloc failed for the pattern counts"; return 3; }
+    CUDA_TRY(cudaMemcpyAsync(s->h_pcounts.p, s->d_pcounts.p, nids * 8, cudaMemcpyDeviceToHost, s->stream));
+    CUDA_TRY(cudaStreamSynchronize(s->stream));
+    const unsigned long long* h = s->h_pcounts.as<unsigned long long>();
+    for (size_t i = 0; i < std::min(nids, sum.size()); i++) sum[i] += h[i];
+    s->pcounts_fresh = true;
     return 0;
 }
 
@@ -1182,7 +1303,7 @@ int slot_collect(ScanSlot* s, SegmentResult& out, std::string& error, size_t spl
             out.num_valid_recs = (size_t)hT->aux_total;
             const size_t nl_total = (size_t)(uint32_t)hT->meta_total;
             out.num_lines = nl_total + ((hT->last_byte & 0xff) != '\n' ? 1 : 0);
-            if (s->reports) {
+            if (s->reports || s->count_db) {
                 int rc = s->run_reports(out, nrec, error, split_above);
                 if (rc == kSplitSegment) out.stats = s->stats;
                 if (rc) return rc;
@@ -1209,7 +1330,7 @@ int slot_collect(ScanSlot* s, SegmentResult& out, std::string& error, size_t spl
                 CUDA_TRY(cudaStreamSynchronize(s->copy_stream));
                 s->stats.d2h_bytes += nrec * sizeof(LineRec);
             }
-            if (!s->reports) {
+            if (!s->reports && !s->count_db) {
                 out.lines = s->want_records ? s->h_recs.as<LineRec>() : nullptr;
                 out.num_line_recs = nrec;
             }

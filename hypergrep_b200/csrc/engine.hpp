@@ -56,6 +56,8 @@ struct SegmentResult {
     size_t num_events = 0;
     const SpanRec* spans = nullptr;   // span stage (slot_set_spans): by line, then start
     size_t num_spans = 0;
+    bool pattern_counts = false;      // pattern-count scan (slot_set_pattern_counts): num_valid_recs is the matched lines, the
+                                      // counts per id stay on the device (slot_read_pattern_counts)
     SegmentStats stats;
 };
 
@@ -126,6 +128,17 @@ __attribute__((weak)) void slot_set_literal_reports(ScanSlot* slot, bool reports
 // selection (inversion, context lines, counts, records) follows from the lines kept.  Call before slot_submit.  Weak like
 // slot_set_invert (a build without it fails such scans with 7).
 __attribute__((weak)) void slot_set_literal_whole(ScanSlot* slot, unsigned whole);
+// Pattern counts (gpugrep_pattern_counts_*), on a slot that wants records: per id of `attribution`, the number of
+// pseudo-lines in which some report of that id fires is added to counts the slot keeps on the device over its segments
+// (read them with slot_read_pattern_counts); a segment's results are SegmentResult::pattern_counts and num_valid_recs, the
+// number of lines with a report; no lines or events.  The call starts the slot's counts from 0.  Regex sets: the slot's database is the
+// simple-mode selection set and `attribution` the same patterns with their own ids (event mode, uploaded to the same
+// device).  Fixed strings: `attribution` is the slot's own report database, with slot_set_literal_reports on.  Null
+// switches it off.  Call before slot_submit.  Weak like slot_set_invert (a build without it fails such scans with 7).
+__attribute__((weak)) void slot_set_pattern_counts(ScanSlot* slot, const DeviceDb* attribution);
+// Add the slot's pattern counts (ids 0 .. sum.size() - 1) to `sum`, one copy from the device, after its last slot_collect;
+// its counts then start from 0 again.  Weak like slot_set_pattern_counts.
+__attribute__((weak)) int slot_read_pattern_counts(ScanSlot* slot, std::vector<unsigned long long>& sum, std::string& error);
 // Wait for the segment and expose its results (valid until the next slot_submit on this slot).
 // Returns kSplitSegment (and no results) when the fast path hit one of its capacity bounds - a line too long for it, a
 // candidate or record overflow - in a segment of more than `split_above` bytes: the caller then scans the same bytes again

@@ -12,6 +12,7 @@ from __future__ import annotations
 
 import argparse
 import multiprocessing
+import os
 import re
 import sys
 import textwrap
@@ -369,7 +370,7 @@ def parse_args(args: list | None = None) -> argparse.Namespace:
                         help="Suppress normal output; print the name of each input file without a match.")
     output.add_argument("-l", "--files-with-matches", action="store_true",
                         help="Suppress normal output; print the name of each input file with a match.")
-    output.add_argument("-m", "--max-count", type=int, default=0, help="Stop reading a file after NUM matching lines.")
+    output.add_argument("-m", "--max-count", type=int, default=None, help="Stop reading a file after NUM matching lines.")
     output.add_argument("-o", "--only-matching", action="store_true",
                         help="Print only the matched (non-empty) parts of a matching line, one per output line.")
     output.add_argument("-q", "--quiet", "--silent", action="store_true",
@@ -405,6 +406,11 @@ def parse_args(args: list | None = None) -> argparse.Namespace:
     extra = parser.add_argument_group("Unique arguments to hyperscanner")
     extra.add_argument("-t", "--total", action="store_true",
                        help="Suppress normal output; print a count of matching lines across all input files.")
+    extra.add_argument("--count-per-pattern", action="store_true",
+                       help="Suppress normal output; for each input file print one line [FILE:]COUNT:PATTERN per pattern,\n"
+                            "in the order given, zeros included: the number of lines the pattern matches in. With -t,\n"
+                            "COUNT:PATTERN summed over all input files. Does not combine with -v -o -w -x -c -l -L -q\n"
+                            "-m -n -A -B -C.")
     extra.add_argument("--no-gnu", dest="gnu_regexp", action="store_false",
                        help="Disable GNU grep compatibility rewrites of BRE/ERE patterns (\\< and \\> become \\b).")
     extra.add_argument("--no-order", dest="ordered", action="store_false",
@@ -423,18 +429,64 @@ def _usage_exit(args: argparse.Namespace) -> None:
     raise SystemExit(2)
 
 
+_NOT_WITH_COUNT_PER_PATTERN = (
+    ("invert_match", "-v"), ("only_matching", "-o"), ("word_regexp", "-w"), ("line_regexp", "-x"), ("count", "-c"),
+    ("files_with_matches", "-l"), ("files_without_match", "-L"), ("quiet", "-q"), ("max_count", "-m"), ("line_number", "-n"),
+    ("after_context", "-A"), ("before_context", "-B"), ("context", "-C"),
+)
+
+
+def count_per_pattern(files: list[str], patterns: list[str], given: list[str], fixed_strings: bool, ignore_case: bool, total: bool,
+                      with_file_name: bool, no_messages: bool) -> int:
+    """``--count-per-pattern``: one line ``[file:]count:pattern`` per file and pattern (``count:pattern`` summed over the files
+    with ``total``), ``given`` being the patterns as the user wrote them.  Returns the exit code: 0 when some count is
+    non-zero, 1 when none is, 2 after an error."""
+    sums = [0] * len(patterns)
+    error = False
+    for file in files:
+        if not os.path.isfile(file):
+            if not no_messages:
+                print(f"hyperscanner: {file}: " + ("Is a directory" if os.path.isdir(file) else "No such file or directory"))
+            error = True
+            continue
+        counts, code = hypergrep.count_patterns(file, patterns, fixed_strings=fixed_strings, ignore_case=ignore_case)
+        if code:
+            print(f"hyperscanner: {file}: the per-pattern count failed (return code {code})")
+            if code == 4:   # the patterns do not compile: the same for every file
+                raise SystemExit(2)
+            error = True
+            continue
+        sums = [a + b for a, b in zip(sums, counts)]
+        if not total:
+            prefix = f"{file}:" if with_file_name else ""
+            print("".join(f"{prefix}{count}:{pattern}\n" for count, pattern in zip(counts, given)), end="")
+    if total:
+        print("".join(f"{count}:{pattern}\n" for count, pattern in zip(sums, given)), end="")
+    if error:
+        return 2
+    return 0 if any(sums) else 1
+
+
 def main() -> None:
     """Entry point of the ``hyperscanner`` command (reference multiscanner.py:551-606)."""
     args = parse_args()
+    given: list[str] = []
     try:
         patterns = get_argparse_patterns(args)
         if not patterns:
             _usage_exit(args)
+        given = list(patterns)
         if args.regexp == "bre":
             patterns = to_basic_regular_expressions(patterns)
     except ValueError as error:
         print(error)
         raise SystemExit(2) from error
+    if args.count_per_pattern:
+        # (a given value refuses, 0 included: -m 0 selects no line, -A 0 asks for context)
+        clash = [flag for name, flag in _NOT_WITH_COUNT_PER_PATTERN if getattr(args, name) is not None and getattr(args, name) is not False]
+        if clash:
+            print(f"hyperscanner: --count-per-pattern does not combine with {' '.join(clash)}")
+            raise SystemExit(2)
     if (args.word_regexp or args.line_regexp) and (args.regexp != "fixed" or args.only_matching):
         print("hyperscanner: -w / -x need -F and do not combine with -o")
         raise SystemExit(2)
@@ -461,6 +513,9 @@ def main() -> None:
         with_file_name = True
     else:
         with_file_name = len(files) > 1
+    if args.count_per_pattern:
+        raise SystemExit(count_per_pattern(files, patterns, given, args.regexp == "fixed", args.ignore_case, args.total, with_file_name,
+                                           args.no_messages))
 
     raise SystemExit(
         parallel_grep(
@@ -475,7 +530,7 @@ def main() -> None:
             use_multithreading=args.use_multithreading,
             only_matching=args.only_matching,
             no_messages=args.no_messages,
-            max_match_count=args.max_count,
+            max_match_count=args.max_count or 0,
             quiet=args.quiet,
             files_without_match=args.files_without_match,
             files_with_matches=args.files_with_matches,

@@ -376,6 +376,61 @@ def scan_literals(  # pylint: disable=too-many-arguments
     return outcome["rc"]
 
 
+def _pattern_counts_entry(lib: ctypes.CDLL):
+    """gpugrep_pattern_counts_file of the loaded library (see _literal_entry)."""
+    try:
+        entry = lib.gpugrep_pattern_counts_file
+    except AttributeError as error:
+        raise NotImplementedError(
+            "count_patterns needs gpugrep_pattern_counts_file, which the loaded native library does not export "
+            f"({_library_path()}); there is no CPU fallback"
+        ) from error
+    entry.restype = ctypes.c_int
+    entry.argtypes = [ctypes.c_char_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint, ctypes.c_int, ctypes.c_int, ctypes.c_void_p,
+                      ctypes.c_void_p]
+    return entry
+
+
+def count_patterns(  # pylint: disable=too-many-arguments
+    file: str,
+    patterns: Sequence[str],
+    flags: Sequence[int] = (),
+    fixed_strings: bool = False,
+    ignore_case: bool = False,
+    buffer_size: int = 262140,
+) -> tuple[list[int], int]:
+    """Count, for each pattern, the lines of one plain/gzip/zstd file in which it matches (gpugrep_pattern_counts_file).
+
+    Returns ``(counts, return_code)``: ``counts[i]`` is the number of lines (pseudo-lines of ``buffer_size``, as in
+    :func:`scan`) in which ``patterns[i]`` matches, which is the number of records with id ``i`` that :func:`scan` delivers
+    for the same patterns with ``ids = range(len(patterns))`` and every flag plus ``HS_FLAG_SINGLEMATCH``.  Identical
+    patterns each get their own count.  ``flags`` default to DOTALL|MULTILINE|SINGLEMATCH; ``ignore_case`` adds
+    ``HS_FLAG_CASELESS`` to each.  ``fixed_strings``: the patterns are literals (:func:`scan_literals`).  The counts are made on
+    the GPU in one pass over the file; only they are copied back.  On a nonzero code the counts are all 0.
+    """
+    pattern_array, flags_array, _ = prepare_patterns(patterns, flags=flags)
+    count = len(pattern_array)
+    if ignore_case:
+        for i in range(count):
+            flags_array[i] |= HS_FLAG_CASELESS
+    counts = (ctypes.c_ulonglong * max(count, 1))()
+    entry = _pattern_counts_entry(_get_hyperscanner_lib())
+    outcome = {"rc": 0}
+
+    def _run() -> None:
+        outcome["rc"] = entry(file.encode(), pattern_array, flags_array, count, int(fixed_strings), buffer_size, counts, None)
+
+    worker = threading.Thread(target=_run, daemon=True)   # same interruptible wait as scan()
+    worker.start()
+    try:
+        worker.join(timeout=3600)
+    except KeyboardInterrupt:
+        outcome["rc"] = _RC_INTERRUPTED
+    if outcome["rc"]:
+        return [0] * count, outcome["rc"]
+    return list(counts[:count]), 0
+
+
 def _literal_check_entry(lib: ctypes.CDLL):
     """gpugrep_check_literals of the loaded library (see _literal_entry)."""
     try:

@@ -220,6 +220,28 @@ GPUGREP_API int gpugrep_literal_report_scan_buffer(const void* data, size_t size
                                        hs_event on_event, int buffer_size, int buffer_count, unsigned long long max_match_count,
                                        void* stream, gpugrep_stats* stats);
 
+/* ---- per-pattern line counts: which patterns occur, and in how many lines ------------------------------------------
+ * counts[i] (elements entries, overwritten) is the number of pseudo-lines whose scanned block holds at least one report
+ * of pattern i: the number of records with id i that hyperscan() delivers for the same patterns with flags | SINGLEMATCH
+ * and ids 0 .. elements-1.  Pseudo-lines, the scanned block (leading NULs skipped, cut at the next NUL, the trailing '\n'
+ * included) and buffer_size are those of hyperscan().  Identical patterns each get their own count.
+ *  - fixed == 0: the entries are regular expressions; CASELESS, DOTALL and MULTILINE work as in hyperscan(), SINGLEMATCH
+ *    changes nothing.  Returns 4 exactly when hyperscan() returns 4 for the set.
+ *  - fixed != 0: the entries are literals under the gpugrep_literal_* rules (CASELESS folds A-Z / a-z only; return codes
+ *    of gpugrep_check_literals).  A literal with a '\n' before its last byte counts 0.
+ * elements == 0 or counts == NULL returns 4.  stats->matches is the number of lines in which some pattern reports (the
+ * count-only scan of the set).  Inputs are those of gpugrep_scan_file / _buffer (plain, gzip and zstd files; pageable,
+ * pinned and device buffers; $GPUGREP_DEVICES sharding); the counts are summed over segments and shards.  The 2^27
+ * events-per-segment bound of multi-id scans applies (7).  Everything is counted on the GPU and only the counts are
+ * copied back, once per scan.  On a nonzero return code every count is 0.  A build of the engine without the stage returns
+ * 7. */
+GPUGREP_API int gpugrep_pattern_counts_file(const char* file_name, const char* const* patterns, const unsigned int* pattern_flags,
+                                            unsigned int elements, int fixed, int buffer_size, unsigned long long* counts,
+                                            gpugrep_stats* stats);
+GPUGREP_API int gpugrep_pattern_counts_buffer(const void* data, size_t size, int location, const char* const* patterns,
+                                              const unsigned int* pattern_flags, unsigned int elements, int fixed, int buffer_size,
+                                              void* stream, unsigned long long* counts, gpugrep_stats* stats);
+
 /* ---- match END offsets (SURVEY.md section 8f-4: spans for `grep -o`) --------------------------------------------
  * The reference gets the spans of `-o` by re-running Python's re.finditer() over every matched line (utils.py:205-212);
  * Hyperscan itself reports (id, end offset) per match and the reference drops the offset (hyperscanner.c:83-102).
